@@ -10,9 +10,13 @@ CubicLattice((1000,1000,1)) altermagnet/superconductor Josephson junction, 10^6 
 synthetic (SURVEY 8d).  N > 1: one process per GPU (torchrun), a replica of the matrix and its own 8 columns on
 every GPU (weak scaling), one NCCL all-reduce of the moments at the end of the timed region.
 
-Timed region: W warm-up steps, then R x K steps between two CUDA events on the launch stream, R chosen (from a
-pilot of K steps, the same R on every rank) so that the region lasts >= 1 s whatever K the caller passes --
-``steps`` echoes K, ``repeats`` R, ``timed_steps`` R*K; barrier + synchronize on both sides, max over ranks.
+Timed region: W warm-up steps, then K steps between two CUDA events on the launch stream; barrier + synchronize on
+both sides, max over ranks.  ``steps`` echoes K, ``timed_steps`` counts the steps the region ran (K, or K + 1 for an
+odd K on a kernel that advances two steps per launch).  The comparison runs and extras time K steps each as well.
+
+``--dump-outputs DIR``: after the timed steps, the moments the headline recursion has computed are written as
+``DIR/*.npy`` (float64, see ``dump_moments``); the inputs are fixed by the arguments, so two builds run with the same
+arguments can be compared output for output.
 
 Prints ONE JSON line.  ``value`` = whole-job steps/s with everything resident in HBM; ``e2e`` = the same metric
 through the public API with the Hamiltonian terms in pinned HOST memory (upload + scatter + recursion + moments
@@ -32,7 +36,6 @@ from __future__ import annotations
 
 import argparse
 import json
-import math
 import os
 import statistics
 import subprocess
@@ -42,19 +45,20 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the bench leaves the tree as it found it (it may be read-only)
 
 import numpy as np  # noqa: E402
 
 METRIC = "chebyshev_spmm_steps_per_s"
 UNIT = "steps/s"
 FALLBACK_HBM_GBS = 6650.0
-MIN_TIMED_S = 1.0
+DUMP_BYTES = 64 << 20
 
 
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=2000)
+    ap.add_argument("--steps", type=int, default=2000, help="timed steps of every recursion timing")
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", default="C5")
@@ -68,7 +72,11 @@ def parse_args():
     ap.add_argument("--no-plain", action="store_true", help="skip the uncompressed-matrix / three-term comparison runs")
     ap.add_argument("--no-extras", action="store_true",
                     help="skip block_repetition, other_configs and strong_scaling (only run with the default C5 headline)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the moments of the timed recursion to DIR/*.npy")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU path's outputs (--impl ours)")
+    return args
 
 
 def measured_peak():
@@ -298,10 +306,9 @@ class Bench:
         system._sys.set_stream(self.stream.cuda_stream)
         return system
 
-    def timed(self, system, cols, kernel, K, W, *, col_offset=None, probe_rows=None, min_s=MIN_TIMED_S, reduce_moments=True,
-              scale=None):
-        """W warm-up + R x K timed steps of `kernel` (R: see the module docstring), then the single exchange of the
-        path (summed moments of all column shards).  Times are the max over ranks."""
+    def timed(self, system, cols, kernel, K, W, *, col_offset=None, probe_rows=None, reduce_moments=True, scale=None):
+        """W warm-up + K timed steps of `kernel`, then the single exchange of the path (summed moments of all column
+        shards).  Times are the max over ranks."""
         torch, dist, s = self.torch, self.dist, system._sys
         scale = system.spectral_bound() if scale is None else scale
         if probe_rows is not None:
@@ -309,33 +316,19 @@ class Bench:
         else:
             s.cheb_begin(n_random=cols, seed=1234, col_offset=self.rank * cols if col_offset is None else col_offset,
                          scale=scale, kernel=kernel)
-        s.cheb_reserve(W + 2 * K + 8)
+        s.cheb_reserve(W + K + 8)
         s.cheb_steps(W)
-        launches_before_pilot = s.cheb_info()["launches"]
-        # pilot: K steps, to size the timed region (and, the GPU still cool, the kernel at burst clocks)
-        p0, p1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        torch.cuda.synchronize()
-        p0.record(self.stream)
-        s.cheb_steps(K)
-        p1.record(self.stream)
-        torch.cuda.synchronize()
-        pilot_ms = self.max_over_ranks([p0.elapsed_time(p1)])[0]
-        pilot_launches = s.cheb_info()["launches"]
-        R = max(1, int(math.ceil(min_s * 1e3 / max(pilot_ms, 1e-3))))
-        s.cheb_reserve(R * K + 8)
         info, fmt = s.cheb_info(), s.cheb_format()
-        launches0 = info["launches"]
-        n_mom = s.cheb_available() + 2 * R * K
-        mu_dev = torch.empty(n_mom, dtype=torch.float64, device=self.dev)
+        launches0, avail0 = info["launches"], s.cheb_available()
+        mu_dev = torch.empty(avail0 + 2 * (K + 1), dtype=torch.float64, device=self.dev)  # (+1: an odd K rounded up)
         e0, e1, e2 = (torch.cuda.Event(enable_timing=True) for _ in range(3))
         self.barrier()
         torch.cuda.synchronize()
         e0.record(self.stream)
-        for _ in range(R):
-            s.cheb_steps(K)
+        s.cheb_steps(K)
         e1.record(self.stream)
         step_launches = s.cheb_info()["launches"] - launches0
-        n_mom = min(n_mom, s.cheb_available())
+        n_mom = s.cheb_available()
         if reduce_moments:
             s.cheb_read(n_mom, cols, summed=True, device_ptr=mu_dev.data_ptr())
             if self.world > 1:
@@ -344,17 +337,16 @@ class Bench:
         torch.cuda.synchronize()
         self.barrier()
         total_ms, kernel_ms = self.max_over_ranks([e0.elapsed_time(e2), e0.elapsed_time(e1)])
-        steps = R * K
+        steps = (n_mom - avail0) // 2
         n_sites = system.lattice.size
         kname = fmt["kernel"]
         moved_step = fmt["matrix_bytes_per_step"] + VECTOR_PASSES.get(kname, 192) * n_sites * cols
-        return {"kernel": kname, "steps": steps, "repeats": R, "total_ms": total_ms, "kernel_ms": kernel_ms,
+        return {"kernel": kname, "steps": steps, "total_ms": total_ms, "kernel_ms": kernel_ms,
                 "step_launches": step_launches, "gpu_launches": s.cheb_info()["launches"] - launches0,
                 "ms_per_step": total_ms / steps, "kernel_ms_per_step": kernel_ms / steps,
                 "steps_per_launch": steps / max(step_launches, 1), "bytes_per_step": info["bytes_per_step"],
                 "moved_bytes_per_step": moved_step, "distinct_blocks": fmt["distinct_blocks"], "n_blocks": info["n_blocks"],
-                "panel_width": info["panel_width"], "mu": mu_dev[:n_mom] if reduce_moments else None, "scale": scale,
-                "pilot_ms": pilot_ms, "pilot_steps": K, "pilot_launches": pilot_launches - launches_before_pilot}
+                "panel_width": info["panel_width"], "mu": mu_dev[:n_mom] if reduce_moments else None, "scale": scale}
 
     def summary(self, t, cfg_key, cols, *, jobs):
         """Compact record of a `timed()` result: throughput + the physical roofline fraction."""
@@ -425,6 +417,33 @@ def pinned_h2d_peak(torch, local, nbytes=1 << 29):
         torch.cuda.synchronize()
         best = max(best, nbytes / (e0.elapsed_time(e1) * 1e-3) / 1e9)
     return best
+
+
+def dump_moments(B, system, head, cols, out_dir):
+    """``--dump-outputs``: the Chebyshev moments mu_n of the headline recursion once its last timed step is done, as a
+    caller of the path receives them, in float64: ``moments.npy`` [n, columns] per column (every rank's columns in rank
+    order), ``moments_summed.npy`` [n] summed over all columns (what the timed region reads), ``moment_index.npy`` [n]
+    the orders n.  Should the three exceed DUMP_BYTES, a fixed, seeded sample of the orders is kept, the moments of the
+    last step always among them.  Collective over the ranks; rank 0 writes."""
+    torch = B.torch
+    n_mom = len(head["mu"])
+    per_col = system._sys.cheb_read(n_mom, cols)
+    if B.world > 1:
+        mine = torch.from_numpy(per_col).to(B.dev)
+        parts = [torch.empty_like(mine) for _ in range(B.world)]
+        B.dist.all_gather(parts, mine)
+        per_col = torch.cat(parts, dim=1).cpu().numpy()
+    if B.rank != 0:
+        return
+    row_bytes = 8 * (per_col.shape[1] + 2)
+    n = np.arange(n_mom)
+    if n_mom * row_bytes > DUMP_BYTES - 4096:  # (4096: room for the .npy headers)
+        keep = (DUMP_BYTES - 4096) // row_bytes
+        n = np.concatenate([np.sort(np.random.default_rng(0).choice(n_mom - 2, keep - 2, replace=False)), n[-2:]])
+    os.makedirs(out_dir, exist_ok=True)
+    for name, arr in (("moments", per_col[n]), ("moments_summed", head["mu"].cpu().numpy()[n]),
+                      ("moment_index", n.astype(np.float64))):
+        np.save(os.path.join(out_dir, f"{name}.npy"), arr)
 
 
 def run_ours(args):
@@ -502,6 +521,8 @@ def run_ours(args):
     jobs = world if scaling == "weak" else 1
     assert abs(mu0 - 4.0 * n_sites * cols * world) < 1e-6 * mu0, "moment 0 must equal the number of vector entries"
     mu16 = mu_all[:16].cpu().numpy().copy()
+    if args.dump_outputs:
+        dump_moments(B, system, head, cols, args.dump_outputs)
 
     # ---- parity at N > 1: every shard's columns recomputed on rank 0 ----------------------------------
     parity = None
@@ -523,7 +544,7 @@ def run_ours(args):
     plain = three_term = None
     if not args.no_plain and head["kernel"] != "ell":
         try:
-            t = B.timed(system, cols, "ell", K, W, min_s=0.25, scale=scale)
+            t = B.timed(system, cols, "ell", K, W, scale=scale)
             plain = B.summary(t, args.config, cols, jobs=jobs)
         except (ValueError, RuntimeError):
             plain = None
@@ -532,7 +553,7 @@ def run_ours(args):
         three_term = {}
         for name in ("pair", "dict_diag"):
             try:
-                t = B.timed(system, cols, name, K, W, min_s=0.25, scale=scale)
+                t = B.timed(system, cols, name, K, W, scale=scale)
             except (ValueError, RuntimeError):
                 continue
             three_term[t["kernel"]] = B.summary(t, args.config, cols, jobs=jobs)
@@ -541,7 +562,7 @@ def run_ours(args):
     strong = None
     if extras and 64 % world == 0:
         kc = 64 // world
-        t = B.timed(system, kc, args.kernel, K, W, min_s=0.5, col_offset=rank * kc, scale=scale)
+        t = B.timed(system, kc, args.kernel, K, W, col_offset=rank * kc, scale=scale)
         strong = B.summary(t, args.config, kc, jobs=1)
         strong["total_cols"] = 64
         strong["what"] = "one job of 64 columns split over the GPUs: steps/s of the whole job (a step is done when every shard has done it)"
@@ -585,7 +606,7 @@ def run_ours(args):
         for key in ("C5_disordered", "C5_random", "C5_periodic"):
             try:
                 sysx = B.build(key)
-                t = B.timed(sysx, cols, args.kernel, K, W, min_s=0.5)
+                t = B.timed(sysx, cols, args.kernel, K, W)
                 repetition[key] = B.summary(t, key, cols, jobs=jobs)
                 repetition[key]["workload"] = workloads.CONFIGS[key]["label"]
                 del sysx
@@ -596,12 +617,12 @@ def run_ours(args):
         for key, kc in (("C2", 256), ("C4", 8)):
             try:
                 sysx = B.build(key)
-                t = B.timed(sysx, kc, args.kernel, K, W, min_s=0.3)
+                t = B.timed(sysx, kc, args.kernel, K, W)
                 others[key] = B.summary(t, key, kc, jobs=jobs)
                 if key == "C4" and others[key]["kernel"] == "t2":
                     # three-dimensional lattice: the even-vector kernel (csrc/cheb_cube.cu) moves half the bytes in about the
                     # time of the single-step kernel -- both, so that steps/s and the roofline fraction can be read side by side
-                    t1 = B.timed(sysx, kc, "dict_diag", K, W, min_s=0.3)
+                    t1 = B.timed(sysx, kc, "dict_diag", K, W)
                     others["C4_single_step"] = B.summary(t1, key, kc, jobs=jobs)
                 del sysx
             except (RuntimeError, ValueError, MemoryError) as err:
@@ -610,11 +631,11 @@ def run_ours(args):
         sites = [(3 * p + 2, 3 * q + 2, 0) for p in range(32) for q in range(32)]
         rows = sysx._probe_rows(sites)
         lo, hi = b.distributed.shard_range(len(rows), rank, world)
-        t = B.timed(sysx, hi - lo, args.kernel, K, W, min_s=0.3, probe_rows=rows[lo:hi], reduce_moments=False)
+        t = B.timed(sysx, hi - lo, args.kernel, K, W, probe_rows=rows[lo:hi], reduce_moments=False)
         others["C3"] = B.summary(t, "C3", hi - lo, jobs=1)
         others["C3"]["what"] = "4096 probe columns (1024 sites x 4) sharded over the GPUs: steps/s of the whole LDOS job"
         if world == 1:  # BASELINE shards C3 over 2/4/8 GPUs: one GPU's share of the 8-GPU run (512 columns) beside the whole job
-            t8 = B.timed(sysx, 512, args.kernel, K, W, min_s=0.3, probe_rows=rows[:512], reduce_moments=False)
+            t8 = B.timed(sysx, 512, args.kernel, K, W, probe_rows=rows[:512], reduce_moments=False)
             others["C3_share_of_8"] = B.summary(t8, "C3", 512, jobs=1)
             others["C3_share_of_8"]["what"] = "the 512 probe columns one GPU holds when C3 is sharded over 8 GPUs (SURVEY 8d)"
         # the exchange of this path: all-gather of the per-column moments (column order = rank order), checked
@@ -654,15 +675,6 @@ def run_ours(args):
                         "speedup_vs_one_pass_roofline: > 1 because the block dictionary takes the matrix out of the stream and the "
                         "even-vector recursion moves three vector passes per TWO steps",
                 "assembly": assembly}
-    # the same kernel in the K pilot steps right after the warm-up, before the power cap pulls the SM clock down
-    burst_launch_ms = head["pilot_ms"] / max(head["pilot_launches"], 1)
-    phys_launch = roofline["traffic"] or hs["moved_bytes_per_launch"]
-    roofline["burst"] = {"steps": head["pilot_steps"], "kernel_ms_per_launch": burst_launch_ms,
-                         "steps_per_s": jobs * head["pilot_steps"] / (head["pilot_ms"] * 1e-3),
-                         "achieved_GBps": phys_launch / (burst_launch_ms * 1e-3) / 1e9,
-                         "frac": phys_launch / (burst_launch_ms * 1e-3) / 1e9 / B.peak,
-                         "what": "the K pilot steps that size the timed region (GPU still cool); frac above is the sustained figure of "
-                                 "the >= 1 s region, see `clocks`"}
     if three_term:
         roofline["three_term_recursion"] = three_term
     if plain is not None:
@@ -687,7 +699,7 @@ def run_ours(args):
         # weak scaling: every GPU advances its own 8-column job, the job count adds up; strong scaling:
         # one job of --total-cols columns, a step is done when every shard has done it
         "metric": METRIC, "value": jobs * head["steps"] / (head["total_ms"] * 1e-3), "unit": UNIT, "n_gpus": world, "steps": K,
-        "warmup": W, "repeats": head["repeats"], "timed_steps": head["steps"], "timed_s": head["total_ms"] * 1e-3,
+        "warmup": W, "timed_steps": head["steps"], "timed_s": head["total_ms"] * 1e-3,
         "ms_per_step": head["total_ms"] / head["steps"], "higher_is_better": True, "scaling": scaling, "vs_baseline": None,
         "dtype": "f64", "data": "synthetic",
         "config": workload_config(args.config, cfg, n_sites, head["n_blocks"], cols),

@@ -7,14 +7,23 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+import pytest
+
+from util import rel_err
+
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-def run_reference_arm(extra_env=None):
+def run_bench(*args, extra_env=None):
     env = {k: v for k, v in os.environ.items() if k not in ("RANK", "LOCAL_RANK", "WORLD_SIZE")}
     env.update(extra_env or {})
-    return subprocess.run([sys.executable, os.path.join(REPO, "bench.py"), "--impl", "reference", "--config", "C2",
-                           "--steps", "2", "--warmup", "1"], capture_output=True, text=True, env=env, cwd=REPO, timeout=300)
+    return subprocess.run([sys.executable, os.path.join(REPO, "bench.py"), *args], capture_output=True, text=True, env=env,
+                          cwd=REPO, timeout=300)
+
+
+def run_reference_arm(extra_env=None):
+    return run_bench("--impl", "reference", "--config", "C2", "--steps", "2", "--warmup", "1", extra_env=extra_env)
 
 
 def test_reference_arm_prints_one_contract_line():
@@ -37,3 +46,29 @@ def test_reference_arm_prints_one_contract_line():
 def test_reference_arm_is_silent_on_other_ranks():
     out = run_reference_arm({"RANK": "1", "LOCAL_RANK": "1", "WORLD_SIZE": "2"})
     assert out.returncode == 0 and out.stdout.strip() == "", out.stdout + out.stderr[-2000:]
+
+
+@pytest.mark.gpu
+def test_steps_sets_the_timed_steps_and_dump_holds_the_moments(gpu_api, tmp_path):
+    """``--steps K`` times K steps (K + 1 when an odd K meets a kernel that advances two steps per launch), and
+    ``--dump-outputs`` writes the moments of that recursion: those chebyshev_moments returns for the same matrix, seed and
+    scale."""
+    from bodge_b200 import workloads
+
+    K, W = 7, 3
+    out = run_bench("--config", "C2", "--steps", str(K), "--warmup", str(W), "--no-cpu-baseline", "--no-e2e", "--no-plain",
+                    "--dump-outputs", str(tmp_path))
+    assert out.returncode == 0, out.stderr[-2000:]
+    line = json.loads(out.stdout)
+    assert line["steps"] == K
+    assert line["timed_steps"] == (K + 1 if line["run"]["kernel"] == "t2" else K)
+    mu = np.load(tmp_path / "moments.npy")
+    summed = np.load(tmp_path / "moments_summed.npy")
+    assert mu.dtype == summed.dtype == np.float64 and mu.shape[1] == 8
+    assert np.array_equal(np.load(tmp_path / "moment_index.npy"), np.arange(len(mu), dtype=np.float64))
+    cfg = workloads.CONFIGS["C2"]
+    system = gpu_api.Hamiltonian(gpu_api.CubicLattice(cfg["shape"]), device=0)
+    system.fill(*cfg["build"](cfg["shape"]))
+    want = system.chebyshev_moments(len(mu), vectors=8, seed=1234, scale=system.spectral_bound(), kernel="auto_moments")
+    assert rel_err(mu, want) <= 1e-12
+    assert rel_err(summed, want.sum(axis=1)) <= 1e-12
