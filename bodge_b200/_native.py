@@ -66,6 +66,8 @@ SIGNATURES = {
     "bdg_cheb_end": [_vp],
     "bdg_kpm_resolvent": [_vp, C.c_int32, C.c_int32, _vp, _vp, _vp, C.c_int],
     "bdg_kpm_contract": [_vp, C.c_int32, _vp, C.c_int, _vp, C.c_int],
+    "bdg_cheb_local_begin": [_vp, C.c_int32, _vp, C.c_int64, _vp, _vp],
+    "bdg_cheb_local_read": [_vp, _vp, C.c_int],
 }
 
 _lib = None
@@ -401,3 +403,22 @@ class System:
         out = np.empty(1 if summed else n_cols, dtype=np.float64)
         check(load().bdg_kpm_contract(self._h, len(coef), _ptr(coef), int(summed), _ptr(out), 0))
         return float(out[0]) if summed else out
+
+    def cheb_local_begin(self, coef, cols, sites):
+        """Register the local accumulator on the active recursion (``bdg_cheb_local_begin``): series ``coef``, reads
+        ``(cols[r], sites[r])``.  Adds the ``T_0`` and ``T_1`` terms; the rest arrive with ``cheb_steps``."""
+        coef = _as(coef, np.float64)
+        cols, sites = _as_index(cols, "column index"), _as_index(sites)
+        if coef.ndim != 1 or cols.shape != sites.shape or cols.ndim != 1:
+            raise ValueError("coef, cols and sites must be 1-D, cols and sites of equal length")
+        check(load().bdg_cheb_local_begin(self._h, len(coef), _ptr(coef), len(cols), _ptr(cols), _ptr(sites)))
+
+    def cheb_local_read(self, n_reads: int, device_ptr: int | None = None):
+        """The accumulated ``[n_reads, 4]`` complex values; with ``device_ptr`` they are written to that device address
+        instead (``n_reads * 64`` bytes) and ``None`` is returned."""
+        if device_ptr is not None:
+            check(load().bdg_cheb_local_read(self._h, _vp(device_ptr), 1))
+            return None
+        out = np.empty((n_reads, 4), dtype=np.complex128)
+        check(load().bdg_cheb_local_read(self._h, _ptr(out), 0))
+        return out

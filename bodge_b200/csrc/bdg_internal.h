@@ -138,6 +138,13 @@ struct ChebState {
     int n_groups = 0;
     RowWalk walk;              // ELL / DICT kernels: row traversal
     int64_t launches = 0;
+    // Local accumulator (bdg_cheb_local_begin, observables.cu): every launch that writes T_n with n < local_coef.size()
+    // adds local_coef[n] * T_n[4 site + alpha][col] to local_acc[read][alpha].  Cleared by bdg_cheb_begin.
+    bool local = false;
+    std::vector<double> local_coef;
+    int64_t local_reads = 0;
+    DevBuf local_off;  // int64 [n_reads]: element offset of (site, col, alpha = 0) in the panel layout
+    DevBuf local_acc;  // double2 [n_reads][4]
 };
 
 // Kernel-native copy of the packed matrix for the ELL step kernel (cheb_ell.cu): every block row
@@ -219,6 +226,10 @@ int ensure_scratch(bdg_system *sys, int which, size_t bytes);
 void cheb_release(bdg_system *sys);     // free all Chebyshev buffers
 void cheb_deactivate(bdg_system *sys);  // matrix changed: recursion state is stale, keep buffers
 int t2_finish_dots(bdg_system *sys);    // T2 mode: dot rows -> single-step format (call before reading st.dots)
+
+// observables.cu
+// Local accumulator: add the terms of T_n (vector x_a) and T_{n+1} (x_b, may be null) that fall inside the series.
+int local_accumulate(bdg_system *sys, int n, const void *x_a, const void *x_b);
 
 // cheb_ell.cu
 int ell_build(bdg_system *sys);                    // (re)build sys->ell from sys->packed when stale

@@ -445,7 +445,7 @@ int launch_step(bdg_system *sys, bool first) {
         BDG_TRY(ell_launch_step(sys, first, x_cur, x_io, dots_step));
         std::swap(st.cur, st.prev);
         st.launches += 1;
-        return BDG_OK;
+        return local_accumulate(sys, slot + 1, x_io, nullptr);
     }
     const int rows_per_cta = st.kernel == BDG_KERNEL_DMMA_CHUNKED ? (int)ceil_div(m.n_sites, st.grid_x) : 0;
     StepKernel k = pick_kernel(st.kernel, st.panel_width, first, sys->packed_max_row);
@@ -457,7 +457,7 @@ int launch_step(bdg_system *sys, bool first) {
     BDG_CUDA(cudaGetLastError());
     std::swap(st.cur, st.prev);
     st.launches += 1;
-    return BDG_OK;
+    return local_accumulate(sys, slot + 1, x_io, nullptr);  // x_io now holds T_{slot+1}
 }
 
 // Two steps in one launch (cheb_pair.cu): T_{n+1}, T_{n+2} go to the two buffers holding neither
@@ -474,7 +474,7 @@ int launch_pair(bdg_system *sys) {
     st.prev = out[0];
     st.cur = out[1];
     st.launches += 1;
-    return BDG_OK;
+    return local_accumulate(sys, slot + 1, st.vec[out[0]].ptr, st.vec[out[1]].ptr);  // T_{slot+1}, T_{slot+2}
 }
 
 int ensure_dot_capacity(bdg_system *sys, int steps_total) {
@@ -527,6 +527,8 @@ void cheb_release(bdg_system *sys) {
     dev_free(sys, st.mu_tmp);
     dev_free(sys, st.obs_tmp);
     dev_free(sys, st.work_items);
+    dev_free(sys, st.local_off);
+    dev_free(sys, st.local_acc);
     ell_release(sys);
     const int64_t launches = st.launches;
     st = ChebState();
@@ -616,6 +618,7 @@ extern "C" int bdg_cheb_begin(bdg_t *sys, int kind, int32_t n_cols, const int64_
     st.t2 = t2;
     st.cube = cube;
     st.t2_rows_normalized = 0;
+    st.local = false;
     st.dot_capacity = (int)(st.dots.bytes / ((size_t)2 * st.n_panels * st.panel_width * sizeof(double)));
 
     // Grid: enough CTAs to fill every SM at the kernel's occupancy, split over panels; each CTA

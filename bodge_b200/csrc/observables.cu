@@ -54,6 +54,27 @@ kpm_contract(const double *__restrict__ dots, int n_moments, int n_cols, int str
     if (lane == 0) out[c] = s;
 }
 
+// acc[r][alpha] += ca * x_a[off[r] + alpha] (+ cb * x_b[...]): one thread per (read, alpha), each owning its
+// accumulator element, so the sum runs in the order of n on every configuration.  Off-diagonal elements
+// <e_row| T_n |x_c> have no moment doubling: every term is read from its own vector.
+__global__ void __launch_bounds__(kObsThreads)
+local_accumulate_kernel(const double2 *__restrict__ x_a, const double2 *__restrict__ x_b, double ca, double cb,
+                        const int64_t *__restrict__ off, int64_t n_reads, double2 *__restrict__ acc) {
+    const int64_t t = (int64_t)blockIdx.x * kObsThreads + threadIdx.x;
+    if (t >= 4 * n_reads) return;
+    const int64_t o = off[t >> 2] + (t & 3);
+    double2 s = acc[t];
+    const double2 a = x_a[o];
+    s.x += ca * a.x;
+    s.y += ca * a.y;
+    if (x_b) {
+        const double2 b = x_b[o];
+        s.x += cb * b.x;
+        s.y += cb * b.y;
+    }
+    acc[t] = s;
+}
+
 __global__ void sum_columns(const double *__restrict__ in, int n, double *__restrict__ out) {
     // single warp, fixed order
     double s = 0.0;
@@ -130,6 +151,65 @@ extern "C" int bdg_kpm_contract(bdg_t *sys, int32_t n_moments, const double *coe
     }
     if (!out_on_device)
         BDG_CUDA(cudaMemcpyAsync(out, src, n_out * sizeof(double), cudaMemcpyDeviceToHost, sys->stream));
+    BDG_CUDA(cudaStreamSynchronize(sys->stream));
+    return BDG_OK;
+}
+
+int local_accumulate(bdg_system *sys, int n, const void *x_a, const void *x_b) {
+    ChebState &st = sys->cheb;
+    const int n_coef = (int)st.local_coef.size();
+    if (!st.local || n >= n_coef) return BDG_OK;
+    const bool second = x_b && n + 1 < n_coef;
+    local_accumulate_kernel<<<(unsigned)ceil_div(4 * st.local_reads, kObsThreads), kObsThreads, 0, sys->stream>>>(
+        static_cast<const double2 *>(x_a), second ? static_cast<const double2 *>(x_b) : nullptr, st.local_coef[n],
+        second ? st.local_coef[n + 1] : 0.0, st.local_off.as<int64_t>(), st.local_reads, st.local_acc.as<double2>());
+    BDG_CUDA(cudaGetLastError());
+    st.launches += 1;
+    return BDG_OK;
+}
+
+extern "C" int bdg_cheb_local_begin(bdg_t *sys, int32_t n_coef, const double *coef, int64_t n_reads, const int32_t *read_col,
+                                    const int32_t *read_site) {
+    BDG_ENTER(sys);
+    ChebState &st = sys->cheb;
+    BDG_REQUIRE(st.active, "bdg_cheb_begin has not been called");
+    BDG_REQUIRE(!st.t2,
+                "the even-vector recursion (kernel T2) keeps only every second Chebyshev vector, so it cannot accumulate "
+                "local matrix elements of a series: begin the recursion with the pair or a single-step kernel");
+    BDG_REQUIRE(st.steps_done == 0, "register the local accumulator right after bdg_cheb_begin (%d steps already taken)",
+                st.steps_done);
+    BDG_REQUIRE(n_coef >= 1 && coef, "need at least one coefficient");
+    BDG_REQUIRE(n_reads >= 1 && read_col && read_site, "need at least one read");
+    const int64_t n_sites = sys->packed.n_sites;
+    const int pw = st.panel_width;
+    std::vector<int64_t> off((size_t)n_reads);
+    for (int64_t r = 0; r < n_reads; ++r) {
+        const int32_t c = read_col[r], s = read_site[r];
+        BDG_REQUIRE(c >= 0 && c < st.n_cols, "read %lld: column %d outside [0, %d)", (long long)r, c, st.n_cols);
+        BDG_REQUIRE(s >= 0 && s < n_sites, "read %lld: site %d outside [0, %lld)", (long long)r, s, (long long)n_sites);
+        off[(size_t)r] = (((int64_t)(c / pw) * n_sites + s) * pw + c % pw) * 4;
+    }
+    BDG_TRY(dev_alloc(sys, st.local_off, (size_t)n_reads * sizeof(int64_t)));
+    BDG_TRY(dev_alloc(sys, st.local_acc, (size_t)n_reads * 4 * sizeof(double2)));
+    BDG_CUDA(cudaMemcpyAsync(st.local_off.ptr, off.data(), (size_t)n_reads * sizeof(int64_t), cudaMemcpyHostToDevice,
+                             sys->stream));
+    BDG_CUDA(cudaMemsetAsync(st.local_acc.ptr, 0, (size_t)n_reads * 4 * sizeof(double2), sys->stream));
+    st.local_coef.assign(coef, coef + n_coef);
+    st.local_reads = n_reads;
+    st.local = true;
+    // T_0 is still in vec[prev], T_1 in vec[cur] (bdg_cheb_begin took the first step)
+    BDG_TRY(local_accumulate(sys, 0, st.vec[st.prev].ptr, st.vec[st.cur].ptr));
+    BDG_CUDA(cudaStreamSynchronize(sys->stream));  // `off` is a local of this call
+    return BDG_OK;
+}
+
+extern "C" int bdg_cheb_local_read(bdg_t *sys, double *out, int out_on_device) {
+    BDG_ENTER(sys);
+    ChebState &st = sys->cheb;
+    BDG_REQUIRE(st.active && st.local, "no local accumulator on an active recursion (bdg_cheb_local_begin)");
+    BDG_REQUIRE(out, "null output");
+    BDG_CUDA(cudaMemcpyAsync(out, st.local_acc.ptr, (size_t)st.local_reads * 4 * sizeof(double2),
+                             out_on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, sys->stream));
     BDG_CUDA(cudaStreamSynchronize(sys->stream));
     return BDG_OK;
 }

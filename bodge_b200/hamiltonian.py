@@ -277,11 +277,15 @@ class Hamiltonian:
                              rows=rows, vectors=vectors, seed=seed, scale=scale, kernel=kernel, batch=batch, group=group)
 
     def _columns(self, moments, read, summed, *, rows=None, vectors=None, seed=1234, scale=None, kernel="auto",
-                 batch=None, group="auto"):
+                 batch=None, group="auto", begin=None):
         """Run the recursion for ``moments`` moments over all start columns -- sharded over the
         ranks of the process group, in batches on this GPU -- and reduce each batch ON THE DEVICE
         with ``read(system, n_columns)``, which returns ``[m, n_columns]`` (per column) or ``[m]``
-        (``summed``).  One collective combines the ranks."""
+        (``summed``).  One collective combines the ranks.
+
+        ``begin(system, c0, c1)`` is called after each batch's ``cheb_begin`` with the batch's columns ``[c0, c1)`` of
+        the full list, to register a local accumulator.  ``moments`` is then the length of a series without moment
+        doubling (``moments - 1`` steps), and ``kernel="auto"`` stays on kernels that keep every vector."""
         if (rows is None) == (vectors is None):
             raise ValueError("give either rows= (probe columns) or vectors= (random columns)")
         scale = self.spectral_bound() if scale is None else float(scale)
@@ -292,8 +296,8 @@ class Hamiltonian:
         n_local = hi - lo
         if batch is None:  # two vector sets of 64*N*k bytes each (four with the pair kernel); keep two under ~16 GB
             batch = max(8, int(8e9 // (64 * self.lattice.size)) // 8 * 8)
-        steps = (moments + 1) // 2 - 1
-        if kernel == "auto":   # only moments are read here: the library may keep every second vector only
+        steps = (moments + 1) // 2 - 1 if begin is None else moments - 1
+        if kernel == "auto" and begin is None:   # only moments are read here: the library may keep every second vector only
             kernel = "auto_moments"
         parts = []
         for b0 in range(0, n_local, batch):
@@ -302,6 +306,8 @@ class Hamiltonian:
                 self._sys.cheb_begin(probe_rows=rows[lo + b0 : lo + b1], scale=scale, kernel=kernel)
             else:
                 self._sys.cheb_begin(n_random=b1 - b0, seed=seed, col_offset=lo + b0, scale=scale, kernel=kernel)
+            if begin is not None:
+                begin(self._sys, lo + b0, lo + b1)
             done = self._sys.cheb_available() // 2 - 1      # steps bdg_cheb_begin has already taken (1 with T2)
             self._sys.cheb_steps(max(0, steps - done))
             parts.append(np.asarray(read(self._sys, b1 - b0), dtype=np.float64))
@@ -478,3 +484,137 @@ class Hamiltonian:
         out = self._columns(moments, read, False, rows=self._probe_rows(sites), scale=scale, kernel=kernel)
         g_imag = out[len(eps):].T.reshape(len(sites), 4, len(eps))  # Im G[site, α, ε]
         return kpm.ldos_from_resolvent(g_imag, eps, energies)
+
+    # ------------------------------------------------------------------------------------
+    # expectation values: local elements of the Fermi function f(H) (no reference code; the reference
+    # would need diagonalize(), a dense O((4N)^3) eigensolver)
+    # ------------------------------------------------------------------------------------
+    def _flat(self, coords) -> np.ndarray:
+        return np.array([self.lattice[tuple(int(v) for v in c)] for c in coords], dtype=np.int64)
+
+    def _fermi_local(self, temperature, rows, read_col, read_site, *, moments=None, scale=None, tol=1e-13,
+                     kernel="auto", batch=None, caller="density_matrix"):
+        """``acc[r, α] = f(H)[4 read_site[r] + α, rows[read_col[r]]]`` as complex ``[n_reads, 4]``: one probe column
+        per entry of ``rows``, the Fermi series contracted on the device while the recursion runs (``bdg.h``:
+        ``bdg_cheb_local_begin``).  Columns are batched and sharded like every other observable; the reads of a batch
+        land in their slots of one ``[n_reads, 4]`` array, so the ranks combine with a plain sum."""
+        T = float(temperature)
+        if not T > 0:
+            raise ValueError(f"{caller} needs a temperature T > 0 (the Fermi function at T = 0 is a step function)")
+        rows = np.asarray(rows, dtype=np.int64)
+        read_col = np.asarray(read_col, dtype=np.int64)
+        read_site = np.asarray(read_site, dtype=np.int64)
+        n_reads = len(read_col)
+        scale = self.spectral_bound() if scale is None else float(scale)
+        if scale == 0.0:  # H = 0: f(H) = f(0) 1 = 1/2
+            alpha = 4 * read_site[:, None] + np.arange(4)
+            return np.where(alpha == rows[read_col][:, None], 0.5, 0.0).astype(np.complex128)
+        need, reached = kpm.free_energy_moments(T, scale, tol)
+        n_coef = need if moments is None else int(moments)
+        if n_coef < need or reached > tol:
+            level = max(reached, kpm.series_error(n_coef, np.pi * T / scale))
+            warnings.warn(f"{caller}: {n_coef} moments at T = {T:g}, scale = {scale:.3g} truncate the Fermi series at "
+                          f"~{level:.1e} relative (tol = {tol:g} needs {int(np.ceil(-np.log(tol) * scale / (np.pi * T)))})",
+                          AccuracyWarning, stacklevel=3)
+        coef = kpm.fermi_coefficients(T, n_coef, scale)
+        batch_reads = []
+
+        def begin(sysn, c0, c1):
+            mine = np.flatnonzero((read_col >= c0) & (read_col < c1))
+            batch_reads.append(mine)
+            if len(mine):
+                sysn.cheb_local_begin(coef, read_col[mine] - c0, read_site[mine])
+
+        def read(sysn, k):
+            full = np.zeros((n_reads, 4), dtype=np.complex128)
+            mine = batch_reads[-1]
+            if len(mine):
+                full[mine] = sysn.cheb_local_read(len(mine))
+            return full.view(np.float64).ravel()
+
+        read.leading_dim = 8 * n_reads
+        total = self._columns(n_coef, read, True, rows=rows, scale=scale, kernel=kernel, batch=batch, begin=begin)
+        return np.ascontiguousarray(total, dtype=np.float64).view(np.complex128).reshape(n_reads, 4)
+
+    def density_matrix(self, temperature: float, pairs, *, moments: int | None = None, scale: float | None = None,
+                       tol: float = 1e-13, kernel: str = "auto", batch: int | None = None) -> Matrix:
+        """Blocks of the one-body density matrix ``ρ = f(H)``, ``f(ε) = 1/(1 + e^{ε/T})``: complex
+        ``[len(pairs), 4, 4]`` with ``result[p] = f(H)[4i:4i+4, 4j:4j+4]`` for ``pairs[p] = (i, j)`` (coordinates, like
+        ``H[i, j]`` keys; basis e↑, e↓, h↑, h↓).  With the Nambu spinor ``Ψ = (c↑, c↓, c↑†, c↓†)``,
+        ``<Ψ_a Ψ_b†> = δ_ab - ρ_ab``: e.g. ``<c_i↑ c_i↓> = -ρ[4i, 4i+3]``.
+
+        A pair must be on-site or a block of the lattice's skeleton (``IndexError`` otherwise, like ``index()``);
+        coordinates outside the lattice raise ``ValueError``.  The four scalar rows of every distinct ``j`` are probe
+        columns of one Chebyshev recursion of ``f`` (no damping kernel: ``f`` is analytic for T > 0); the blocks are
+        read at the requested ``i`` while it runs, on the GPU.  ``moments=None`` takes the series length for a relative
+        truncation error ``tol``, the rule of ``free_energy`` (capped at 32768 terms); an explicit ``moments`` below
+        that, or the cap, raise an ``AccuracyWarning``.  The series has no moment doubling: ``moments - 1`` steps.
+        ``kernel="auto"`` runs the pair or a single-step kernel (the even-vector ``"t2"`` keeps every second vector
+        only and is refused).  T <= 0 raises ``ValueError``."""
+        pairs = list(pairs)
+        i = self._flat([p[0] for p in pairs])
+        j = self._flat([p[1] for p in pairs])
+        off = i != j
+        if off.any():
+            self._sys.lookup(i[off], j[off])  # IndexError for a pair that is no block of the skeleton
+        uj, pos = np.unique(j, return_inverse=True)
+        rows = (4 * uj[:, None] + np.arange(4)).ravel()
+        read_col = (4 * pos[:, None] + np.arange(4)).ravel()  # read 4p + β: column (j_p, β) at site i_p
+        read_site = np.repeat(i, 4)
+        acc = self._fermi_local(temperature, rows, read_col, read_site, moments=moments, scale=scale, tol=tol,
+                                kernel=kernel, batch=batch, caller="density_matrix")
+        return acc.reshape(len(pairs), 4, 4).transpose(0, 2, 1).copy()  # acc[4p + β, α] -> [p, α, β]
+
+    def _potential(self, potential, sites):
+        """``(coordinates, flat indices, V)`` of the sites an order parameter is asked for."""
+        if isinstance(potential, dict):
+            table = {int(k): float(v) for k, v in zip(self._flat(list(potential)), potential.values())}
+        else:
+            table = None
+        if sites is None:
+            sites = [s for s in self.lattice.sites()
+                     if (table.get(self.lattice[s], 0.0) if table is not None else float(potential)) != 0.0]
+        sites = [tuple(int(v) for v in s) for s in sites]
+        flat = self._flat(sites)
+        V = np.array([table.get(int(k), 0.0) for k in flat] if table is not None else np.full(len(flat), float(potential)))
+        return sites, flat, V
+
+    def order_parameter(self, temperature: float, potential, sites=None, **kpm_options) -> Matrix:
+        """Mean-field s-wave order parameter ``Δ_i = -V_i ρ[4i, 4i+3]`` (complex, one per site) of an on-site attraction
+        ``-V_i n_i↑ n_i↓``; ``Δ[i, i] = Δ_i jσ2`` is the pairing entry that reproduces it (``Δ[i, i] = -Δs jσ2`` is
+        ``Δ_i = -Δs``).  It makes ``F + Σ_i |Δ_i|²/V_i`` stationary, with ``F`` from ``free_energy``.
+
+        ``potential``: one ``V`` for every site, or a ``{site: V}`` dict; ``sites`` defaults to every site with
+        ``V_i != 0``.  One probe column per site (row ``4i+3``) and one read, a quarter of ``density_matrix``'s work
+        for the same sites.  ``kpm_options``: ``moments``, ``scale``, ``tol``, ``kernel``, ``batch`` as there."""
+        sites, flat, V = self._potential(potential, sites)
+        if len(flat) == 0:
+            return np.zeros(0, dtype=np.complex128)
+        acc = self._fermi_local(temperature, 4 * flat + 3, np.arange(len(flat)), flat, caller="order_parameter",
+                                **kpm_options)
+        return -V * acc[:, 0]
+
+    def selfconsistent(self, temperature: float, potential, *, tol: float = 1e-8, max_iter: int = 500,
+                       mixing: float = 1.0, **kpm_options) -> tuple[Matrix, int]:
+        """Solve the s-wave gap equation ``Δ_i = -V_i ρ[4i, 4i+3]`` by plain fixed-point iteration: compute ``Δ``
+        (``order_parameter``), write ``Δ[i, i] = Δ_i jσ2`` back (pairing entries only: the hopping stays), repeat until
+        ``max_i |Δ_i^new - Δ_i| <= tol``.  ``mixing`` < 1 moves only that fraction of the way per iteration.  Starts
+        from the pairing the system holds (set a non-zero guess: ``Δ = 0`` is always a fixed point) and leaves the
+        last state in it.  Each iteration rewrites N of the ~5N blocks of a square lattice, which the library patches
+        into its copies of the matrix in place.  Returns ``(Δ, iterations)``; warns if ``max_iter`` is reached."""
+        if not 0 < mixing <= 1:
+            raise ValueError("mixing must be in (0, 1]")
+        sites, flat, V = self._potential(potential, None)
+        if len(flat) == 0:
+            return np.zeros(0, dtype=np.complex128), 0
+        delta = self._sys.export_bsr(False)[2][self._sys.lookup(flat, flat), 0, 3]
+        for it in range(1, int(max_iter) + 1):
+            new = self.order_parameter(temperature, potential, sites, **kpm_options)
+            step = np.max(np.abs(new - delta))
+            delta = delta + mixing * (new - delta)
+            self.fill((), (), (), flat, flat, delta[:, None, None] * jσ2)
+            if step <= tol:
+                return delta, it
+        warnings.warn(f"selfconsistent: no convergence in {max_iter} iterations (last change {step:.2e} > tol = {tol:g})",
+                      AccuracyWarning, stacklevel=2)
+        return delta, int(max_iter)

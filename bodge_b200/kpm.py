@@ -18,6 +18,7 @@ import math
 
 import numpy as np
 from scipy.fft import dct
+from scipy.special import expit
 
 
 def free_energy_density(eps, temperature: float):
@@ -39,6 +40,15 @@ def chebyshev_coefficients(func, n_coef: int, scale: float) -> np.ndarray:
     coef = dct(samples, type=2)[:n_coef] / nodes
     coef[0] /= 2
     return coef
+
+
+def fermi_coefficients(temperature: float, n_coef: int, scale: float) -> np.ndarray:
+    """Coefficients ``c_n`` of the Fermi function ``f(ε) = 1/(1 + e^{ε/T})`` in ``f(scale * x) = sum_n c_n T_n(x)``, the
+    series behind ``Hamiltonian.density_matrix``.  Like ``g`` of the free energy, ``f`` has its nearest poles at
+    ``±iπT``, so ``free_energy_moments`` gives the length for a truncation error ``tol``.  T must be positive."""
+    if not temperature > 0:
+        raise ValueError("the Fermi function needs a temperature T > 0")
+    return chebyshev_coefficients(lambda e: expit(-e / temperature), n_coef, scale)
 
 
 def free_energy_from_trace(mu_trace, temperature: float, scale: float) -> float:

@@ -219,6 +219,21 @@ int bdg_kpm_resolvent(bdg_t *sys, int32_t n_moments, int32_t n_z, const double *
  * (BDG_MU_SUM, one double): e.g. coef = Chebyshev coefficients of the free-energy density. */
 int bdg_kpm_contract(bdg_t *sys, int32_t n_moments, const double *coef, int reduce, double *out,
                      int out_on_device);
+/* Local accumulator: off-diagonal elements of a matrix function, f(H~) ~ sum_n coef[n] T_n(H~), read while the recursion
+ * runs.  Register it right after bdg_cheb_begin with the series coef[0 .. n_coef) and a list of reads (column
+ * read_col[r] < n_cols of this recursion, row site read_site[r]); it adds the T_0 and T_1 terms at once, and from then on
+ * every launch that writes T_n with n < n_coef adds
+ *     acc[r][alpha] += coef[n] * T_n[4 * read_site[r] + alpha][read_col[r]],   alpha = 0..3 (complex),
+ * one small kernel per launch (4 * n_reads scattered 16-byte loads) next to the unchanged step kernels.  With probe
+ * columns x_c = e_q this is acc[r][alpha] = f(H~)[4 site + alpha, q].  There is no moment doubling: the full series needs
+ * n_coef - 1 steps (bdg_cheb_steps).  Works with the PAIR and single-step kernels (AUTO, DICT_DIAG, DICT, ELL, DMMA,
+ * FMA); the even-vector recursion (T2, also what AUTO_MOMENTS may choose) does not keep the odd vectors and is refused
+ * with BDG_E_INVALID.  bdg_cheb_begin discards the accumulator. */
+int bdg_cheb_local_begin(bdg_t *sys, int32_t n_coef, const double *coef, int64_t n_reads, const int32_t *read_col,
+                         const int32_t *read_site);
+/* out[r][alpha] = acc[r][alpha] as complex (interleaved re, im: n_reads * 8 doubles); out_on_device != 0: out is a device
+ * pointer on this handle's GPU (e.g. for an NCCL reduce over column shards). */
+int bdg_cheb_local_read(bdg_t *sys, double *out, int out_on_device);
 
 #ifdef __cplusplus
 }
