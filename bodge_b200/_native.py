@@ -20,8 +20,8 @@ OK, E_INVALID, E_CUDA, E_NOT_NEIGHBOUR, E_NOT_HERMITIAN, E_OUT_OF_BOUNDS, E_NO_D
 X0_PROBE, X0_RADEMACHER = 0, 1
 MU_PER_COLUMN, MU_SUM = 0, 1
 KERNEL_AUTO, KERNEL_DMMA, KERNEL_FMA = 0, 1, 2
-KERNELS = {"auto": KERNEL_AUTO, "dmma": KERNEL_DMMA, "fma": KERNEL_FMA, "ell": 3, "dmma_simple": 4, "dmma_chunked": 5,
-           "dict": 6, "dict_diag": 7, "pair": 8, "t2": 9, "auto_moments": 10}
+KERNELS = {"auto": KERNEL_AUTO, "dmma": KERNEL_DMMA, "fma": KERNEL_FMA, "ell": 3, "dict": 6, "dict_diag": 7, "pair": 8, "t2": 9,
+           "auto_moments": 10}
 KERNEL_NAMES = {v: k for k, v in KERNELS.items()}
 
 _i32p = C.POINTER(C.c_int32)

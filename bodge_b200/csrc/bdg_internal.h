@@ -3,6 +3,7 @@
 
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <stdlib.h>
 
 #include <string>
 #include <vector>
@@ -134,7 +135,6 @@ struct ChebState {
     DevBuf work_items;  // work lists of the two-step kernel (PairWalk)
     int grid_x = 0;
     int panels_per_group = 1;  // ELL kernel: panels sharing one pass over the matrix (grid.y = groups)
-    int panel_batch = 1;       // ... of which this many have their loads in flight together
     int n_groups = 0;
     RowWalk walk;              // ELL / DICT kernels: row traversal
     int64_t launches = 0;
@@ -254,3 +254,9 @@ int cube_configure(bdg_system *sys);  // patch shape / segment plan and grid for
 int cube_launch(bdg_system *sys, bool first, const void *x_cur, void *x_io, double *dots_step);
 
 static inline int64_t ceil_div(int64_t a, int64_t b) { return (a + b - 1) / b; }
+
+// Integer switch from the environment (plan and kernel overrides, INTEGRATION.md); unset or empty: `fallback`.
+static inline int env_int(const char *name, int fallback) {
+    const char *v = getenv(name);
+    return v && *v ? atoi(v) : fallback;
+}

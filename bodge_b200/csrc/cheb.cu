@@ -51,7 +51,7 @@ template <int PW, bool FIRST, int CH>
 __global__ void __launch_bounds__(kThreads, 4)
 cheb_step_dmma(const int32_t *__restrict__ indptr, const int32_t *__restrict__ indices,
                const double2 *__restrict__ data, const double2 *__restrict__ x_cur, double2 *__restrict__ x_io,
-               int n_sites, int rows_per_cta, double alpha, double beta, double *__restrict__ partials,
+               int n_sites, double alpha, double beta, double *__restrict__ partials,
                unsigned *__restrict__ tickets, double *__restrict__ dots_step, int n_panels) {
     constexpr int REC = PW * 4;  // complex elements per site record
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -62,7 +62,6 @@ cheb_step_dmma(const int32_t *__restrict__ indptr, const int32_t *__restrict__ i
     // rows (t * gridDim.x + b) * kWarps ... + kWarps - 1.  All SMs then touch one window of a few
     // thousand consecutive sites at a time, so the records of the +-Ly / +-LyLz neighbours (read
     // again one or two passes later) are still in L2 and every vector byte leaves HBM once.
-    (void)rows_per_cta;
     const int stride = gridDim.x * kWarps;
 
     // A-operand role: lanes 0-15 feed rows 0-3 of [[Br,-Bi],[Bi,Br]], lanes 16-31 rows 4-7.
@@ -160,80 +159,12 @@ cheb_step_dmma(const int32_t *__restrict__ indptr, const int32_t *__restrict__ i
     finish_dots<PW>(d0, d1, col, o_lane && a == 0, panel, n_panels, partials, tickets, dots_step);
 }
 
-// ---- unpipelined variant of the MMA formulation (tuning reference) ----------------------------
-template <int PW, bool FIRST>
-__global__ void __launch_bounds__(kThreads)
-cheb_step_dmma_simple(const int32_t *__restrict__ indptr, const int32_t *__restrict__ indices,
-                      const double2 *__restrict__ data, const double2 *__restrict__ x_cur,
-                      double2 *__restrict__ x_io, int n_sites, int rows_per_cta, double alpha, double beta,
-                      double *__restrict__ partials, unsigned *__restrict__ tickets, double *__restrict__ dots_step,
-                      int n_panels) {
-    constexpr int REC = PW * 4;
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int panel = blockIdx.y;
-    const double2 *__restrict__ xc = x_cur + (size_t)panel * n_sites * REC;
-    double2 *__restrict__ xo = x_io + (size_t)panel * n_sites * REC;
-    const int elem = lane & 15;
-    const bool hi = lane >= 16;
-    const bool x_lane = lane < REC;
-    const int a = (lane >> 2) & 3;
-    const int col = 2 * (lane & 3) + (lane >> 4);
-    const bool o_lane = col < PW;
-    const int o_elem = col * 4 + a;
-    // rows_per_cta > 0: every CTA walks its own contiguous range; == 0: wavefront traversal
-    const int row_first = rows_per_cta > 0 ? blockIdx.x * rows_per_cta + warp : blockIdx.x * kWarps + warp;
-    const int row_end = rows_per_cta > 0 ? min(n_sites, (int)(blockIdx.x + 1) * rows_per_cta) : n_sites;
-    const int stride = rows_per_cta > 0 ? kWarps : gridDim.x * kWarps;
-
-    double d0 = 0.0, d1 = 0.0;
-    for (int row = row_first; row < row_end; row += stride) {
-        const int p0 = indptr[row], p1 = indptr[row + 1];
-        double re0 = 0.0, re1 = 0.0, im0 = 0.0, im1 = 0.0;
-        for (int pb = p0; pb < p1; pb += 32) {
-            const int cnt = min(32, p1 - pb);
-            const int jv = lane < cnt ? indices[pb + lane] : 0;
-#pragma unroll 4
-            for (int t = 0; t < cnt; ++t) {
-                const int j = __shfl_sync(kFull, jv, t);
-                const double2 bv = __ldcs(data + (size_t)(pb + t) * 16 + elem);
-                double2 xv = make_double2(0.0, 0.0);
-                if (x_lane) xv = __ldg(xc + (size_t)j * REC + lane);
-                dmma_8x8x4(re0, re1, hi ? bv.y : bv.x, xv.x);
-                dmma_8x8x4(im0, im1, hi ? bv.x : -bv.y, xv.y);
-            }
-        }
-        const double c0 = re0 + im0, c1 = re1 + im1;
-        const double recv = __shfl_xor_sync(kFull, hi ? c0 : c1, 16);
-        const double yr = hi ? recv : c0;
-        const double yi = hi ? c1 : recv;
-        if (o_lane) {
-            const size_t off = (size_t)row * REC + o_elem;
-            const double2 tn = __ldg(xc + off);
-            double2 out;
-            if (FIRST) {
-                out = make_double2(alpha * yr, alpha * yi);
-            } else {
-                const double2 pv = xo[off];
-                out = make_double2(alpha * yr - beta * pv.x, alpha * yi - beta * pv.y);
-            }
-            xo[off] = out;
-            d0 += tn.x * tn.x + tn.y * tn.y;
-            d1 += out.x * tn.x + out.y * tn.y;
-        }
-    }
-    d0 += __shfl_xor_sync(kFull, d0, 4);
-    d1 += __shfl_xor_sync(kFull, d1, 4);
-    d0 += __shfl_xor_sync(kFull, d0, 8);
-    d1 += __shfl_xor_sync(kFull, d1, 8);
-    finish_dots<PW>(d0, d1, col, o_lane && a == 0, panel, n_panels, partials, tickets, dots_step);
-}
-
 // ---- the fused step: scalar FMA formulation (one thread per (site, column)) ----------------------
 template <int PW, bool FIRST>
 __global__ void __launch_bounds__(kThreads)
 cheb_step_fma(const int32_t *__restrict__ indptr, const int32_t *__restrict__ indices,
               const double2 *__restrict__ data, const double2 *__restrict__ x_cur, double2 *__restrict__ x_io,
-              int n_sites, int rows_per_cta, double alpha, double beta, double *__restrict__ partials,
+              int n_sites, double alpha, double beta, double *__restrict__ partials,
               unsigned *__restrict__ tickets, double *__restrict__ dots_step, int n_panels) {
     constexpr int REC = PW * 4;
     constexpr int ROWS_PER_WARP = 32 / PW;
@@ -241,7 +172,7 @@ cheb_step_fma(const int32_t *__restrict__ indptr, const int32_t *__restrict__ in
     const int panel = blockIdx.y;
     const double2 *__restrict__ xc = x_cur + (size_t)panel * n_sites * REC;
     double2 *__restrict__ xo = x_io + (size_t)panel * n_sites * REC;
-    (void)rows_per_cta;  // same wavefront traversal as cheb_step_dmma
+    // same wavefront traversal as cheb_step_dmma
     const int col = lane % PW, sub = lane / PW;
 
     double d0 = 0.0, d1 = 0.0;
@@ -400,13 +331,11 @@ unpack_vectors(const double2 *__restrict__ x, int n_sites, int pw, int n_cols, d
     out[t] = x[(((size_t)(c / pw) * n_sites + site) * pw + (c % pw)) * 4 + alpha];
 }
 
-using StepKernel = void (*)(const int32_t *, const int32_t *, const double2 *, const double2 *, double2 *, int, int,
-                            double, double, double *, unsigned *, double *, int);
+using StepKernel = void (*)(const int32_t *, const int32_t *, const double2 *, const double2 *, double2 *, int, double,
+                            double, double *, unsigned *, double *, int);
 
 template <int PW> StepKernel pick_pw(int kernel, bool first, int max_row) {
     if (kernel == BDG_KERNEL_FMA) return first ? cheb_step_fma<PW, true> : cheb_step_fma<PW, false>;
-    if (kernel == BDG_KERNEL_DMMA_SIMPLE || kernel == BDG_KERNEL_DMMA_CHUNKED)
-        return first ? cheb_step_dmma_simple<PW, true> : cheb_step_dmma_simple<PW, false>;
     if (max_row <= 3) return first ? cheb_step_dmma<PW, true, 3> : cheb_step_dmma<PW, false, 3>;
     if (max_row <= 5) return first ? cheb_step_dmma<PW, true, 5> : cheb_step_dmma<PW, false, 5>;
     if (max_row <= 7) return first ? cheb_step_dmma<PW, true, 7> : cheb_step_dmma<PW, false, 7>;
@@ -423,15 +352,9 @@ StepKernel pick_kernel(int kernel, int pw, bool first, int max_row) {
 }
 
 // AUTO prefers the two-steps-per-pass kernel wherever it applies (BDG_AUTO_PAIR=0 turns that off).
-bool auto_pair_enabled() {
-    const char *v = getenv("BDG_AUTO_PAIR");
-    return v && *v ? atoi(v) != 0 : kAutoPairDefault;
-}
+bool auto_pair_enabled() { return env_int("BDG_AUTO_PAIR", kAutoPairDefault) != 0; }
 // ... and, for callers that only read moments, the even-vector recursion on three-dimensional lattices (BDG_AUTO_CUBE=0: off)
-bool auto_cube_enabled() {
-    const char *v = getenv("BDG_AUTO_CUBE");
-    return v && *v ? atoi(v) != 0 : true;
-}
+bool auto_cube_enabled() { return env_int("BDG_AUTO_CUBE", 1) != 0; }
 
 int launch_step(bdg_system *sys, bool first) {
     ChebState &st = sys->cheb;
@@ -447,11 +370,10 @@ int launch_step(bdg_system *sys, bool first) {
         st.launches += 1;
         return local_accumulate(sys, slot + 1, x_io, nullptr);
     }
-    const int rows_per_cta = st.kernel == BDG_KERNEL_DMMA_CHUNKED ? (int)ceil_div(m.n_sites, st.grid_x) : 0;
     StepKernel k = pick_kernel(st.kernel, st.panel_width, first, sys->packed_max_row);
     dim3 grid((unsigned)st.grid_x, (unsigned)st.n_panels);
     k<<<grid, kThreads, 0, sys->stream>>>(m.indptr.as<int32_t>(), m.indices.as<int32_t>(), m.data.as<double2>(), x_cur,
-                                          x_io, (int)m.n_sites, rows_per_cta, (first ? 1.0 : 2.0) / st.scale,
+                                          x_io, (int)m.n_sites, (first ? 1.0 : 2.0) / st.scale,
                                           first ? 0.0 : 1.0, st.partials.as<double>(), st.tickets.as<unsigned>(),
                                           dots_step, st.n_panels);
     BDG_CUDA(cudaGetLastError());
@@ -546,7 +468,8 @@ extern "C" int bdg_cheb_begin(bdg_t *sys, int kind, int32_t n_cols, const int64_
     BDG_REQUIRE(n_cols >= 1, "need at least one column");
     BDG_REQUIRE(scale > 0.0, "scale must be positive");
     BDG_REQUIRE(kind != BDG_X0_PROBE || probe_rows != nullptr, "probe rows missing");
-    BDG_REQUIRE(kernel >= BDG_KERNEL_AUTO && kernel <= BDG_KERNEL_AUTO_MOMENTS, "unknown kernel %d", kernel);
+    BDG_REQUIRE(kernel >= BDG_KERNEL_AUTO && kernel <= BDG_KERNEL_AUTO_MOMENTS && kernel != 4 && kernel != 5,  // 4, 5: unassigned (bdg.h)
+                "unknown kernel %d", kernel);
     BDG_TRY(build_packed(sys));
     bool pair = false, t2 = false, cube = false;
     if (kernel == BDG_KERNEL_AUTO || kernel == BDG_KERNEL_ELL || kernel == BDG_KERNEL_DICT || kernel == BDG_KERNEL_DICT_DIAG ||

@@ -117,67 +117,6 @@ __device__ __forceinline__ void hop(const double2 &x, double b, double &yr, doub
     yi = fma(b, x.y, yi);
 }
 
-// The four dot products of a run (cheb_pair.cu: flush_dots) on 4-column panels: components -> site halves -> warp -> CTA ->
-// partials[run]; the last run of a panel (runs r0 .. r1) adds them up in run order.
-template <int NW>
-__device__ __forceinline__ void flush_dots4(double d0, double d1, double d2, double d3, unsigned char *scratch, int run, int r0, int r1,
-                                            int panel, int n_panels, double *__restrict__ partials, unsigned *__restrict__ tickets,
-                                            double *__restrict__ dots_step) {
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    __shared__ bool is_last;
-    d0 += __shfl_xor_sync(kFull, d0, 1);
-    d1 += __shfl_xor_sync(kFull, d1, 1);
-    d2 += __shfl_xor_sync(kFull, d2, 1);
-    d3 += __shfl_xor_sync(kFull, d3, 1);
-    d0 += __shfl_xor_sync(kFull, d0, 2);
-    d1 += __shfl_xor_sync(kFull, d1, 2);
-    d2 += __shfl_xor_sync(kFull, d2, 2);
-    d3 += __shfl_xor_sync(kFull, d3, 2);
-    d0 += __shfl_xor_sync(kFull, d0, 16);
-    d1 += __shfl_xor_sync(kFull, d1, 16);
-    d2 += __shfl_xor_sync(kFull, d2, 16);
-    d3 += __shfl_xor_sync(kFull, d3, 16);
-    __syncthreads();  // the rings are idle: reuse them as reduction scratch
-    double *red = reinterpret_cast<double *>(scratch);  // [NW][4 which][4 columns], then comb [NW][16]
-    double *comb = red + NW * 16;
-    if (lane < 16 && (lane & 3) == 0) {
-        const int col = lane >> 2;
-        red[(warp * 4 + 0) * 4 + col] = d0;
-        red[(warp * 4 + 1) * 4 + col] = d1;
-        red[(warp * 4 + 2) * 4 + col] = d2;
-        red[(warp * 4 + 3) * 4 + col] = d3;
-    }
-    __syncthreads();
-    if (threadIdx.x < 16) {
-        double s = 0.0;
-#pragma unroll
-        for (int w = 0; w < NW; ++w) s += red[w * 16 + threadIdx.x];
-        partials[(size_t)run * 16 + threadIdx.x] = s;
-    }
-    __threadfence();
-    __syncthreads();
-    if (threadIdx.x == 0) is_last = atomicAdd(&tickets[panel], 1u) == (unsigned)(r1 - r0 - 1);
-    __syncthreads();
-    if (is_last) {
-        __threadfence();
-        if (lane < 16) {
-            double s = 0.0;
-            for (int b = r0 + warp; b < r1; b += NW) s += __ldcg(&partials[(size_t)b * 16 + lane]);
-            comb[warp * 16 + lane] = s;
-        }
-        __syncthreads();
-        if (threadIdx.x < 16) {
-            double t = 0.0;
-#pragma unroll
-            for (int g = 0; g < NW; ++g) t += comb[g * 16 + threadIdx.x];
-            // slot = which * 4 + column; which = (a, c, b, d) as in cheb_pair.cu
-            dots_step[(size_t)(threadIdx.x >> 2) * n_panels * 4 + panel * 4 + (threadIdx.x & 3)] = t;
-        }
-        if (threadIdx.x == 0) tickets[panel] = 0u;
-    }
-    __syncthreads();  // scratch and is_last are free again
-}
-
 // NW warps, one CTA per SM.  Body lists (one body = two z-adjacent sites): [A] the u region = the patch and its halo
 // ring without the corners -- rows 0 and PY + 1 of the region hold PZ / 2 bodies, the PY rows between (PZ + 2) / 2 --,
 // [B] the PY x PZ / 2 owned bodies; body b goes to warp b % NW.  At PY = PZ = 8, NW = 16: 48 + 32 bodies, three + two per warp.
@@ -250,8 +189,8 @@ cheb_cube_step(const int32_t *__restrict__ dcode, const double *__restrict__ tab
             piece = wk.pieces[item];  // (run, patch, x0, len)
             if (piece.x != run) {
                 if (run >= 0) {
-                    flush_dots4<NW>(d0, d1, d2, d3, cube_smem, run, wk.panel_runs[panel], wk.panel_runs[panel + 1], panel, n_panels, partials,
-                                   tickets, dots_step);
+                    flush_dots<NW, 4>(d0, d1, d2, d3, cube_smem, run, wk.panel_runs[panel], wk.panel_runs[panel + 1], panel, n_panels, partials,
+                                      tickets, dots_step);
                     d0 = d1 = d2 = d3 = 0.0;
                 }
                 run = piece.x;
@@ -455,11 +394,11 @@ cheb_cube_step(const int32_t *__restrict__ dcode, const double *__restrict__ tab
 
     if (LISTED) {
         if (panel >= 0)
-            flush_dots4<NW>(d0, d1, d2, d3, cube_smem, run, wk.panel_runs[panel], wk.panel_runs[panel + 1], panel, n_panels, partials, tickets,
-                            dots_step);
+            flush_dots<NW, 4>(d0, d1, d2, d3, cube_smem, run, wk.panel_runs[panel], wk.panel_runs[panel + 1], panel, n_panels, partials, tickets,
+                              dots_step);
     } else {
         const int p = (int)blockIdx.y, r0 = p * (int)gridDim.x;
-        flush_dots4<NW>(d0, d1, d2, d3, cube_smem, r0 + (int)blockIdx.x, r0, r0 + (int)gridDim.x, p, n_panels, partials, tickets, dots_step);
+        flush_dots<NW, 4>(d0, d1, d2, d3, cube_smem, r0 + (int)blockIdx.x, r0, r0 + (int)gridDim.x, p, n_panels, partials, tickets, dots_step);
     }
 }
 
@@ -517,11 +456,6 @@ template <int NW, int PY, int PZ, int NE> CubeShape make_shape() {
     return s;
 }
 
-int cube_env(const char *name, int fallback) {
-    const char *v = getenv(name);
-    return v && *v ? atoi(v) : fallback;
-}
-
 constexpr int kCubeShapes = 3;
 CubeShape cube_shape(int which) {
     switch (which) {
@@ -566,7 +500,7 @@ int cube_configure(bdg_system *sys) {
     ChebState &st = sys->cheb;
     const int Lx = sys->cubic[0], Ly = sys->cubic[1], Lz = sys->cubic[2];
     const int64_t slots = std::max<int64_t>(1, (int64_t)sys->sm_count / st.n_panels);
-    const int forced_shape = cube_env("BDG_CUBE_SHAPE", -1), forced_seg = cube_env("BDG_CUBE_SEG", 0);
+    const int forced_shape = env_int("BDG_CUBE_SHAPE", -1), forced_seg = env_int("BDG_CUBE_SEG", 0);
     double best = -1.0;
     for (int which = 0; which < kCubeShapes; ++which) {
         if (forced_shape >= 0 && which != forced_shape) continue;
@@ -601,7 +535,7 @@ int cube_configure(bdg_system *sys) {
     constexpr int kPieceCost = 6;
     const double classic_cost = (double)ceil_div((int64_t)gx * st.n_panels, (int64_t)sys->sm_count) * (double)ceil_div(w.n_items, gx) * (w.seg_len + kPieceCost);
     const WorkPlan plan = best_balanced_plan(st.n_panels, w.n_patches, Lx, sys->sm_count, kPieceCost, 1.0);
-    const int force = cube_env("BDG_CUBE_BALANCE", -1);
+    const int force = env_int("BDG_CUBE_BALANCE", -1);
     if (!(force >= 0 ? force != 0 : plan.longest < 0.93 * classic_cost)) return BDG_OK;
     WorkLists lists;
     BDG_TRY(upload_work_lists(sys, st.work_items, plan, st.n_panels, lists));

@@ -78,14 +78,13 @@ __device__ __forceinline__ void ld_table_if(double &v, const double *p, unsigned
 // general: the on-site product is two multiplications instead of two MMAs (a tenth of the row's FP64-pipe time at five
 // blocks per row; the complex-hopping models are the ones the FP64 pipe bounds).  The MMA accumulators START from those
 // products, which is what the MMA of a real-diagonal block leaves in them: same sums, same order as DICT.
-template <int PW, int CH, int NP, int PB, bool DICT, bool DIAG, bool SD = false>
+template <int PW, int CH, int NP, bool DICT, bool DIAG, bool SD = false>
 __global__ void __launch_bounds__(kThreads, 4)
 cheb_step_ell(const int32_t *__restrict__ cidx, const int32_t *__restrict__ ccode, const double *__restrict__ cdata,
               const double *__restrict__ dtab, const double2 *__restrict__ x_cur, double2 *__restrict__ x_io, int n_sites, int n_panels, double alpha,
               double beta, int first, int stream_matrix, double *__restrict__ partials,
               unsigned *__restrict__ tickets, double *__restrict__ dots_step, const RowWalk wk) {
     constexpr int REC = PW * 4;           // complex elements per site record
-    static_assert(NP % PB == 0, "PB = panels whose loads are in flight together");
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int panel0 = blockIdx.y * NP;
     const size_t plane = (size_t)n_sites * REC;
@@ -195,44 +194,42 @@ cheb_step_ell(const int32_t *__restrict__ cidx, const int32_t *__restrict__ ccod
         }
         const size_t off = (size_t)row * REC + x_elem;
 
+        // all loads of the NP panels first, then their products
+        double2 xv[NP][CH], pv[NP];
+        bool on[NP];
 #pragma unroll
-        for (int pb = 0; pb < NP; pb += PB) {
-            double2 xv[PB][CH], pv[PB];
-            bool on[PB];
+        for (int pp = 0; pp < NP; ++pp) {
+            const int panel = panel0 + pp;
+            on[pp] = NP == 1 || panel < n_panels;          // uniform; ragged last group only
+            const size_t base = (size_t)(on[pp] ? panel : n_panels - 1) * plane;
 #pragma unroll
-            for (int pp = 0; pp < PB; ++pp) {
-                const int panel = panel0 + pb + pp;
-                on[pp] = NP == 1 || panel < n_panels;          // uniform; ragged last group only
-                const size_t base = (size_t)(on[pp] ? panel : n_panels - 1) * plane;
+            for (int u = 0; u < CH; ++u) xv[pp][u] = ld_reuse(x_cur + base + (size_t)jn[u] * REC + x_elem);
+            pv[pp] = make_double2(0.0, 0.0);
+            if (!first) pv[pp] = ld_plain(x_io + base + off);
+        }
 #pragma unroll
-                for (int u = 0; u < CH; ++u) xv[pp][u] = ld_reuse(x_cur + base + (size_t)jn[u] * REC + x_elem);
-                pv[pp] = make_double2(0.0, 0.0);
-                if (!first) pv[pp] = ld_plain(x_io + base + off);
+        for (int pp = 0; pp < NP; ++pp) {
+            double a10 = 0.0, a11 = 0.0, a20 = 0.0, a21 = 0.0;
+            if (SD) a10 = bop[0] * xv[pp][0].x, a20 = bop[0] * xv[pp][0].y;
+#pragma unroll
+            for (int u = SD ? 1 : 0; u < (DIAG ? 1 : CH); ++u) {
+                dmma_8x8x4(a10, a11, xv[pp][u].x, bop[u]);
+                dmma_8x8x4(a20, a21, xv[pp][u].y, bop[u]);
             }
+            double yr = a10 - a21, yi = a11 + a20;
+            if (DIAG) {
 #pragma unroll
-            for (int pp = 0; pp < PB; ++pp) {
-                double a10 = 0.0, a11 = 0.0, a20 = 0.0, a21 = 0.0;
-                if (SD) a10 = bop[0] * xv[pp][0].x, a20 = bop[0] * xv[pp][0].y;
-#pragma unroll
-                for (int u = SD ? 1 : 0; u < (DIAG ? 1 : CH); ++u) {
-                    dmma_8x8x4(a10, a11, xv[pp][u].x, bop[u]);
-                    dmma_8x8x4(a20, a21, xv[pp][u].y, bop[u]);
+                for (int u = 1; u < CH; ++u) {
+                    yr = fma(bop[u], xv[pp][u].x, yr);
+                    yi = fma(bop[u], xv[pp][u].y, yi);
                 }
-                double yr = a10 - a21, yi = a11 + a20;
-                if (DIAG) {
-#pragma unroll
-                    for (int u = 1; u < CH; ++u) {
-                        yr = fma(bop[u], xv[pp][u].x, yr);
-                        yi = fma(bop[u], xv[pp][u].y, yi);
-                    }
-                }
-                if (on[pp] && x_lane) {
-                    const double2 tn = xv[pp][0];  // slot 0 is the row's own record
-                    const double2 out = make_double2(alpha * yr - beta * pv[pp].x, alpha * yi - beta * pv[pp].y);
-                    x_io[(size_t)(panel0 + pb + pp) * plane + off] = out;
-                    d0[pb + pp] += tn.x * tn.x + tn.y * tn.y;
-                    d1[pb + pp] += out.x * tn.x + out.y * tn.y;
-                }
+            }
+            if (on[pp] && x_lane) {
+                const double2 tn = xv[pp][0];  // slot 0 is the row's own record
+                const double2 out = make_double2(alpha * yr - beta * pv[pp].x, alpha * yi - beta * pv[pp].y);
+                x_io[(size_t)(panel0 + pp) * plane + off] = out;
+                d0[pp] += tn.x * tn.x + tn.y * tn.y;
+                d1[pp] += out.x * tn.x + out.y * tn.y;
             }
         }
         jv = jnext;
@@ -527,46 +524,35 @@ patch_blocks(int64_t n, const int32_t *__restrict__ klist, const PatchArgs a) {
 using EllKernel = void (*)(const int32_t *, const int32_t *, const double *, const double *, const double2 *, double2 *,
                            int, int, double, double, int, int, double *, unsigned *, double *, const RowWalk);
 
-template <int PW, int NP, int PB, bool DICT, bool DIAG, bool SD> EllKernel pick_ch(int width) {
+template <int PW, int NP, bool DICT, bool DIAG, bool SD> EllKernel pick_ch(int width) {
     switch (width) {
-        case 3: return cheb_step_ell<PW, 3, NP, PB, DICT, DIAG, SD>;
-        case 4: return cheb_step_ell<PW, 4, NP, PB, DICT, DIAG, SD>;
-        case 5: return cheb_step_ell<PW, 5, NP, PB, DICT, DIAG, SD>;
-        case 6: return cheb_step_ell<PW, 6, NP, PB, DICT, DIAG, SD>;
-        case 7: return cheb_step_ell<PW, 7, NP, PB, DICT, DIAG, SD>;
-        default: return cheb_step_ell<PW, 8, NP, PB, DICT, DIAG, SD>;
+        case 3: return cheb_step_ell<PW, 3, NP, DICT, DIAG, SD>;
+        case 4: return cheb_step_ell<PW, 4, NP, DICT, DIAG, SD>;
+        case 5: return cheb_step_ell<PW, 5, NP, DICT, DIAG, SD>;
+        case 6: return cheb_step_ell<PW, 6, NP, DICT, DIAG, SD>;
+        case 7: return cheb_step_ell<PW, 7, NP, DICT, DIAG, SD>;
+        default: return cheb_step_ell<PW, 8, NP, DICT, DIAG, SD>;
     }
 }
 
-template <bool DICT, bool DIAG, bool SD = false> EllKernel pick_shape(int pw, int np, int pb, int width) {
+template <bool DICT, bool DIAG, bool SD = false> EllKernel pick_shape(int pw, int width) {
     switch (pw) {
-        case 1: return pick_ch<1, 1, 1, DICT, DIAG, SD>(width);
-        case 2: return pick_ch<2, 1, 1, DICT, DIAG, SD>(width);
-        case 4: return pick_ch<4, 1, 1, DICT, DIAG, SD>(width);
-        default:
-            if (np >= 8) return pick_ch<8, 8, 1, DICT, DIAG, SD>(width);
-            if (np >= 4) return pb >= 2 ? pick_ch<8, 4, 2, DICT, DIAG, SD>(width) : pick_ch<8, 4, 1, DICT, DIAG, SD>(width);
-            if (np >= 2) return pb >= 2 ? pick_ch<8, 2, 2, DICT, DIAG, SD>(width) : pick_ch<8, 2, 1, DICT, DIAG, SD>(width);
-            return pick_ch<8, 1, 1, DICT, DIAG, SD>(width);
+        case 1: return pick_ch<1, 1, DICT, DIAG, SD>(width);
+        case 2: return pick_ch<2, 1, DICT, DIAG, SD>(width);
+        case 4: return pick_ch<4, 1, DICT, DIAG, SD>(width);
+        default: return pick_ch<8, 1, DICT, DIAG, SD>(width);
     }
 }
 
-// fmt: BDG_KERNEL_ELL, BDG_KERNEL_DICT or BDG_KERNEL_DICT_DIAG; self_diag: DICT with real-diagonal on-site blocks (SD)
-EllKernel pick_ell(int fmt, int pw, int np, int pb, int width, bool self_diag) {
-    if (fmt == BDG_KERNEL_DICT_DIAG) return pick_shape<true, true>(pw, np, pb, width);
-    if (fmt == BDG_KERNEL_DICT) return self_diag ? pick_shape<true, false, true>(pw, np, pb, width) : pick_shape<true, false>(pw, np, pb, width);
-    return pick_shape<false, false>(pw, np, pb, width);
+// fmt: BDG_KERNEL_ELL, BDG_KERNEL_DICT or BDG_KERNEL_DICT_DIAG; np: panels per pass (ell_configure); self_diag: DICT with
+// real-diagonal on-site blocks (SD)
+EllKernel pick_ell(int fmt, int pw, int np, int width, bool self_diag) {
+    if (fmt == BDG_KERNEL_DICT_DIAG) return pick_shape<true, true>(pw, width);
+    if (fmt == BDG_KERNEL_DICT) return self_diag ? pick_shape<true, false, true>(pw, width) : pick_shape<true, false>(pw, width);
+    return np == 2 ? pick_ch<8, 2, false, false, false>(width) : pick_shape<false, false>(pw, width);
 }
 
-bool ell_self_diag(const EllDev &e) {
-    const char *v = getenv("BDG_ELL_SD");
-    return e.self_diag_usable && (v && *v ? atoi(v) != 0 : true);
-}
-
-int env_int(const char *name, int fallback) {
-    const char *v = getenv(name);
-    return v && *v ? atoi(v) : fallback;
-}
+bool ell_self_diag(const EllDev &e) { return e.self_diag_usable && env_int("BDG_ELL_SD", 1) != 0; }
 
 // Plan the row traversal for `slots` resident CTAs per panel group (RowWalk, bdg_internal.h).
 RowWalk plan_walk(const bdg_system *sys, int n_sites, int64_t slots) {
@@ -817,18 +803,10 @@ int ell_configure(bdg_system *sys) {
     const bool dict = st.kernel != BDG_KERNEL_ELL;
     const bool pair = !dict && st.panel_width == 8 && st.n_panels >= 2 && e.width >= 6;
     st.panels_per_group = pair ? 2 : 1;
-    st.panel_batch = st.panels_per_group;
-    // tuning overrides (development): BDG_ELL_NP in {1,2,4,8}, BDG_ELL_PB in {1,2}
-    if (st.panel_width == 8) {
-        st.panels_per_group = std::min(env_int("BDG_ELL_NP", st.panels_per_group), std::max(st.n_panels, 1));
-        st.panels_per_group = st.panels_per_group >= 8 ? 8 : st.panels_per_group >= 4 ? 4 : st.panels_per_group >= 2 ? 2 : 1;
-        st.panel_batch = st.panels_per_group >= 8 ? 1 : std::min(env_int("BDG_ELL_PB", st.panel_batch), st.panels_per_group);
-    }
     st.n_groups = (int)ceil_div(st.n_panels, st.panels_per_group);
     int per_sm = 1;
     BDG_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(
-        &per_sm, pick_ell(st.kernel, st.panel_width, st.panels_per_group, st.panel_batch, e.width, ell_self_diag(e)), kThreads,
-        (size_t)env_int("BDG_ELL_PAD", 0)));
+        &per_sm, pick_ell(st.kernel, st.panel_width, st.panels_per_group, e.width, ell_self_diag(e)), kThreads, 0));
     per_sm = std::max(per_sm, 1);
     const int64_t slots = std::max<int64_t>(1, (int64_t)sys->sm_count * per_sm / st.n_groups);
     st.walk = plan_walk(sys, (int)e.n_sites, slots);
@@ -840,15 +818,13 @@ int ell_launch_step(bdg_system *sys, bool first, const void *x_cur, void *x_io, 
     ChebState &st = sys->cheb;
     const EllDev &e = sys->ell;
     const bool dict = st.kernel == BDG_KERNEL_DICT || st.kernel == BDG_KERNEL_DICT_DIAG;
-    EllKernel k = pick_ell(st.kernel, st.panel_width, st.panels_per_group, st.panel_batch, e.width, ell_self_diag(e));
+    EllKernel k = pick_ell(st.kernel, st.panel_width, st.panels_per_group, e.width, ell_self_diag(e));
     // Stream the matrix through L2 (evict-first) only when nothing will read it again soon: one
     // group per pass and a matrix that cannot stay resident in the 126 MB L2 anyway.
     const size_t matrix_bytes = (size_t)e.n_sites * e.width * 260;
     const int stream_matrix = st.n_groups == 1 && matrix_bytes > (size_t)64 << 20;
     dim3 grid((unsigned)st.grid_x, (unsigned)st.n_groups);
-    const size_t pad = (size_t)env_int("BDG_ELL_PAD", 0);  // occupancy experiments: unused dynamic shared memory
-    if (pad > 48 * 1024) cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pad);
-    k<<<grid, kThreads, pad, sys->stream>>>(e.idx.as<int32_t>(), dict ? e.code.as<int32_t>() : nullptr,
+    k<<<grid, kThreads, 0, sys->stream>>>(e.idx.as<int32_t>(), dict ? e.code.as<int32_t>() : nullptr,
                                           dict ? e.table.as<double>() : e.data.as<double>(), e.dtab.as<double>(),
                                           static_cast<const double2 *>(x_cur), static_cast<double2 *>(x_io),
                                           (int)e.n_sites, st.n_panels, (first ? 1.0 : 2.0) / st.scale, first ? 0.0 : 1.0,

@@ -36,10 +36,8 @@
 // column there: equal to rounding); the dot products are summed over a different partition of the rows (agree to
 // rounding).
 //
-// Compile-time experiments kept for the record (DESIGN 4.1-iv; all within +-1 % of the default at 10^6 sites):
-// -DBDG_PAIR_PV3 (E_{j-1} two planes ahead), -DBDG_PAIR_SPLIT (split-phase mbarrier hand-over between [A] and [B],
-// [B] started on the warp's own records before the wait); run time: BDG_PAIR_WARPS=12 (REG: own records in registers,
-// one CTA per SM), =16; BDG_PAIR_SELF, BDG_PAIR_P, BDG_PAIR_SEG.
+// The other shapes, hand-overs between [A] and [B] and prefetch distances that were measured against this one, and
+// why none was kept, are in DESIGN 4.1-iv.
 #include <algorithm>
 #include <array>
 #include <cstdlib>
@@ -56,15 +54,11 @@ namespace {
 constexpr int kRecBytes = 512;  // one site record at PW = 8: 8 columns x 4 components x complex128
 constexpr int kRing = 4;        // planes of the T_{n+1} ring (three read by [B], one being written)
 constexpr int kRingN = 8;       // planes of the T_n ring: three in use, five in flight (power of two)
-// Hand-over between the warps of a CTA: the __syncthreads between [A] and [B] (default); -DBDG_PAIR_LAZY = arrive at the end of an
-// iteration, wait after [A] of the next (see the loop: +2.8 % at burst clocks, -1 % under the sustained power cap: its 256
-// polling threads cost the clock what the slack gains; one poller per warp is 9 % slower; profiles/r02/54_* .. 58_*);
-// -DBDG_PAIR_SPLIT = the earlier split-phase experiment.
-#ifdef BDG_PAIR_LAZY
-constexpr int kRingGuard = 1;
-#else
-constexpr int kRingGuard = 0;
-#endif
+// 8 warps x 2 sites per CTA, two CTAs per SM: one computes while the other waits at its barrier.  The shape sweep
+// (profiles/r01/s4_pair_shape_sweep.log: 16 x 2 one CTA per SM -2 %, 8 x 3 -11 %, 12 x 1 with 24 warps per SM -14 %,
+// 6 x 2 with three CTAs per SM -15 %) and the 12-warp shape with its own records in registers (0.159 against 0.141
+// ms/step, DESIGN 4.1-iv) left this one ahead.
+constexpr int kPairWarps = 8, kPairSites = 2, kPairMinBlocks = 2;
 
 constexpr int kDirs = 5;  // direction-ordered row: self, x-1, y-1, y+1, x+1 (= ascending block column)
 
@@ -109,8 +103,8 @@ __device__ __forceinline__ void self_fragments(int jv, double (&f)[S], const dou
 }
 
 // y = sum_u B_u x_u for this lane's element; order and operations of cheb_step_ell (directions: self, x-1, y-1,
-// y+1, x+1 = ascending block column on an open lattice), in stages so that sub-step [B] can start on the records its
-// own warp wrote while the rest of the CTA is still arriving at the barrier: begin (self), add x 4, end.
+// y+1, x+1 = ascending block column on an open lattice), in stages so that sub-step [A] can wait for its newest plane
+// only before the last term: begin (self), add x 4, end.
 // SD (without DIAG): the on-site block is real and diagonal (cheb_ell.cu: SD) -- its product is two multiplications, and
 // the accumulators of the hopping blocks' MMAs start from them (what the MMA of such a block leaves there).
 template <bool DIAG, bool SD = false> struct RowSum {
@@ -152,16 +146,10 @@ __device__ __forceinline__ void row_product(const double2 &x0, const double2 &x1
     yi = r.yi;
 }
 
-#if defined(BDG_PAIR_SPLIT) || defined(BDG_PAIR_LAZY)
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];\n" ::"r"(bar) : "memory");
-}
-#endif
-
-// NW warps per CTA, two ADJACENT sites per warp and plane: W = 2 NW sites per plane in sub-step [A]
+// NW warps per CTA, S = 2 ADJACENT sites per warp and plane: W = 2 NW sites per plane in sub-step [A]
 // (P <= W - 2 of them owned).  Dynamic shared memory: kRingN planes of W + 2 records (T_n), kRing
-// planes of W records (T_{n+1}), two guard records, one mbarrier per T_n plane: 105 KB at NW = 8, so two
-// CTAs share an SM (one computes while the other waits at its barrier).
+// planes of W records (T_{n+1}), two guard records, one mbarrier per T_n plane and one more: 105 KB, so two
+// CTAs share an SM.
 //
 // Geometry is a TORUS: planes x and in-plane sites y are taken modulo Lx and M, so the halo of the first /
 // last patch and of the first / last segment is the opposite face of the lattice (staged by its own small bulk
@@ -189,82 +177,19 @@ __device__ __forceinline__ void mbar_arrive(uint32_t bar) {
 // from which the same four moments follow (cheb.cu: t2_normalize), but it moves THREE vector passes instead
 // of four, and two vector buffers suffice.  `first`: E_1 = T_2(H~) E_0 = 2 H~ u - E_0 (E_{-1} = E_1).
 //
-// REG (the 12-warp shape: one CTA per SM, 168 registers per thread): the warp's OWN records stay in registers from
-// plane to plane -- the T_n records it read as its x+1 neighbours are its centre records one iteration later and its x-1
-// neighbours (and the T_n of [B]) two iterations later, and the T_{n+1} records it computes are its own operands of [B]
-// for three iterations -- so shared memory is read only for what OTHER warps own: 6 instead of 16 LDS.128 per warp and
-// iteration.  The shared-memory / L1 data pipe is what bounds the 8-warp shape (DESIGN 4.1-iv).
-// The four dot products of a run (= the pieces of one panel a CTA works through): quad -> warp -> CTA -> partials[run]; the
-// last run of a panel to arrive (runs r0 .. r1) adds the panel's partials up in a fixed order.  Called by all threads between
-// two pieces or at the end: the rings are idle and serve as scratch.
-template <int NW>
-__device__ __forceinline__ void flush_dots(double d0, double d1, double d2, double d3, unsigned char *scratch, int run, int r0, int r1,
-                                           int panel, int n_panels, double *__restrict__ partials, unsigned *__restrict__ tickets,
-                                           double *__restrict__ dots_step) {
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    __shared__ bool is_last;
-    d0 += __shfl_xor_sync(kFull, d0, 1);
-    d1 += __shfl_xor_sync(kFull, d1, 1);
-    d2 += __shfl_xor_sync(kFull, d2, 1);
-    d3 += __shfl_xor_sync(kFull, d3, 1);
-    d0 += __shfl_xor_sync(kFull, d0, 2);
-    d1 += __shfl_xor_sync(kFull, d1, 2);
-    d2 += __shfl_xor_sync(kFull, d2, 2);
-    d3 += __shfl_xor_sync(kFull, d3, 2);
-    __syncthreads();
-    double *red = reinterpret_cast<double *>(scratch);  // [NW][4][8], then comb [NW][32] behind it
-    double *comb = red + NW * 32;
-    if ((lane & 3) == 0) {
-        const int col = lane >> 2;
-        red[(warp * 4 + 0) * 8 + col] = d0;
-        red[(warp * 4 + 1) * 8 + col] = d1;
-        red[(warp * 4 + 2) * 8 + col] = d2;
-        red[(warp * 4 + 3) * 8 + col] = d3;
-    }
-    __syncthreads();
-    if (threadIdx.x < 32) {
-        double s = 0.0;
-#pragma unroll
-        for (int w = 0; w < NW; ++w) s += red[w * 32 + threadIdx.x];
-        partials[(size_t)run * 32 + threadIdx.x] = s;
-    }
-    __threadfence();
-    __syncthreads();
-    if (threadIdx.x == 0) is_last = atomicAdd(&tickets[panel], 1u) == (unsigned)(r1 - r0 - 1);
-    __syncthreads();
-    if (is_last) {
-        __threadfence();
-        double s = 0.0;
-        for (int b = r0 + warp; b < r1; b += NW) s += __ldcg(&partials[(size_t)b * 32 + lane]);
-        comb[warp * 32 + lane] = s;
-        __syncthreads();
-        if (threadIdx.x < 32) {
-            double t = 0.0;
-#pragma unroll
-            for (int g = 0; g < NW; ++g) t += comb[g * 32 + threadIdx.x];
-            // slot = which * 8 + column; which = (step within the pair) * 2 + (0: <T,T>, 1: <T',T>)
-            dots_step[(size_t)(threadIdx.x >> 3) * n_panels * 8 + panel * 8 + (threadIdx.x & 7)] = t;
-        }
-        if (threadIdx.x == 0) tickets[panel] = 0u;
-    }
-    __syncthreads();  // scratch and is_last are free again
-}
-
 // LISTED: the CTA's pieces come from the work lists of PairWalk (balanced plan, grid = (n_ctas, 1)); otherwise they are
 // computed from the item index (classic plan, grid = (CTAs per panel, panels)) -- kept as arithmetic on kernel parameters
 // because values loaded from memory leave the uniform datapath and the plane loop's predicates with them (+2 % time).
-template <bool DIAG, bool SELF, int NW, int S, int MINB, int MODE, bool REG = false, bool SD = false, bool LISTED = false>
-__global__ void __launch_bounds__(NW * 32, MINB)
+template <bool DIAG, bool SELF, int MODE, bool SD = false, bool LISTED = false>
+__global__ void __launch_bounds__(kPairWarps * 32, kPairMinBlocks)
 cheb_pair_step(const int32_t *__restrict__ dcode, const double *__restrict__ table, const double *__restrict__ dtab,
                const double2 *__restrict__ xa /* T_{n-1} */, const double2 *__restrict__ xb /* T_n */,
                double2 *__restrict__ xc /* T_{n+1} */, double2 *__restrict__ xd /* T_{n+2} */, int n_sites, int n_panels,
                double alpha, double alpha2, double csub, int first, double *__restrict__ partials, unsigned *__restrict__ tickets,
                double *__restrict__ dots_step, const PairWalk wk) {
     // MODE 1: E_{j+1} = alpha2 H~u - (csub E_j + E_{j-1}); csub = 2, or 1 in the first launch, where E_{-1} is never loaded (= 0)
-    constexpr int W = NW * S, R = kRecBytes;
-    // (lazy hand-over: one guard record behind every T_{n+1} plane -- the first / last warp's outer neighbour read, whose
-    // value never matters, must not land in the slot [A] is writing while [B] of the same iteration reads)
-    constexpr uint32_t PLANE_N = (W + 2) * R, PLANE_W = (W + kRingGuard) * R;
+    constexpr int NW = kPairWarps, S = kPairSites, W = NW * S, R = kRecBytes;
+    constexpr uint32_t PLANE_N = (W + 2) * R, PLANE_W = W * R;
     extern __shared__ __align__(128) unsigned char pair_smem[];
     const uint32_t sTn = smem_u32(pair_smem);         // T_n planes, local site l2 = y - (y0 - 2)
     const uint32_t sT1 = sTn + kRingN * PLANE_N + R;  // guard record, then T_{n+1} planes (computed here), local site l = y - (y0 - 1)
@@ -279,19 +204,16 @@ cheb_pair_step(const int32_t *__restrict__ dcode, const double *__restrict__ tab
     if (threadIdx.x == 0) {
 #pragma unroll
         for (int r = 0; r < kRingN; ++r) mbar_init(sBar + 8 * r, 1);
-        mbar_init(sBar + 8 * kRingN, NW * 32);  // [A] -> [B] hand-over: every thread arrives, waits later (split phase)
+        // Nothing waits on this ninth barrier; it is initialised so that the kernel's code stays the code DESIGN 4.1-iv measured.
+        mbar_init(sBar + 8 * kRingN, NW * 32);
         asm volatile("fence.mbarrier_init.release.cluster;\n" ::: "memory");
     }
     asm volatile("fence.proxy.async.shared::cta;\n" ::: "memory");  // the clears are ordered before the bulk copies
     __syncthreads();
     uint32_t cnt = 0;  // T_n planes consumed by the items before this one
-#if defined(BDG_PAIR_SPLIT) || defined(BDG_PAIR_LAZY)
-    uint32_t xphase = 0;  // parity of the hand-over barrier's current phase (one phase per iteration)
-#endif
     const size_t gstep = (size_t)wk.M * 32;
     double d0 = 0.0, d1 = 0.0, d2 = 0.0, d3 = 0.0;
 
-    {
     const int l0 = S * warp;  // this warp's sites: l0, l0 + 1
     // own-record addresses of site l0 in slot 0 of each ring (+ lane's 16 bytes)
     uint32_t aN = sTn + (uint32_t)(l0 + 1) * R + (uint32_t)lane * 16u;
@@ -316,8 +238,8 @@ cheb_pair_step(const int32_t *__restrict__ dcode, const double *__restrict__ tab
             piece = wk.pieces[item];  // (run, patch, x0, len)
             if (piece.x != run) {
                 if (run >= 0) {
-                    flush_dots<NW>(d0, d1, d2, d3, pair_smem, run, wk.panel_runs[panel], wk.panel_runs[panel + 1], panel, n_panels, partials,
-                                   tickets, dots_step);
+                    flush_dots<NW, 8>(d0, d1, d2, d3, pair_smem, run, wk.panel_runs[panel], wk.panel_runs[panel + 1], panel, n_panels, partials,
+                                      tickets, dots_step);
                     d0 = d1 = d2 = d3 = 0.0;
                 }
                 run = piece.x;
@@ -413,11 +335,6 @@ cheb_pair_step(const int32_t *__restrict__ dcode, const double *__restrict__ tab
         int xprev = x0 - 1;  // wrapped plane of [A]
         xprev += xprev < 0 ? wk.Lx : 0;
         double2 pv[S], pvn[S];  // MODE 1: E_{j-1} of the plane of [B] in this / in the next iteration
-#ifdef BDG_PAIR_PV3
-        double2 pvn2[S];        // ... and in the one after: the load is issued two and a half iterations ahead of its use
-#pragma unroll
-        for (int s = 0; s < S; ++s) pvn2[s] = make_double2(0.0, 0.0);
-#endif
 #pragma unroll
         for (int s = 0; s < S; ++s) {
             pv[s] = pvn[s] = make_double2(0.0, 0.0);
@@ -425,36 +342,17 @@ cheb_pair_step(const int32_t *__restrict__ dcode, const double *__restrict__ tab
         }
         wait(0);
         wait(1);
-        double2 rt[S], rc[S], o1[S], o2[S];  // REG: own records of T_n planes i, i + 1 and of T_{n+1} planes i - 1, i - 2
-#pragma unroll
-        for (int s = 0; s < S; ++s) {
-            rt[s] = rc[s] = o1[s] = o2[s] = make_double2(0.0, 0.0);
-            if (REG) {
-                rt[s] = lds_rec(aN + (cnt & (kRingN - 1)) * PLANE_N + (uint32_t)s * R);
-                rc[s] = lds_rec(aN + ((cnt + 1) & (kRingN - 1)) * PLANE_N + (uint32_t)s * R);
-            }
-        }
 
         for (int i = 0; i <= len + 1; ++i, pin_ += gstep, pout1 += gstep, pout2 += gstep) {
             const bool store = i >= 1 && i <= len;
             if (MODE == 1) {
                 // E_{j-1} of the plane of [A]: [B] of the NEXT iteration works on that plane (and overwrites it) -- issued
                 // here, an iteration and a half ahead of its use (half an iteration does not cover the HBM latency: measured)
-#ifdef BDG_PAIR_PV3
-                const bool store_next = i + 1 <= len;  // the plane of [A] in the next iteration is an owned plane
-#pragma unroll
-                for (int s = 0; s < S; ++s) {
-                    pv[s] = pvn[s];
-                    pvn[s] = pvn2[s];
-                    if (store_next && owned[s] && !first) pvn2[s] = ld_prev_rw(pin_ + gstep + 32 * s);
-                }
-#else
 #pragma unroll
                 for (int s = 0; s < S; ++s) {
                     pv[s] = pvn[s];
                     if (store && owned[s] && !first) pvn[s] = ld_prev_rw(pin_ + 32 * s);
                 }
-#endif
             } else {  // T_{n-1} of the next plane of [A], one iteration ahead
                 if (i <= len) {
                     xprev += 1;
@@ -500,17 +398,10 @@ cheb_pair_step(const int32_t *__restrict__ dcode, const double *__restrict__ tab
                 const uint32_t np = aN + ((c + 2) & (kRingN - 1)) * PLANE_N;
                 hold_fragments<DIAG, SELF, S, SD>(jvA, jheld, keep, table, dtab, lane, self_lane);
                 double2 c_[S + 2], q[S];  // c_[1 + s] = the own record of site s; c_[0], c_[S + 1] = the warp's in-plane neighbours
-                if (REG) {
-                    c_[0] = lds_rec(n0 - R);
-                    c_[S + 1] = lds_rec(n0 + (uint32_t)S * R);
 #pragma unroll
-                    for (int s = 0; s < S; ++s) c_[1 + s] = rc[s], tn[s] = rt[s];
-                } else {
+                for (int k = 0; k < S + 2; ++k) c_[k] = lds_rec(n0 + (uint32_t)(k - 1) * R);
 #pragma unroll
-                    for (int k = 0; k < S + 2; ++k) c_[k] = lds_rec(n0 + (uint32_t)(k - 1) * R);
-#pragma unroll
-                    for (int s = 0; s < S; ++s) tn[s] = lds_rec(nm + (uint32_t)s * R);
-                }
+                for (int s = 0; s < S; ++s) tn[s] = lds_rec(nm + (uint32_t)s * R);
                 const uint32_t t1 = a1 + (uint32_t)(i & (kRing - 1)) * PLANE_W;
                 // The newest plane (x+1 neighbours) feeds the LAST term of a row: its barrier is waited for only after the
                 // other four terms are under way (+1 %: profiles/r02/21_latewait.log).
@@ -535,10 +426,6 @@ cheb_pair_step(const int32_t *__restrict__ dcode, const double *__restrict__ tab
                     else out[s] = make_double2(alpha * yr, alpha * yi);
                     sts_rec(t1 + (uint32_t)s * R, out[s]);
                 }
-                if (REG) {
-#pragma unroll
-                    for (int s = 0; s < S; ++s) rt[s] = rc[s], rc[s] = q[s];
-                }
                 if (store) {
 #pragma unroll
                     for (int s = 0; s < S; ++s) {
@@ -550,42 +437,22 @@ cheb_pair_step(const int32_t *__restrict__ dcode, const double *__restrict__ tab
                     }
                 }
             }
-#ifndef BDG_PAIR_SPLIT
-#ifdef BDG_PAIR_LAZY
-            // What [B] of this iteration reads from OTHER warps is a plane old: the in-plane neighbours of T_{n+1}(x - 1), written
-            // in [A] of the previous iteration (the planes x - 2 and x it reads at the warp's own sites only).  So the CTA-wide
-            // hand-over it needs is the one of the PREVIOUS iteration: every thread arrives at the end of an iteration and waits
-            // for that phase only after [A] of the next one -- half an iteration of slack instead of none.
-            if (i >= 1) {
-                mbar_wait(sBar + 8 * kRingN, xphase);
-                xphase ^= 1u;
-                issue(i - 1 + kRingN);  // every warp is through [A] of iteration i - 1: plane i - 1 is dead
-            }
-#else
             __syncthreads();  // T_{n+1} of this plane complete in the ring
             // ... and [A] is done in every warp: plane i (its x-1 neighbours) is dead, its slot takes plane i + 8 -- seven
             // planes in flight beyond the one in use.
             issue(i + kRingN);
-#endif
             if (i >= 2) {
                 const uint32_t t0 = a1 + (uint32_t)((i - 1) & (kRing - 1)) * PLANE_W;
                 const uint32_t tm = a1 + (uint32_t)((i - 2) & (kRing - 1)) * PLANE_W;
                 const uint32_t tp = a1 + (uint32_t)(i & (kRing - 1)) * PLANE_W;
                 hold_fragments<DIAG, SELF, S, SD>(jvB, jheld, keep, table, dtab, lane, self_lane);
                 double2 c_[S + 2], m[S], q[S];
-                if (REG) {
-                    c_[0] = lds_rec(t0 - R);
-                    c_[S + 1] = lds_rec(t0 + (uint32_t)S * R);
 #pragma unroll
-                    for (int s = 0; s < S; ++s) c_[1 + s] = o1[s], m[s] = o2[s], q[s] = out[s];
-                } else {
+                for (int k = 0; k < S + 2; ++k) c_[k] = lds_rec(t0 + (uint32_t)(k - 1) * R);
 #pragma unroll
-                    for (int k = 0; k < S + 2; ++k) c_[k] = lds_rec(t0 + (uint32_t)(k - 1) * R);
+                for (int s = 0; s < S; ++s) m[s] = lds_rec(tm + (uint32_t)s * R);
 #pragma unroll
-                    for (int s = 0; s < S; ++s) m[s] = lds_rec(tm + (uint32_t)s * R);
-#pragma unroll
-                    for (int s = 0; s < S; ++s) q[s] = lds_rec(tp + (uint32_t)s * R);
-                }
+                for (int s = 0; s < S; ++s) q[s] = lds_rec(tp + (uint32_t)s * R);
 #pragma unroll
                 for (int s = 0; s < S; ++s) {
                     double yr, yi;
@@ -593,81 +460,21 @@ cheb_pair_step(const int32_t *__restrict__ dcode, const double *__restrict__ tab
                     finish_b(s, yr, yi, c_[1 + s]);
                 }
             }
-#else
-            // Split-phase hand-over: arrive, start [B] on the T_{n+1} records this warp wrote itself (own sites of the
-            // three planes: the on-site product, the x-1 term, and for the upper site its lower neighbour), and only then
-            // wait for the other warps' records (one neighbour below, one above).  The order of the terms of a row is
-            // unchanged (self, x-1, y-1, y+1, x+1).
-            static_assert(S == 2, "the staged [B] is written for two sites per warp");
-            mbar_arrive(sBar + 8 * kRingN);
-            if (i >= 2) {
-                const uint32_t t0 = a1 + (uint32_t)((i - 1) & (kRing - 1)) * PLANE_W;
-                const uint32_t tm = a1 + (uint32_t)((i - 2) & (kRing - 1)) * PLANE_W;
-                const uint32_t tp = a1 + (uint32_t)(i & (kRing - 1)) * PLANE_W;
-                hold_fragments<DIAG, SELF, S, SD>(jvB, jheld, keep, table, dtab, lane, self_lane);
-                double2 own[S], m[S], q[S];
-                if (REG) {
-#pragma unroll
-                    for (int s = 0; s < S; ++s) own[s] = o1[s], m[s] = o2[s], q[s] = out[s];
-                } else {
-#pragma unroll
-                    for (int s = 0; s < S; ++s) own[s] = lds_rec(t0 + (uint32_t)s * R);
-#pragma unroll
-                    for (int s = 0; s < S; ++s) m[s] = lds_rec(tm + (uint32_t)s * R);
-#pragma unroll
-                    for (int s = 0; s < S; ++s) q[s] = lds_rec(tp + (uint32_t)s * R);
-                }
-                RowSum<DIAG, SD> r0, r1;
-                r0.begin(own[0], SELF ? fsB[0] : keep[0][0]);
-                r1.begin(own[1], SELF ? fsB[1] : keep[1][0]);
-                r0.add(m[0], keep[0][1]);
-                r1.add(m[1], keep[1][1]);
-                r1.add(own[0], keep[1][2]);
-                mbar_wait(sBar + 8 * kRingN, xphase);
-                issue(i + kRingN);
-                const double2 lo = lds_rec(t0 - R), hi = lds_rec(t0 + 2 * R);
-                r0.add(lo, keep[0][2]);
-                r0.add(own[1], keep[0][3]);
-                r1.add(hi, keep[1][3]);
-                r0.add(q[0], keep[0][4]);
-                r1.add(q[1], keep[1][4]);
-                r0.end();
-                r1.end();
-                finish_b(0, r0.yr, r0.yi, own[0]);
-                finish_b(1, r1.yr, r1.yi, own[1]);
-            } else {
-                mbar_wait(sBar + 8 * kRingN, xphase);
-                issue(i + kRingN);
-            }
-            xphase ^= 1u;
-#endif
-#ifdef BDG_PAIR_LAZY
-            mbar_arrive(sBar + 8 * kRingN);  // this thread's T_{n+1} records of the plane are in the ring, its reads of older planes done
-#endif
-            if (REG) {
-#pragma unroll
-                for (int s = 0; s < S; ++s) o2[s] = o1[s], o1[s] = out[s];
-            }
             jvB = jvA;
             jvA = jnext;
             jnext = jn2;
 #pragma unroll
             for (int s = 0; s < S; ++s) fsB[s] = fsA[s], fsA[s] = fsN[s];
         }
-#ifdef BDG_PAIR_LAZY
-        mbar_wait(sBar + 8 * kRingN, xphase);  // the last iteration's phase: every arrival has its wait
-        xphase ^= 1u;
-#endif
         cnt += (uint32_t)n_planes;
-    }
     }
     if (LISTED) {
         if (panel >= 0)
-            flush_dots<NW>(d0, d1, d2, d3, pair_smem, run, wk.panel_runs[panel], wk.panel_runs[panel + 1], panel, n_panels, partials, tickets,
-                           dots_step);
+            flush_dots<NW, 8>(d0, d1, d2, d3, pair_smem, run, wk.panel_runs[panel], wk.panel_runs[panel + 1], panel, n_panels, partials, tickets,
+                              dots_step);
     } else {
         const int p = (int)blockIdx.y, r0 = p * (int)gridDim.x;
-        flush_dots<NW>(d0, d1, d2, d3, pair_smem, r0 + (int)blockIdx.x, r0, r0 + (int)gridDim.x, p, n_panels, partials, tickets, dots_step);
+        flush_dots<NW, 8>(d0, d1, d2, d3, pair_smem, r0 + (int)blockIdx.x, r0, r0 + (int)gridDim.x, p, n_panels, partials, tickets, dots_step);
     }
 }
 
@@ -707,49 +514,23 @@ pair_codes(int n_sites, int width, int Lx, int M, const int32_t *__restrict__ ci
 using PairKernel = void (*)(const int32_t *, const double *, const double *, const double2 *, const double2 *, double2 *,
                             double2 *, int, int, double, double, double, int, double *, unsigned *, double *, const PairWalk);
 
-template <int NW, int S, int MINB, bool REG = false, bool LISTED = false>
-PairKernel pick_pair_shape(bool diag, bool self, bool t2, bool sd = false) {
+template <bool LISTED> PairKernel pick_pair(bool diag, bool self, bool t2, bool sd) {
     if (sd && !diag) {  // general hopping blocks, real-diagonal on-site blocks
-        if (self) return t2 ? cheb_pair_step<false, true, NW, S, MINB, 1, REG, true, LISTED> : cheb_pair_step<false, true, NW, S, MINB, 0, REG, true, LISTED>;
-        return t2 ? cheb_pair_step<false, false, NW, S, MINB, 1, REG, true, LISTED> : cheb_pair_step<false, false, NW, S, MINB, 0, REG, true, LISTED>;
+        if (self) return t2 ? cheb_pair_step<false, true, 1, true, LISTED> : cheb_pair_step<false, true, 0, true, LISTED>;
+        return t2 ? cheb_pair_step<false, false, 1, true, LISTED> : cheb_pair_step<false, false, 0, true, LISTED>;
     }
     if (self) {
-        if (t2) return diag ? cheb_pair_step<true, true, NW, S, MINB, 1, REG, false, LISTED> : cheb_pair_step<false, true, NW, S, MINB, 1, REG, false, LISTED>;
-        return diag ? cheb_pair_step<true, true, NW, S, MINB, 0, REG, false, LISTED> : cheb_pair_step<false, true, NW, S, MINB, 0, REG, false, LISTED>;
+        if (t2) return diag ? cheb_pair_step<true, true, 1, false, LISTED> : cheb_pair_step<false, true, 1, false, LISTED>;
+        return diag ? cheb_pair_step<true, true, 0, false, LISTED> : cheb_pair_step<false, true, 0, false, LISTED>;
     }
-    if (t2) return diag ? cheb_pair_step<true, false, NW, S, MINB, 1, REG, false, LISTED> : cheb_pair_step<false, false, NW, S, MINB, 1, REG, false, LISTED>;
-    return diag ? cheb_pair_step<true, false, NW, S, MINB, 0, REG, false, LISTED> : cheb_pair_step<false, false, NW, S, MINB, 0, REG, false, LISTED>;
+    if (t2) return diag ? cheb_pair_step<true, false, 1, false, LISTED> : cheb_pair_step<false, false, 1, false, LISTED>;
+    return diag ? cheb_pair_step<true, false, 0, false, LISTED> : cheb_pair_step<false, false, 0, false, LISTED>;
 }
 
-int env_int(const char *name, int fallback) {
-    const char *v = getenv(name);
-    return v && *v ? atoi(v) : fallback;
-}
-
-struct PairShape {
-    int warps, sites;  // NW, S
-    PairKernel kernel;
-    PairKernel listed;  // the same kernel working through the lists of a balanced plan (8-warp shape only), else null
-    size_t smem;
-};
-
-PairShape pair_shape(bool diag, bool self, bool t2, bool sd) {
-    PairShape s;
-    // 8 warps x 2 sites: two CTAs per SM, one computes while the other waits at its barrier.  The shape
-    // sweep (profiles/r01/s4_pair_shape_sweep.log: 16 x 2 one CTA per SM -2 %, 8 x 3 -11 %, 12 x 1 with 24
-    // warps per SM -14 %, 6 x 2 with three CTAs per SM -15 %) left this one ahead; 16 x 2 is kept for the tests.
-    const int warps = env_int("BDG_PAIR_WARPS", 8);
-    s.listed = nullptr;
-    if (warps <= 8)
-        s.warps = 8, s.sites = 2, s.kernel = pick_pair_shape<8, 2, 2>(diag, self, t2, sd), s.listed = pick_pair_shape<8, 2, 2, false, true>(diag, self, t2, sd);
-    else if (warps <= 12)  // one CTA per SM, 168 registers: the warp's own records stay in registers (REG)
-        s.warps = 12, s.sites = 2, s.kernel = pick_pair_shape<12, 2, 1, true>(diag, self, t2, sd);
-    else
-        s.warps = 16, s.sites = 2, s.kernel = pick_pair_shape<16, 2, 1>(diag, self, t2, sd);
-    const int W = s.warps * s.sites;
-    s.smem = ((size_t)kRingN * (W + 2) + (size_t)kRing * (W + kRingGuard) + 2) * kRecBytes + 8 * (kRingN + 1);
-    return s;
-}
+constexpr int kPairThreads = kPairWarps * 32;
+// Dynamic shared memory of cheb_pair_step: the T_n ring, the T_{n+1} ring, two guard records, kRingN + 1 mbarriers.
+constexpr size_t kPairSmem = ((size_t)kRingN * (kPairWarps * kPairSites + 2) + (size_t)kRing * kPairWarps * kPairSites + 2) * kRecBytes +
+                             8 * (kRingN + 1);
 
 // On-site fragments per row straight from the table (SELF) when the dictionary is large: then the on-site blocks
 // differ from site to site (disorder, a self-consistent gap, a phase winding) and holding them in registers from
@@ -760,6 +541,12 @@ bool pair_sd(const EllDev &e) { return e.self_diag_usable && !e.diag_usable && e
 bool pair_self(const EllDev &e) {
     const int forced = env_int("BDG_PAIR_SELF", -1);
     return forced >= 0 ? forced != 0 : e.n_unique > 64;
+}
+
+// The kernel for the matrix in hand; `listed`: the one that works through the lists of a balanced plan.
+PairKernel pair_kernel(const bdg_system *sys, bool t2, bool listed) {
+    const bool diag = sys->cheb.kernel == BDG_KERNEL_DICT_DIAG, self = pair_self(sys->ell), sd = pair_sd(sys->ell);
+    return listed ? pick_pair<true>(diag, self, t2, sd) : pick_pair<false>(diag, self, t2, sd);
 }
 
 }  // namespace
@@ -806,17 +593,17 @@ int pair_probe(bdg_system *sys) {
 int pair_configure(bdg_system *sys) {
     ChebState &st = sys->cheb;
     const EllDev &e = sys->ell;
-    const PairShape shape = pair_shape(st.kernel == BDG_KERNEL_DICT_DIAG, pair_self(e), st.t2, pair_sd(e));
-    BDG_CUDA(cudaFuncSetAttribute(shape.kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)shape.smem));
-    if (shape.listed) BDG_CUDA(cudaFuncSetAttribute(shape.listed, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)shape.smem));
+    const PairKernel kernel = pair_kernel(sys, st.t2, false), listed = pair_kernel(sys, st.t2, true);
+    BDG_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPairSmem));
+    BDG_CUDA(cudaFuncSetAttribute(listed, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPairSmem));
     int per_sm = 1;
-    BDG_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, shape.kernel, shape.warps * 32, shape.smem));
+    BDG_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kPairThreads, kPairSmem));
     per_sm = std::max(per_sm, 1);
     const int64_t slots = std::max<int64_t>(1, (int64_t)sys->sm_count * per_sm / st.n_panels);
     PairWalk &w = st.pair_walk;
     w.Lx = sys->cubic[0];
     w.M = e.pair_M;
-    const int p_max = shape.warps * shape.sites - 2;
+    const int p_max = kPairWarps * kPairSites - 2;
     w.open = e.pair_open && env_int("BDG_PAIR_OPEN", 1) != 0 ? 1 : 0;
     const int to_cover = std::max(1, w.M - 2 * w.open);  // n patches own n P (+ 2: the rim sites of a plane with open ends) sites
     const int n_patches_min = (int)ceil_div(to_cover, p_max);
@@ -855,7 +642,6 @@ int pair_configure(bdg_system *sys) {
     w.pieces = nullptr, w.cta_begin = w.run_panel = w.panel_runs = nullptr;
     w.n_ctas = gx, w.n_runs = gx * st.n_panels;
     st.pair_grid_x = gx;
-    if (!shape.listed) return BDG_OK;
     const WorkPlan plan = best_balanced_plan(st.n_panels, w.n_patches, w.Lx, all_slots, kPieceCost, 1.08);
     const int force = env_int("BDG_PAIR_BALANCE", -1);
     if (!(force >= 0 ? force != 0 : plan.longest < 0.93 * classic_cost)) return BDG_OK;
@@ -871,10 +657,9 @@ int pair_configure(bdg_system *sys) {
 int pair_launch(bdg_system *sys, const void *x_prev, const void *x_cur, void *x_next1, void *x_next2, double *dots_step) {
     ChebState &st = sys->cheb;
     const EllDev &e = sys->ell;
-    const PairShape shape = pair_shape(st.kernel == BDG_KERNEL_DICT_DIAG, pair_self(e), false, pair_sd(e));
     const bool listed = st.pair_walk.pieces != nullptr;
     dim3 grid((unsigned)st.pair_walk.n_ctas, listed ? 1u : (unsigned)st.n_panels);
-    (listed ? shape.listed : shape.kernel)<<<grid, shape.warps * 32, shape.smem, sys->stream>>>(
+    pair_kernel(sys, false, listed)<<<grid, kPairThreads, kPairSmem, sys->stream>>>(
         e.dcode.as<int32_t>(), e.table.as<double>(), e.dtab.as<double>(), static_cast<const double2 *>(x_prev),
         static_cast<const double2 *>(x_cur), static_cast<double2 *>(x_next1), static_cast<double2 *>(x_next2),
         (int)e.n_sites, st.n_panels, 2.0 / st.scale, 0.0, 0.0, 0, st.partials.as<double>(), st.tickets.as<unsigned>(), dots_step,
@@ -888,10 +673,9 @@ int t2_launch(bdg_system *sys, bool first, const void *x_cur, void *x_io, double
     ChebState &st = sys->cheb;
     if (st.cube) return cube_launch(sys, first, x_cur, x_io, dots_step);
     const EllDev &e = sys->ell;
-    const PairShape shape = pair_shape(st.kernel == BDG_KERNEL_DICT_DIAG, pair_self(e), true, pair_sd(e));
     const bool listed = st.pair_walk.pieces != nullptr;
     dim3 grid((unsigned)st.pair_walk.n_ctas, listed ? 1u : (unsigned)st.n_panels);
-    (listed ? shape.listed : shape.kernel)<<<grid, shape.warps * 32, shape.smem, sys->stream>>>(
+    pair_kernel(sys, true, listed)<<<grid, kPairThreads, kPairSmem, sys->stream>>>(
         e.dcode.as<int32_t>(), e.table.as<double>(), e.dtab.as<double>(), static_cast<const double2 *>(x_io),
         static_cast<const double2 *>(x_cur), nullptr, static_cast<double2 *>(x_io), (int)e.n_sites, st.n_panels,
         1.0 / st.scale, (first ? 2.0 : 4.0) / st.scale, first ? 1.0 : 2.0, first ? 1 : 0, st.partials.as<double>(), st.tickets.as<unsigned>(),

@@ -1,9 +1,11 @@
 // Shared-memory staging helpers of the two-steps-per-pass kernels (cheb_pair.cu: one-dimensional x-planes,
-// cheb_cube.cu: three-dimensional lattices): mbarriers, bulk async copies (TMA), 128-bit shared-memory accesses.
-// Internal, not part of the ABI.
+// cheb_cube.cu: three-dimensional lattices): mbarriers, bulk async copies (TMA), 128-bit shared-memory accesses,
+// and their reduction of the dot products.  Internal, not part of the ABI.
 #pragma once
 
 #include <stdint.h>
+
+#include "cheb_device.cuh"
 
 namespace {
 
@@ -59,5 +61,71 @@ __device__ __forceinline__ void ld_table_pred(double &v, const double *p, unsign
 // Keep a value in its register: the compiler otherwise re-derives loop invariants (shared-memory
 // base, lane offsets) inside the row loop, which is instruction-issue-bound.
 __device__ __forceinline__ void pin(uint32_t &v) { asm volatile("" : "+r"(v)); }
+
+// The four dot products of a run (= the pieces of one panel a CTA works through) on PW-column panels: components (quad of
+// lanes) -> at PW = 4 the two sites of a warp (lane halves) -> warp -> CTA -> partials[run]; the last run of a panel to
+// arrive (runs r0 .. r1) adds the panel's partials up in run order, so the result is bit-reproducible.  Called by all
+// NW warps between two pieces or at the end: the rings are idle and serve as scratch.
+template <int NW, int PW>
+__device__ __forceinline__ void flush_dots(double d0, double d1, double d2, double d3, unsigned char *scratch, int run, int r0, int r1,
+                                           int panel, int n_panels, double *__restrict__ partials, unsigned *__restrict__ tickets,
+                                           double *__restrict__ dots_step) {
+    static_assert(PW == 4 || PW == 8, "a lane holds one (column, component) element of one site");
+    constexpr int N = 4 * PW;  // slots: which * PW + column; which = (step within the pair) * 2 + (0: <T,T>, 1: <T',T>)
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    __shared__ bool is_last;
+    d0 += __shfl_xor_sync(kFull, d0, 1);
+    d1 += __shfl_xor_sync(kFull, d1, 1);
+    d2 += __shfl_xor_sync(kFull, d2, 1);
+    d3 += __shfl_xor_sync(kFull, d3, 1);
+    d0 += __shfl_xor_sync(kFull, d0, 2);
+    d1 += __shfl_xor_sync(kFull, d1, 2);
+    d2 += __shfl_xor_sync(kFull, d2, 2);
+    d3 += __shfl_xor_sync(kFull, d3, 2);
+    if (PW == 4) {
+        d0 += __shfl_xor_sync(kFull, d0, 16);
+        d1 += __shfl_xor_sync(kFull, d1, 16);
+        d2 += __shfl_xor_sync(kFull, d2, 16);
+        d3 += __shfl_xor_sync(kFull, d3, 16);
+    }
+    __syncthreads();
+    double *red = reinterpret_cast<double *>(scratch);  // [NW][4 which][PW columns], then comb [NW][N] behind it
+    double *comb = red + NW * N;
+    if ((PW == 8 || lane < 16) && (lane & 3) == 0) {
+        const int col = lane >> 2;
+        red[(warp * 4 + 0) * PW + col] = d0;
+        red[(warp * 4 + 1) * PW + col] = d1;
+        red[(warp * 4 + 2) * PW + col] = d2;
+        red[(warp * 4 + 3) * PW + col] = d3;
+    }
+    __syncthreads();
+    if (threadIdx.x < N) {
+        double s = 0.0;
+#pragma unroll
+        for (int w = 0; w < NW; ++w) s += red[w * N + threadIdx.x];
+        partials[(size_t)run * N + threadIdx.x] = s;
+    }
+    __threadfence();
+    __syncthreads();
+    if (threadIdx.x == 0) is_last = atomicAdd(&tickets[panel], 1u) == (unsigned)(r1 - r0 - 1);
+    __syncthreads();
+    if (is_last) {
+        __threadfence();
+        if (PW == 8 || lane < 16) {
+            double s = 0.0;
+            for (int b = r0 + warp; b < r1; b += NW) s += __ldcg(&partials[(size_t)b * N + lane]);
+            comb[warp * N + lane] = s;
+        }
+        __syncthreads();
+        if (threadIdx.x < N) {
+            double t = 0.0;
+#pragma unroll
+            for (int g = 0; g < NW; ++g) t += comb[g * N + threadIdx.x];
+            dots_step[(size_t)(threadIdx.x / PW) * n_panels * PW + panel * PW + (threadIdx.x % PW)] = t;
+        }
+        if (threadIdx.x == 0) tickets[panel] = 0u;
+    }
+    __syncthreads();  // scratch and is_last are free again
+}
 
 }  // namespace

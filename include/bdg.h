@@ -156,10 +156,11 @@ enum { BDG_MU_PER_COLUMN = 0, BDG_MU_SUM = 1 };
  * ELL  = FP64 warp-MMA on the kernel-native fixed-width row format (block rows of <= 8 blocks: every
  *        lattice Hamiltonian), one pass over the matrix serving up to 32 columns;
  * DMMA = FP64 warp-MMA on the BSR arrays as exported (any row length);
- * FMA  = scalar formulation (A/B reference); SIMPLE / CHUNKED = unpipelined DMMA with wavefront /
- *        per-CTA-chunk row traversal (tuning references). */
+ * FMA  = scalar formulation (A/B reference).
+ * 4 and 5 are unassigned: bdg_cheb_begin refuses them, and they are not to be reused, so that a caller built against an
+ * older header gets an error instead of another kernel. */
 enum { BDG_KERNEL_AUTO = 0, BDG_KERNEL_DMMA = 1, BDG_KERNEL_FMA = 2, BDG_KERNEL_ELL = 3,
-       BDG_KERNEL_DMMA_SIMPLE = 4, BDG_KERNEL_DMMA_CHUNKED = 5, BDG_KERNEL_DICT = 6, BDG_KERNEL_DICT_DIAG = 7,
+       BDG_KERNEL_DICT = 6, BDG_KERNEL_DICT_DIAG = 7,
        BDG_KERNEL_PAIR = 8, BDG_KERNEL_T2 = 9, BDG_KERNEL_AUTO_MOMENTS = 10 };
 
 /* Start a recursion on n_cols start vectors resident on this GPU.

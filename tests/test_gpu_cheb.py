@@ -439,6 +439,16 @@ def test_dictionary_format_declines_matrices_without_repetition(random_system):
     sysn.cheb_end()
 
 
+def test_unassigned_kernel_numbers_are_refused(random_system):
+    """4 and 5 name no kernel (include/bdg.h): bdg_cheb_begin refuses them like the numbers outside the enum."""
+    from bodge_b200 import _native
+
+    lib, sysn = _native.load(), random_system._sys
+    for kernel in (4, 5, -1, 11):
+        rc = lib.bdg_cheb_begin(sysn._h, _native.X0_RADEMACHER, 4, None, 1, 0, 10.0, kernel)
+        assert rc == _native.E_INVALID and f"unknown kernel {kernel}" in _native.last_error()
+
+
 def test_dictionary_format_with_every_block_distinct(gpu_api, monkeypatch):
     """Forced on a random matrix (table as large as the matrix): still exact."""
     monkeypatch.setenv("BDG_DICT_MAX_PERCENT", "100")

@@ -77,12 +77,12 @@ SYSTEMS = {
                                                              onsite_pairing=False), False),
 }
 
-# (BDG_PAIR_SEG, BDG_PAIR_P, BDG_PAIR_WARPS): None = planner's choice
-PLANS = [(None, None, None), (5, 7, None), (1, 1, None), (4, 30, 8), (3, 14, 8), (1000, 2, None), (6, 22, 12), (2, 5, 12)]
+# (BDG_PAIR_SEG, BDG_PAIR_P): None = planner's choice
+PLANS = [(None, None), (5, 7), (1, 1), (4, 30), (3, 14), (1000, 2), (6, 22), (2, 5)]
 
 
 def _set_plan(monkeypatch, plan):
-    for name, value in zip(("BDG_PAIR_SEG", "BDG_PAIR_P", "BDG_PAIR_WARPS"), plan):
+    for name, value in zip(("BDG_PAIR_SEG", "BDG_PAIR_P"), plan):
         if value is None:
             monkeypatch.delenv(name, raising=False)
         else:
@@ -282,8 +282,7 @@ def test_two_step_kernels_on_random_shapes_and_plans(monkeypatch):
         assert system.fill(*build(shape)) == 0.0
         scale = system.spectral_bound()
         plan = (int(rng.integers(1, Lx + 3)) if rng.random() < 0.7 else None,
-                int(rng.integers(1, 31)) if rng.random() < 0.7 else None,
-                (12 if rng.random() < 0.5 else 16) if rng.random() < 0.4 else None)
+                int(rng.integers(1, 31)) if rng.random() < 0.7 else None)
         _set_plan(monkeypatch, plan)
         n_cols, steps = int(rng.integers(1, 20)), int(rng.integers(1, 12))
         (cur, prev), fmt = _vectors(system._sys, "pair", n_cols, steps, scale)
