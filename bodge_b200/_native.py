@@ -63,6 +63,7 @@ SIGNATURES = {
     "bdg_cheb_vectors": [_vp, C.c_int, _vp],
     "bdg_cheb_info": [_vp, _i64p, _i64p, C.POINTER(C.c_int32), C.POINTER(C.c_int32), _i64p],
     "bdg_cheb_format": [_vp, C.POINTER(C.c_int32), _i64p, _i64p],
+    "bdg_cheb_launched": [_vp, C.c_char_p, C.c_int64, _i64p],
     "bdg_cheb_end": [_vp],
     "bdg_kpm_resolvent": [_vp, C.c_int32, C.c_int32, _vp, _vp, _vp, C.c_int],
     "bdg_kpm_contract": [_vp, C.c_int32, _vp, C.c_int, _vp, C.c_int],
@@ -376,6 +377,17 @@ class System:
         k, mb, nu = C.c_int32(), C.c_int64(), C.c_int64()
         check(load().bdg_cheb_format(self._h, C.byref(k), C.byref(mb), C.byref(nu)))
         return {"kernel": KERNEL_NAMES[k.value], "matrix_bytes_per_step": mb.value, "distinct_blocks": nu.value}
+
+    def cheb_launched(self) -> list[str]:
+        """Names of the recursion kernels the current recursion has launched (``bdg_cheb_launched``), as
+        ``cudaFuncGetName`` gives them, in the order of their first launch."""
+        lib = load()
+        needed = C.c_int64()
+        check(lib.bdg_cheb_launched(self._h, None, 0, C.byref(needed)))
+        buf = C.create_string_buffer(needed.value)
+        check(lib.bdg_cheb_launched(self._h, buf, needed.value, C.byref(needed)))
+        text = buf.value.decode("utf-8")
+        return text.split("\n") if text else []
 
     def cheb_info(self) -> dict:
         nb, by, la = C.c_int64(), C.c_int64(), C.c_int64()

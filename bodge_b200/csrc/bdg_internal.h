@@ -145,7 +145,19 @@ struct ChebState {
     int64_t local_reads = 0;
     DevBuf local_off;  // int64 [n_reads]: element offset of (site, col, alpha = 0) in the panel layout
     DevBuf local_acc;  // double2 [n_reads][4]
+    // Recursion kernels launched since bdg_cheb_begin (bdg_cheb_launched): distinct entry points in the order of their
+    // first launch.  `last_launched` makes a launch of the same kernel as the one before cost one compare.
+    std::vector<const void *> launched;
+    const void *last_launched = nullptr;
 };
+
+static inline void note_launch(ChebState &st, const void *kernel) {
+    if (kernel == st.last_launched) return;
+    st.last_launched = kernel;
+    for (const void *k : st.launched)
+        if (k == kernel) return;
+    st.launched.push_back(kernel);
+}
 
 // Kernel-native copy of the packed matrix for the ELL step kernel (cheb_ell.cu): every block row
 // padded to `width` slots, slot 0 = the diagonal block (zero block if absent), then the other

@@ -371,6 +371,7 @@ int launch_step(bdg_system *sys, bool first) {
         return local_accumulate(sys, slot + 1, x_io, nullptr);
     }
     StepKernel k = pick_kernel(st.kernel, st.panel_width, first, sys->packed_max_row);
+    note_launch(st, reinterpret_cast<const void *>(k));
     dim3 grid((unsigned)st.grid_x, (unsigned)st.n_panels);
     k<<<grid, kThreads, 0, sys->stream>>>(m.indptr.as<int32_t>(), m.indices.as<int32_t>(), m.data.as<double2>(), x_cur,
                                           x_io, (int)m.n_sites, (first ? 1.0 : 2.0) / st.scale,
@@ -542,6 +543,8 @@ extern "C" int bdg_cheb_begin(bdg_t *sys, int kind, int32_t n_cols, const int64_
     st.cube = cube;
     st.t2_rows_normalized = 0;
     st.local = false;
+    st.launched.clear();
+    st.last_launched = nullptr;
     st.dot_capacity = (int)(st.dots.bytes / ((size_t)2 * st.n_panels * st.panel_width * sizeof(double)));
 
     // Grid: enough CTAs to fill every SM at the kernel's occupancy, split over panels; each CTA
@@ -756,6 +759,25 @@ extern "C" int bdg_cheb_format(bdg_t *sys, int32_t *kernel, int64_t *matrix_byte
         else
             *matrix_bytes_per_step = 260 * m.n_blocks + 4 * (m.n_sites + 1);
     }
+    return BDG_OK;
+}
+
+extern "C" int bdg_cheb_launched(bdg_t *sys, char *names, int64_t capacity, int64_t *needed) {
+    BDG_ENTER(sys);
+    const ChebState &st = sys->cheb;
+    BDG_REQUIRE(st.active, "bdg_cheb_begin has not been called");
+    BDG_REQUIRE(needed != nullptr, "null argument");
+    std::string all;
+    for (const void *k : st.launched) {
+        const char *name = nullptr;
+        BDG_CUDA(cudaFuncGetName(&name, k));
+        if (!all.empty()) all += '\n';
+        all += name;
+    }
+    *needed = (int64_t)all.size() + 1;
+    if (!names) return BDG_OK;
+    BDG_REQUIRE(capacity >= *needed, "a buffer of %lld bytes is needed, %lld given", (long long)*needed, (long long)capacity);
+    std::memcpy(names, all.c_str(), all.size() + 1);
     return BDG_OK;
 }
 

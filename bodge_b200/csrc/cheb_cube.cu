@@ -552,7 +552,9 @@ int cube_launch(bdg_system *sys, bool first, const void *x_cur, void *x_io, doub
     const CubeShape shape = cube_shape(st.cube_shape);
     const bool listed = st.cube_walk.pieces != nullptr;
     dim3 grid((unsigned)st.cube_walk.n_ctas, listed ? 1u : (unsigned)st.n_panels);
-    (listed ? shape.listed : shape.kernel)<<<grid, shape.warps * 32, shape.smem, sys->stream>>>(
+    const CubeKernel k = listed ? shape.listed : shape.kernel;
+    note_launch(st, reinterpret_cast<const void *>(k));
+    k<<<grid, shape.warps * 32, shape.smem, sys->stream>>>(
         e.dcode3.as<int32_t>(), e.table.as<double>(), e.dtab.as<double>(), static_cast<const double2 *>(x_cur),
         static_cast<double2 *>(x_io), (int)e.n_sites, st.n_panels, 1.0 / st.scale, (first ? 2.0 : 4.0) / st.scale, first ? 1.0 : 2.0,
         first ? 1 : 0, st.partials.as<double>(), st.tickets.as<unsigned>(), dots_step, st.cube_walk);

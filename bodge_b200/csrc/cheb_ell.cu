@@ -544,12 +544,22 @@ template <bool DICT, bool DIAG, bool SD = false> EllKernel pick_shape(int pw, in
     }
 }
 
+// Two panels per pass: the plain format on 8-column panels with rows of >= 6 blocks (ell_configure), so only those widths
+// are built.
+EllKernel pick_two_panels(int width) {
+    switch (width) {
+        case 6: return cheb_step_ell<8, 6, 2, false, false, false>;
+        case 7: return cheb_step_ell<8, 7, 2, false, false, false>;
+        default: return cheb_step_ell<8, 8, 2, false, false, false>;
+    }
+}
+
 // fmt: BDG_KERNEL_ELL, BDG_KERNEL_DICT or BDG_KERNEL_DICT_DIAG; np: panels per pass (ell_configure); self_diag: DICT with
 // real-diagonal on-site blocks (SD)
 EllKernel pick_ell(int fmt, int pw, int np, int width, bool self_diag) {
     if (fmt == BDG_KERNEL_DICT_DIAG) return pick_shape<true, true>(pw, width);
     if (fmt == BDG_KERNEL_DICT) return self_diag ? pick_shape<true, false, true>(pw, width) : pick_shape<true, false>(pw, width);
-    return np == 2 ? pick_ch<8, 2, false, false, false>(width) : pick_shape<false, false>(pw, width);
+    return np == 2 ? pick_two_panels(width) : pick_shape<false, false>(pw, width);
 }
 
 bool ell_self_diag(const EllDev &e) { return e.self_diag_usable && env_int("BDG_ELL_SD", 1) != 0; }
@@ -801,7 +811,7 @@ int ell_configure(bdg_system *sys) {
     // dictionary workload measured (profiles/r01/quickperf_np_v2.log).  The plain kernel on 3-D
     // lattices (long rows: more block bytes per record byte) still gains from two panels per pass.
     const bool dict = st.kernel != BDG_KERNEL_ELL;
-    const bool pair = !dict && st.panel_width == 8 && st.n_panels >= 2 && e.width >= 6;
+    const bool pair = !dict && st.panel_width == 8 && st.n_panels >= 2 && e.width >= 6;  // (pick_two_panels)
     st.panels_per_group = pair ? 2 : 1;
     st.n_groups = (int)ceil_div(st.n_panels, st.panels_per_group);
     int per_sm = 1;
@@ -819,6 +829,7 @@ int ell_launch_step(bdg_system *sys, bool first, const void *x_cur, void *x_io, 
     const EllDev &e = sys->ell;
     const bool dict = st.kernel == BDG_KERNEL_DICT || st.kernel == BDG_KERNEL_DICT_DIAG;
     EllKernel k = pick_ell(st.kernel, st.panel_width, st.panels_per_group, e.width, ell_self_diag(e));
+    note_launch(st, reinterpret_cast<const void *>(k));
     // Stream the matrix through L2 (evict-first) only when nothing will read it again soon: one
     // group per pass and a matrix that cannot stay resident in the 126 MB L2 anyway.
     const size_t matrix_bytes = (size_t)e.n_sites * e.width * 260;

@@ -659,7 +659,9 @@ int pair_launch(bdg_system *sys, const void *x_prev, const void *x_cur, void *x_
     const EllDev &e = sys->ell;
     const bool listed = st.pair_walk.pieces != nullptr;
     dim3 grid((unsigned)st.pair_walk.n_ctas, listed ? 1u : (unsigned)st.n_panels);
-    pair_kernel(sys, false, listed)<<<grid, kPairThreads, kPairSmem, sys->stream>>>(
+    const PairKernel k = pair_kernel(sys, false, listed);
+    note_launch(st, reinterpret_cast<const void *>(k));
+    k<<<grid, kPairThreads, kPairSmem, sys->stream>>>(
         e.dcode.as<int32_t>(), e.table.as<double>(), e.dtab.as<double>(), static_cast<const double2 *>(x_prev),
         static_cast<const double2 *>(x_cur), static_cast<double2 *>(x_next1), static_cast<double2 *>(x_next2),
         (int)e.n_sites, st.n_panels, 2.0 / st.scale, 0.0, 0.0, 0, st.partials.as<double>(), st.tickets.as<unsigned>(), dots_step,
@@ -675,7 +677,9 @@ int t2_launch(bdg_system *sys, bool first, const void *x_cur, void *x_io, double
     const EllDev &e = sys->ell;
     const bool listed = st.pair_walk.pieces != nullptr;
     dim3 grid((unsigned)st.pair_walk.n_ctas, listed ? 1u : (unsigned)st.n_panels);
-    pair_kernel(sys, true, listed)<<<grid, kPairThreads, kPairSmem, sys->stream>>>(
+    const PairKernel k = pair_kernel(sys, true, listed);
+    note_launch(st, reinterpret_cast<const void *>(k));
+    k<<<grid, kPairThreads, kPairSmem, sys->stream>>>(
         e.dcode.as<int32_t>(), e.table.as<double>(), e.dtab.as<double>(), static_cast<const double2 *>(x_io),
         static_cast<const double2 *>(x_cur), nullptr, static_cast<double2 *>(x_io), (int)e.n_sites, st.n_panels,
         1.0 / st.scale, (first ? 2.0 : 4.0) / st.scale, first ? 1.0 : 2.0, first ? 1 : 0, st.partials.as<double>(), st.tickets.as<unsigned>(),

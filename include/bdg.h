@@ -207,6 +207,10 @@ int bdg_cheb_info(bdg_t *sys, int64_t *n_blocks, int64_t *bytes_per_step, int32_
  * *matrix_bytes_per_step = bytes of matrix data one step reads in that format (blocks or table +
  * codes + indices), *n_distinct_blocks = size of the block dictionary (0 if none was built). */
 int bdg_cheb_format(bdg_t *sys, int32_t *kernel, int64_t *matrix_bytes_per_step, int64_t *n_distinct_blocks);
+/* Which recursion kernels the current recursion has launched since bdg_cheb_begin (testing): their names as
+ * cudaFuncGetName reports them, newline-separated, each once, in the order of their first launch.  *needed = bytes of
+ * the NUL-terminated list; names = NULL only sets it, otherwise capacity must be >= *needed.  Host-side bookkeeping. */
+int bdg_cheb_launched(bdg_t *sys, char *names, int64_t capacity, int64_t *needed);
 int bdg_cheb_end(bdg_t *sys);
 
 /* ---- observables from the moments of the current recursion, evaluated on the device ----------
