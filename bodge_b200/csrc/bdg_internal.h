@@ -76,6 +76,17 @@ struct RowWalk {
     int prefetch = 0;            // rows ahead (a multiple of Ly*Lz) whose records are prefetched into L1; 0 = off
 };
 
+// Work lists of the two-applications-per-pass kernels (device, ChebState::work_items; work_lists.h): CTA c works through
+// pieces[cta_begin[c] .. cta_begin[c + 1]), a piece = (run, patch, x0, len).  A maximal sequence of pieces of one panel inside
+// a CTA is a "run": its dot products go to partials[run]; run_panel[run] = its panel, and the runs of panel p are
+// panel_runs[p] .. panel_runs[p + 1].  The classic plan has no lists (null pointers): n_ctas CTAs per panel, n_runs =
+// n_ctas x panels.
+struct WorkLists {
+    const int4 *pieces = nullptr;
+    const int *cta_begin = nullptr, *run_panel = nullptr, *panel_runs = nullptr;
+    int n_ctas = 0, n_runs = 0;
+};
+
 // Item grid of the two-steps-per-pass kernel (cheb_pair.cu): x-planes of M sites, cut into patches of
 // P owned sites; an item = (patch, segment of seg_len consecutive x), handed out segment-major.
 struct PairWalk {
@@ -83,12 +94,7 @@ struct PairWalk {
     int open = 0;  // the plane has open ends (no in-plane wrap-around block): the rim patches own their rim site
     int P = 1, n_patches = 1;
     int seg_len = 1, n_segs = 1, n_items = 1;
-    // Work lists (device, ChebState::work_items; work_lists.h): CTA c works through pieces[cta_begin[c] .. cta_begin[c + 1]), a
-    // piece = (run, patch, x0, len).  A maximal sequence of pieces of one panel inside a CTA is a "run": its dot products go to
-    // partials[run]; run_panel[run] = its panel, and the runs of panel p are panel_runs[p] .. panel_runs[p + 1].
-    const int4 *pieces = nullptr;
-    const int *cta_begin = nullptr, *run_panel = nullptr, *panel_runs = nullptr;
-    int n_ctas = 0, n_runs = 0;
+    WorkLists lists;
 };
 
 // Item grid of the two-applications-per-pass kernel for three-dimensional lattices (cheb_cube.cu): the (y, z) plane
@@ -97,13 +103,49 @@ struct CubeWalk {
     int Lx = 1, Ly = 1, Lz = 1;
     int nPy = 1, nPz = 1, n_patches = 1;
     int seg_len = 1, n_segs = 1, n_items = 1;
-    // work lists of a balanced plan (see PairWalk), null for the classic plan
-    const int4 *pieces = nullptr;
-    const int *cta_begin = nullptr, *run_panel = nullptr, *panel_runs = nullptr;
-    int n_ctas = 0, n_runs = 0;
+    WorkLists lists;
 };
 
 // ---- Chebyshev state ----------------------------------------------------------------------
+// Plan switches (INTEGRATION.md): member x_y holds BDG_X_Y.  bdg_cheb_begin reads them once (read_plan_switches, which
+// holds the defaults) and the configure functions plan from this copy, so they hold for the whole recursion.  Extents and
+// segment lengths: <= 0 = the planner's; pair_self, cube_shape and the balances: < 0 = the planner's.
+struct PlanSwitches {
+    bool auto_pair, auto_cube;
+    bool ell_sd, ell_walk;
+    int ell_pz, ell_seg, ell_prefetch;
+    int pair_self, pair_p, pair_seg, pair_balance;
+    bool pair_open;
+    int cube_shape, cube_seg, cube_balance;
+};
+
+// How the recursion advances; ChebState::kernel keeps the matrix format of the single-step kernel.
+enum class Stepping {
+    Single,     // one step per launch (cheb.cu, cheb_ell.cu)
+    Pair,       // two steps per launch whenever two or more remain (cheb_pair.cu); T_1 and odd leftovers: single-step kernel
+    EvenPlane,  // even-vector recursion E_{j+1} = 2 T_2(H~) E_j - E_{j-1} on one-dimensional x-planes (cheb_pair.cu)
+    EvenCube,   // ... on a three-dimensional lattice (cheb_cube.cu, 4-column panels)
+};
+
+// Signatures of the recursion kernel families: BSR (cheb.cu), fixed-width / dictionary (cheb_ell.cu), two steps per pass on
+// planes (cheb_pair.cu) and on three-dimensional lattices (cheb_cube.cu).
+using StepKernel = void (*)(const int32_t *, const int32_t *, const double2 *, const double2 *, double2 *, int, double,
+                            double, double *, unsigned *, double *, int);
+using EllKernel = void (*)(const int32_t *, const int32_t *, const double *, const double *, const double2 *, double2 *,
+                           int, int, double, double, int, int, double *, unsigned *, double *, const RowWalk);
+using PairKernel = void (*)(const int32_t *, const double *, const double *, const double2 *, const double2 *, double2 *,
+                            double2 *, int, int, double, double, double, int, double *, unsigned *, double *, const PairWalk);
+using CubeKernel = void (*)(const int32_t *, const double *, const double *, const double2 *, double2 *, int, int, double,
+                            double, double, int, double *, unsigned *, double *, const CubeWalk);
+
+// A kernel the plan chose and its launch shape: set by the configure functions, launched as is.
+template <class Kernel> struct Launch {
+    Kernel fn = nullptr;
+    dim3 grid;
+    unsigned threads = 0;
+    size_t smem = 0;
+};
+
 struct ChebState {
     bool active = false;
     int kernel = BDG_KERNEL_DMMA;
@@ -118,25 +160,27 @@ struct ChebState {
     // exist only then); the single-step kernels overwrite prev in place.
     DevBuf vec[4];
     int cur = 0, prev = 1;
-    bool pair = false;         // two steps per launch whenever two or more remain (cheb_pair.cu)
-    bool t2 = false;           // even-vector recursion E_{j+1} = 2 T_2(H~) E_j - E_{j-1}: vec[cur] = T_n, vec[prev] = T_{n-2}
+    Stepping stepping = Stepping::Single;  // even-vector recursions: vec[cur] = T_n, vec[prev] = T_{n-2}
+    bool even() const { return stepping == Stepping::EvenPlane || stepping == Stepping::EvenCube; }
     int t2_rows_normalized = 0;  // launches whose dot rows have been rewritten in the single-step format
-    int pair_grid_x = 0;
+    // What the plan launches (bdg_cheb_begin and the configure functions):
+    Launch<StepKernel> bsr_first, bsr_next;  // DMMA / FMA: T_1 and every later step
+    Launch<EllKernel> ell_step;              // ELL / DICT / DICT_DIAG: every single step
+    Launch<PairKernel> two_step;             // Pair / EvenPlane
+    Launch<CubeKernel> cube_step;            // EvenCube
+    RowWalk walk;                            // ell_step's row traversal
     PairWalk pair_walk;
-    bool cube = false;         // t2 on a three-dimensional lattice: cheb_cube.cu (4-column panels)
-    int cube_shape = 0;        // which patch shape of cheb_cube.cu
     CubeWalk cube_walk;
+    bool onsite_per_row = false;  // two_step: on-site fragments fetched per row from the table (SELF) instead of held
+    bool onsite_diag = false;     // two_step: real-diagonal on-site product (SD)
+    int partial_runs = 0;         // the most partial-sum slots (runs) per panel any launch of the plan writes
     // dots[(step * 2 + which) * n_panels * PW + panel * PW + c]; which 0 = <T_n,T_n>, 1 = <T_{n+1},T_n>
     DevBuf dots;
     DevBuf partials;  // per-CTA partial dot products of the step in flight
     DevBuf tickets;   // uint32 [n_panels] arrival counters (last CTA reduces)
     DevBuf mu_tmp;    // staging for moment read-out
     DevBuf obs_tmp;   // staging for observables.cu (coefficients, energies, results)
-    DevBuf work_items;  // work lists of the two-step kernel (PairWalk)
-    int grid_x = 0;
-    int panels_per_group = 1;  // ELL kernel: panels sharing one pass over the matrix (grid.y = groups)
-    int n_groups = 0;
-    RowWalk walk;              // ELL / DICT kernels: row traversal
+    DevBuf work_items;  // work lists of a balanced plan (WorkLists)
     int64_t launches = 0;
     // Local accumulator (bdg_cheb_local_begin, observables.cu): every launch that writes T_n with n < local_coef.size()
     // adds local_coef[n] * T_n[4 site + alpha][col] to local_acc[read][alpha].  Cleared by bdg_cheb_begin.
@@ -245,7 +289,7 @@ int local_accumulate(bdg_system *sys, int n, const void *x_a, const void *x_b);
 
 // cheb_ell.cu
 int ell_build(bdg_system *sys);                    // (re)build sys->ell from sys->packed when stale
-int ell_configure(bdg_system *sys);                // pick panels_per_group / grid for the current ChebState
+int ell_configure(bdg_system *sys, const PlanSwitches &sw);  // ChebState::ell_step and its row traversal
 int ell_launch_step(bdg_system *sys, bool first, const void *x_cur, void *x_io, double *dots_step);
 // After a scatter: bring `packed` and the kernel-native copies (fixed-width rows, dictionary, direction codes) up to date
 // for the `n` skeleton blocks listed in `klist` (device; < 0 = skip) instead of rebuilding them.  *ok = false: the zero
@@ -255,19 +299,18 @@ void ell_release(bdg_system *sys);
 
 // cheb_pair.cu
 int pair_probe(bdg_system *sys);      // sets sys->ell.pair_usable / pair_M (called by ell_build)
-int pair_configure(bdg_system *sys);  // patch / segment plan and grid for the current ChebState
+int pair_configure(bdg_system *sys, const PlanSwitches &sw);  // ChebState::two_step and its patch / segment plan
 int pair_launch(bdg_system *sys, const void *x_prev, const void *x_cur, void *x_next1, void *x_next2, double *dots_step);
 int t2_launch(bdg_system *sys, bool first, const void *x_cur, void *x_io, double *dots_step);
-bool pair_streams_onsite(const bdg_system *sys);  // on-site fragments fetched per row (large dictionaries) instead of held
 
 // cheb_cube.cu
 int cube_probe(bdg_system *sys);      // sets sys->ell.cube_usable / dcode3 (called by ell_build)
-int cube_configure(bdg_system *sys);  // patch shape / segment plan and grid for the current ChebState
+int cube_configure(bdg_system *sys, const PlanSwitches &sw);  // ChebState::cube_step: patch shape, segment plan
 int cube_launch(bdg_system *sys, bool first, const void *x_cur, void *x_io, double *dots_step);
 
 static inline int64_t ceil_div(int64_t a, int64_t b) { return (a + b - 1) / b; }
 
-// Integer switch from the environment (plan and kernel overrides, INTEGRATION.md); unset or empty: `fallback`.
+// Integer switch from the environment (INTEGRATION.md); unset or empty: `fallback`.
 static inline int env_int(const char *name, int fallback) {
     const char *v = getenv(name);
     return v && *v ? atoi(v) : fallback;

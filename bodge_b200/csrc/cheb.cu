@@ -331,9 +331,6 @@ unpack_vectors(const double2 *__restrict__ x, int n_sites, int pw, int n_cols, d
     out[t] = x[(((size_t)(c / pw) * n_sites + site) * pw + (c % pw)) * 4 + alpha];
 }
 
-using StepKernel = void (*)(const int32_t *, const int32_t *, const double2 *, const double2 *, double2 *, int, double,
-                            double, double *, unsigned *, double *, int);
-
 template <int PW> StepKernel pick_pw(int kernel, bool first, int max_row) {
     if (kernel == BDG_KERNEL_FMA) return first ? cheb_step_fma<PW, true> : cheb_step_fma<PW, false>;
     if (max_row <= 3) return first ? cheb_step_dmma<PW, true, 3> : cheb_step_dmma<PW, false, 3>;
@@ -351,10 +348,52 @@ StepKernel pick_kernel(int kernel, int pw, bool first, int max_row) {
     }
 }
 
-// AUTO prefers the two-steps-per-pass kernel wherever it applies (BDG_AUTO_PAIR=0 turns that off).
-bool auto_pair_enabled() { return env_int("BDG_AUTO_PAIR", kAutoPairDefault) != 0; }
-// ... and, for callers that only read moments, the even-vector recursion on three-dimensional lattices (BDG_AUTO_CUBE=0: off)
-bool auto_cube_enabled() { return env_int("BDG_AUTO_CUBE", 1) != 0; }
+// Every plan switch (PlanSwitches), read once per recursion.
+PlanSwitches read_plan_switches() {
+    // BDG_ELL_PZ, BDG_PAIR_P: a set value counts as at least 1; unset or empty: 0
+    const auto extent = [](const char *name) {
+        const char *v = getenv(name);
+        return v && *v ? std::max(1, atoi(v)) : 0;
+    };
+    PlanSwitches s;
+    s.auto_pair = env_int("BDG_AUTO_PAIR", kAutoPairDefault) != 0;
+    s.auto_cube = env_int("BDG_AUTO_CUBE", 1) != 0;
+    s.ell_sd = env_int("BDG_ELL_SD", 1) != 0;
+    s.ell_walk = env_int("BDG_ELL_WALK", 1) != 0;
+    s.ell_pz = extent("BDG_ELL_PZ");
+    s.ell_seg = env_int("BDG_ELL_SEG", 0);
+    s.ell_prefetch = env_int("BDG_ELL_PREFETCH", 1);
+    s.pair_self = env_int("BDG_PAIR_SELF", -1);
+    s.pair_open = env_int("BDG_PAIR_OPEN", 1) != 0;
+    s.pair_p = extent("BDG_PAIR_P");
+    s.pair_seg = env_int("BDG_PAIR_SEG", 0);
+    s.pair_balance = env_int("BDG_PAIR_BALANCE", -1);
+    s.cube_shape = env_int("BDG_CUBE_SHAPE", -1);
+    s.cube_seg = env_int("BDG_CUBE_SEG", 0);
+    s.cube_balance = env_int("BDG_CUBE_BALANCE", -1);
+    return s;
+}
+
+bool ell_format(int kernel) { return kernel == BDG_KERNEL_ELL || kernel == BDG_KERNEL_DICT || kernel == BDG_KERNEL_DICT_DIAG; }
+
+// DMMA / FMA: the FIRST and the next-step kernel on one grid -- enough CTAs to fill every SM at the kernel's occupancy, split
+// over panels; each CTA walks one contiguous range of block rows (neighbouring rows share their X records in L1).
+int bsr_configure(bdg_system *sys) {
+    ChebState &st = sys->cheb;
+    const StepKernel next = pick_kernel(st.kernel, st.panel_width, false, sys->packed_max_row);
+    int per_sm = 1;
+    BDG_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, next, kThreads, 0));
+    per_sm = std::max(per_sm, 1);
+    const int64_t target = (int64_t)sys->sm_count * per_sm;
+    int64_t gx = std::max<int64_t>(1, target / st.n_panels);
+    const int rows_per_warp_pass = st.kernel == BDG_KERNEL_FMA ? kWarps * (32 / st.panel_width) : kWarps;
+    gx = std::min<int64_t>(gx, ceil_div(sys->packed.n_sites, rows_per_warp_pass));
+    const dim3 grid((unsigned)gx, (unsigned)st.n_panels);
+    st.bsr_first = {pick_kernel(st.kernel, st.panel_width, true, sys->packed_max_row), grid, kThreads, 0};
+    st.bsr_next = {next, grid, kThreads, 0};
+    st.partial_runs = std::max(st.partial_runs, (int)gx);
+    return BDG_OK;
+}
 
 int launch_step(bdg_system *sys, bool first) {
     ChebState &st = sys->cheb;
@@ -364,20 +403,17 @@ int launch_step(bdg_system *sys, bool first) {
     double *dots_step = st.dots.as<double>() + (size_t)slot * 2 * stride;
     const double2 *x_cur = st.vec[st.cur].as<double2>();
     double2 *x_io = st.vec[st.prev].as<double2>();
-    if (st.kernel == BDG_KERNEL_ELL || st.kernel == BDG_KERNEL_DICT || st.kernel == BDG_KERNEL_DICT_DIAG) {
+    if (ell_format(st.kernel)) {
         BDG_TRY(ell_launch_step(sys, first, x_cur, x_io, dots_step));
-        std::swap(st.cur, st.prev);
-        st.launches += 1;
-        return local_accumulate(sys, slot + 1, x_io, nullptr);
+    } else {
+        const Launch<StepKernel> &l = first ? st.bsr_first : st.bsr_next;
+        note_launch(st, reinterpret_cast<const void *>(l.fn));
+        l.fn<<<l.grid, l.threads, l.smem, sys->stream>>>(m.indptr.as<int32_t>(), m.indices.as<int32_t>(), m.data.as<double2>(), x_cur,
+                                                         x_io, (int)m.n_sites, (first ? 1.0 : 2.0) / st.scale,
+                                                         first ? 0.0 : 1.0, st.partials.as<double>(), st.tickets.as<unsigned>(),
+                                                         dots_step, st.n_panels);
+        BDG_CUDA(cudaGetLastError());
     }
-    StepKernel k = pick_kernel(st.kernel, st.panel_width, first, sys->packed_max_row);
-    note_launch(st, reinterpret_cast<const void *>(k));
-    dim3 grid((unsigned)st.grid_x, (unsigned)st.n_panels);
-    k<<<grid, kThreads, 0, sys->stream>>>(m.indptr.as<int32_t>(), m.indices.as<int32_t>(), m.data.as<double2>(), x_cur,
-                                          x_io, (int)m.n_sites, (first ? 1.0 : 2.0) / st.scale,
-                                          first ? 0.0 : 1.0, st.partials.as<double>(), st.tickets.as<unsigned>(),
-                                          dots_step, st.n_panels);
-    BDG_CUDA(cudaGetLastError());
     std::swap(st.cur, st.prev);
     st.launches += 1;
     return local_accumulate(sys, slot + 1, x_io, nullptr);  // x_io now holds T_{slot+1}
@@ -423,7 +459,7 @@ int ensure_dot_capacity(bdg_system *sys, int steps_total) {
 // T2 mode: bring the dot rows written since the last call into the single-step format (t2_normalize).
 int t2_finish_dots(bdg_system *sys) {
     ChebState &st = sys->cheb;
-    if (!st.t2 || !st.active) return BDG_OK;
+    if (!st.even() || !st.active) return BDG_OK;
     const int launches = (st.steps_done + 1) / 2;  // rows = 2 (steps_done + 1) = 4 per launch
     if (st.t2_rows_normalized >= launches) return BDG_OK;
     const int stride = st.n_panels * st.panel_width;
@@ -472,7 +508,8 @@ extern "C" int bdg_cheb_begin(bdg_t *sys, int kind, int32_t n_cols, const int64_
     BDG_REQUIRE(kernel >= BDG_KERNEL_AUTO && kernel <= BDG_KERNEL_AUTO_MOMENTS && kernel != 4 && kernel != 5,  // 4, 5: unassigned (bdg.h)
                 "unknown kernel %d", kernel);
     BDG_TRY(build_packed(sys));
-    bool pair = false, t2 = false, cube = false;
+    const PlanSwitches sw = read_plan_switches();
+    Stepping stepping = Stepping::Single;
     if (kernel == BDG_KERNEL_AUTO || kernel == BDG_KERNEL_ELL || kernel == BDG_KERNEL_DICT || kernel == BDG_KERNEL_DICT_DIAG ||
         kernel == BDG_KERNEL_PAIR || kernel == BDG_KERNEL_T2 || kernel == BDG_KERNEL_AUTO_MOMENTS) {
         BDG_TRY(ell_build(sys));
@@ -498,16 +535,18 @@ extern "C" int bdg_cheb_begin(bdg_t *sys, int kind, int32_t n_cols, const int64_
         // diagonal hopping blocks (DFMA), general hopping blocks next to real-diagonal on-site blocks (SD: d-wave / Rashba
         // models, +12..44 % over the single-step kernel) and rows of ten MMAs (+22..42 % at 8 columns, +24..32 % at >= 64
         // columns on 10^6 sites, level at C3 with 64..512 columns).
-        const bool prefer = pair_ok && auto_pair_enabled();
+        const bool prefer = pair_ok && sw.auto_pair;
         // Callers that only read moments / observables get the even-vector recursion (three vector passes per
         // two steps); callers that step and look at T_n, T_{n-1} the pair kernel (four).
         // ... preferred where its items fill the machine without cutting x into segments (one CTA per SM marches an 8 x 8 patch:
         // C4 = 64 patches x 2 panels); on smaller lattices the single-step kernel's finer grid wins.
         const int64_t cube_items = ceil_div(sys->cubic[1], 8) * ceil_div(sys->cubic[2], 8) * ceil_div(n_cols, 4);
-        const bool prefer_cube = cube_ok && auto_cube_enabled() && 4 * cube_items >= 3 * (int64_t)sys->sm_count;
-        t2 = kernel == BDG_KERNEL_T2 || (kernel == BDG_KERNEL_AUTO_MOMENTS && (prefer || prefer_cube));
-        cube = t2 && !pair_ok && cube_ok;
-        pair = kernel == BDG_KERNEL_PAIR || (kernel == BDG_KERNEL_AUTO && prefer);
+        const bool prefer_cube = cube_ok && sw.auto_cube && 4 * cube_items >= 3 * (int64_t)sys->sm_count;
+        // (the even-vector recursion without pair_ok has cube_ok: the requirement above, or prefer_cube)
+        if (kernel == BDG_KERNEL_T2 || (kernel == BDG_KERNEL_AUTO_MOMENTS && (prefer || prefer_cube)))
+            stepping = pair_ok ? Stepping::EvenPlane : Stepping::EvenCube;
+        else if (kernel == BDG_KERNEL_PAIR || (kernel == BDG_KERNEL_AUTO && prefer))
+            stepping = Stepping::Pair;
         if (kernel == BDG_KERNEL_PAIR || kernel == BDG_KERNEL_T2 || kernel == BDG_KERNEL_AUTO_MOMENTS) kernel = BDG_KERNEL_AUTO;
         BDG_REQUIRE(kernel != BDG_KERNEL_ELL || sys->ell.usable,
                     "the fixed-width (ELL) kernel needs block rows of <= 8 blocks with little padding");
@@ -532,46 +571,31 @@ extern "C" int bdg_cheb_begin(bdg_t *sys, int kind, int32_t n_cols, const int64_
     st.active = false;
     st.kernel = kernel;
     st.n_cols = n_cols;
-    st.panel_width = cube ? 4 : (n_cols >= 5 || pair || t2) ? 8 : (n_cols >= 3 ? 4 : n_cols);
+    st.stepping = stepping;
+    st.panel_width = stepping == Stepping::EvenCube ? 4 : (n_cols >= 5 || stepping != Stepping::Single) ? 8 : (n_cols >= 3 ? 4 : n_cols);
     st.n_panels = (int)ceil_div(n_cols, st.panel_width);
     st.scale = scale;
     st.steps_done = 0;
     st.cur = 0;
     st.prev = 1;
-    st.pair = pair;
-    st.t2 = t2;
-    st.cube = cube;
     st.t2_rows_normalized = 0;
     st.local = false;
     st.launched.clear();
     st.last_launched = nullptr;
     st.dot_capacity = (int)(st.dots.bytes / ((size_t)2 * st.n_panels * st.panel_width * sizeof(double)));
 
-    // Grid: enough CTAs to fill every SM at the kernel's occupancy, split over panels; each CTA
-    // walks one contiguous range of block rows (neighbouring rows share their X records in L1).
-    if (st.kernel == BDG_KERNEL_ELL || st.kernel == BDG_KERNEL_DICT || st.kernel == BDG_KERNEL_DICT_DIAG) {
-        BDG_TRY(ell_configure(sys));
-    } else {
-        int per_sm = 1;
-        BDG_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, pick_kernel(st.kernel, st.panel_width, false, sys->packed_max_row), kThreads, 0));
-        per_sm = std::max(per_sm, 1);
-        const int64_t target = (int64_t)sys->sm_count * per_sm;
-        int64_t gx = std::max<int64_t>(1, target / st.n_panels);
-        const int rows_per_warp_pass = st.kernel == BDG_KERNEL_FMA ? kWarps * (32 / st.panel_width) : kWarps;
-        gx = std::min<int64_t>(gx, ceil_div(n, rows_per_warp_pass));
-        st.grid_x = (int)gx;
-        st.panels_per_group = 1;
-        st.n_groups = st.n_panels;
-    }
-
-    st.pair_grid_x = 0;
-    if (st.cube) BDG_TRY(cube_configure(sys));
-    else if (st.pair || st.t2) BDG_TRY(pair_configure(sys));
+    // The kernels the recursion will launch: the single-step kernel (every step, or T_1 and odd leftovers of the pair
+    // plan), the two-step kernel, or the even-vector one.
+    st.partial_runs = 0;
+    if (stepping == Stepping::Single || stepping == Stepping::Pair)
+        BDG_TRY(ell_format(st.kernel) ? ell_configure(sys, sw) : bsr_configure(sys));
+    if (stepping == Stepping::Pair || stepping == Stepping::EvenPlane) BDG_TRY(pair_configure(sys, sw));
+    if (stepping == Stepping::EvenCube) BDG_TRY(cube_configure(sys, sw));
 
     const size_t vec_elems = (size_t)st.n_panels * n * st.panel_width * 4;
-    for (int b = 0; b < (st.pair ? 4 : 2); ++b) BDG_TRY(dev_alloc(sys, st.vec[b], vec_elems * sizeof(double2)));
+    for (int b = 0; b < (stepping == Stepping::Pair ? 4 : 2); ++b) BDG_TRY(dev_alloc(sys, st.vec[b], vec_elems * sizeof(double2)));
     BDG_TRY(dev_alloc(sys, st.partials,
-                      (size_t)st.n_panels * std::max(st.grid_x, st.pair_grid_x) * (st.pair || st.t2 ? 32 : 16) * sizeof(double)));
+                      (size_t)st.n_panels * st.partial_runs * (stepping == Stepping::Single ? 16 : 32) * sizeof(double)));
     BDG_TRY(dev_alloc(sys, st.tickets, (size_t)st.n_panels * sizeof(unsigned)));
     BDG_CUDA(cudaMemsetAsync(st.tickets.ptr, 0, (size_t)st.n_panels * sizeof(unsigned), sys->stream));
     BDG_TRY(ensure_dot_capacity(sys, 1024));
@@ -591,7 +615,7 @@ extern "C" int bdg_cheb_begin(bdg_t *sys, int kind, int32_t n_cols, const int64_
     }
     BDG_CUDA(cudaGetLastError());
     st.launches += 1;
-    if (st.t2) {
+    if (st.even()) {
         // E_1 = T_2(H~) E_0 into vec[1] and the dot products of steps 0 and 1 (moments 0..3): one step done.
         BDG_TRY(ensure_dot_capacity(sys, 2));
         BDG_TRY(t2_launch(sys, true, st.vec[0].ptr, st.vec[1].ptr, st.dots.as<double>()));
@@ -628,7 +652,7 @@ extern "C" int bdg_cheb_steps(bdg_t *sys, int32_t n_steps, float *elapsed_ms) {
         BDG_CUDA(cudaEventRecord(e0, sys->stream));
     }
     for (int s = 0; s < n_steps;) {
-        if (st.t2) {  // two steps per launch, always: an odd request is rounded up (moments-only mode)
+        if (st.even()) {  // two steps per launch, always: an odd request is rounded up (moments-only mode)
             const int stride = st.n_panels * st.panel_width;
             BDG_TRY(ensure_dot_capacity(sys, st.steps_done + 2));
             BDG_TRY(t2_launch(sys, false, st.vec[st.cur].ptr, st.vec[st.prev].ptr,
@@ -637,7 +661,7 @@ extern "C" int bdg_cheb_steps(bdg_t *sys, int32_t n_steps, float *elapsed_ms) {
             st.launches += 1;
             st.steps_done += 2;
             s += 2;
-        } else if (st.pair && n_steps - s >= 2) {
+        } else if (st.stepping == Stepping::Pair && n_steps - s >= 2) {
             BDG_TRY(launch_pair(sys));
             st.steps_done += 2;
             s += 2;
@@ -709,7 +733,7 @@ extern "C" int bdg_cheb_vectors(bdg_t *sys, int which, double *out) {
     ChebState &st = sys->cheb;
     BDG_REQUIRE(st.active && out, "no active recursion or null output");
     BDG_REQUIRE(which == 0 || which == 1, "which must be 0 (T_n) or 1 (T_{n-1})");
-    BDG_REQUIRE(which == 0 || !st.t2, "the even-vector recursion (kernel T2) keeps T_n and T_{n-2}, not T_{n-1}");
+    BDG_REQUIRE(which == 0 || !st.even(), "the even-vector recursion (kernel T2) keeps T_n and T_{n-2}, not T_{n-1}");
     const BsrDev &m = sys->packed;
     const size_t count = (size_t)m.n_sites * 4 * st.n_cols;
     DevBuf tmp;
@@ -744,14 +768,14 @@ extern "C" int bdg_cheb_format(bdg_t *sys, int32_t *kernel, int64_t *matrix_byte
     BDG_REQUIRE(st.active, "bdg_cheb_begin has not been called");
     const BsrDev &m = sys->packed;
     const EllDev &e = sys->ell;
-    if (kernel) *kernel = st.t2 ? BDG_KERNEL_T2 : st.pair ? BDG_KERNEL_PAIR : st.kernel;
+    if (kernel) *kernel = st.even() ? BDG_KERNEL_T2 : st.stepping == Stepping::Pair ? BDG_KERNEL_PAIR : st.kernel;
     if (n_distinct_blocks) *n_distinct_blocks = e.valid ? e.n_unique : 0;
     if (matrix_bytes_per_step) {
-        if (st.cube)  // eight 4-byte codes per site, read once per panel and launch (= two steps)
+        if (st.stepping == Stepping::EvenCube)  // eight 4-byte codes per site, read once per panel and launch (= two steps)
             *matrix_bytes_per_step = e.n_sites * 32 * st.n_panels / 2 + e.n_unique * 256;
-        else if (st.pair || st.t2)  // one pass over the codes (and, site-dependent on-site blocks: over those) serves two steps
-            *matrix_bytes_per_step = e.n_sites * 5 * 4 / 2 + (pair_streams_onsite(sys) ? std::min(e.n_unique, e.n_sites) * (e.self_diag_usable && !e.diag_usable ? 32 : 256) / 2
-                                                                                        : e.n_unique * 256);
+        else if (st.stepping != Stepping::Single)  // one pass over the codes (and, site-dependent on-site blocks: over those) serves two steps
+            *matrix_bytes_per_step = e.n_sites * 5 * 4 / 2 + (st.onsite_per_row ? std::min(e.n_unique, e.n_sites) * (st.onsite_diag ? 32 : 256) / 2
+                                                                                  : e.n_unique * 256);
         else if (st.kernel == BDG_KERNEL_DICT || st.kernel == BDG_KERNEL_DICT_DIAG)
             *matrix_bytes_per_step = e.n_sites * e.width * 8 + e.n_unique * 256;
         else if (st.kernel == BDG_KERNEL_ELL)

@@ -182,19 +182,19 @@ cheb_cube_step(const int32_t *__restrict__ dcode, const double *__restrict__ tab
     const bool code_lane = lane < 16 && (lane & 7) < 7;
     const int cs = lane >> 3, cu = lane & 7;  // code lanes: site of the pair, direction
 
-    const int item0 = LISTED ? wk.cta_begin[blockIdx.x] : (int)blockIdx.x, item1 = LISTED ? wk.cta_begin[blockIdx.x + 1] : wk.n_items;
+    const int item0 = LISTED ? wk.lists.cta_begin[blockIdx.x] : (int)blockIdx.x, item1 = LISTED ? wk.lists.cta_begin[blockIdx.x + 1] : wk.n_items;
     for (int item = item0; item < item1; item += LISTED ? 1 : (int)gridDim.x) {
         int4 piece;  // panel, patch, x0, len
         if (LISTED) {
-            piece = wk.pieces[item];  // (run, patch, x0, len)
+            piece = wk.lists.pieces[item];  // (run, patch, x0, len)
             if (piece.x != run) {
                 if (run >= 0) {
-                    flush_dots<NW, 4>(d0, d1, d2, d3, cube_smem, run, wk.panel_runs[panel], wk.panel_runs[panel + 1], panel, n_panels, partials,
+                    flush_dots<NW, 4>(d0, d1, d2, d3, cube_smem, run, wk.lists.panel_runs[panel], wk.lists.panel_runs[panel + 1], panel, n_panels, partials,
                                       tickets, dots_step);
                     d0 = d1 = d2 = d3 = 0.0;
                 }
                 run = piece.x;
-                panel = wk.run_panel[run];
+                panel = wk.lists.run_panel[run];
             }
             piece.x = panel;
         } else {
@@ -394,7 +394,7 @@ cheb_cube_step(const int32_t *__restrict__ dcode, const double *__restrict__ tab
 
     if (LISTED) {
         if (panel >= 0)
-            flush_dots<NW, 4>(d0, d1, d2, d3, cube_smem, run, wk.panel_runs[panel], wk.panel_runs[panel + 1], panel, n_panels, partials, tickets,
+            flush_dots<NW, 4>(d0, d1, d2, d3, cube_smem, run, wk.lists.panel_runs[panel], wk.lists.panel_runs[panel + 1], panel, n_panels, partials, tickets,
                               dots_step);
     } else {
         const int p = (int)blockIdx.y, r0 = p * (int)gridDim.x;
@@ -434,9 +434,6 @@ cube_codes(int n_sites, int width, int Ly, int Lz, const int32_t *__restrict__ c
 #pragma unroll
     for (int k = 0; k < kCodeStride; ++k) dcode[(size_t)row * kCodeStride + k] = out[k];
 }
-
-using CubeKernel = void (*)(const int32_t *, const double *, const double *, const double2 *, double2 *, int, int, double,
-                            double, double, int, double *, unsigned *, double *, const CubeWalk);
 
 struct CubeShape {
     int warps, py, pz, ne;
@@ -496,19 +493,19 @@ int cube_probe(bdg_system *sys) {
 
 // Patch shape, segment length and grid for the current recursion: the plan with the fewest body rounds on the
 // critical path (waves x planes per item x bodies per warp and plane).
-int cube_configure(bdg_system *sys) {
+int cube_configure(bdg_system *sys, const PlanSwitches &sw) {
     ChebState &st = sys->cheb;
     const int Lx = sys->cubic[0], Ly = sys->cubic[1], Lz = sys->cubic[2];
     const int64_t slots = std::max<int64_t>(1, (int64_t)sys->sm_count / st.n_panels);
-    const int forced_shape = env_int("BDG_CUBE_SHAPE", -1), forced_seg = env_int("BDG_CUBE_SEG", 0);
     double best = -1.0;
+    int chosen = 0;
     for (int which = 0; which < kCubeShapes; ++which) {
-        if (forced_shape >= 0 && which != forced_shape) continue;
+        if (sw.cube_shape >= 0 && which != sw.cube_shape) continue;
         const CubeShape shape = cube_shape(which);
         const int nPy = (int)ceil_div(Ly, shape.py), nPz = (int)ceil_div(Lz, shape.pz);
         const int64_t patches = (int64_t)nPy * nPz;
         for (int n_seg = 1; n_seg <= std::max(1, Lx / 4); ++n_seg) {
-            const int len = forced_seg > 0 ? std::min(forced_seg, Lx) : (int)ceil_div(Lx, n_seg);
+            const int len = sw.cube_seg > 0 ? std::min(sw.cube_seg, Lx) : (int)ceil_div(Lx, n_seg);
             const int64_t segs = ceil_div(Lx, len), items = patches * segs;
             const double cost = (double)ceil_div(items, slots) * (len + 4.0) * shape.rounds;
             if (best < 0.0 || cost < best) {
@@ -517,31 +514,23 @@ int cube_configure(bdg_system *sys) {
                 w.Lx = Lx, w.Ly = Ly, w.Lz = Lz;
                 w.nPy = nPy, w.nPz = nPz, w.n_patches = (int)patches;
                 w.seg_len = len, w.n_segs = (int)segs, w.n_items = (int)items;
-                st.cube_shape = which;
+                chosen = which;
             }
-            if (forced_seg > 0) break;
+            if (sw.cube_seg > 0) break;
         }
     }
-    const CubeShape shape = cube_shape(st.cube_shape);
-    BDG_CUDA(cudaFuncSetAttribute(shape.kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)shape.smem));
-    BDG_CUDA(cudaFuncSetAttribute(shape.listed, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)shape.smem));
     CubeWalk &w = st.cube_walk;
-    const int gx = (int)std::min<int64_t>(slots, w.n_items);
-    w.pieces = nullptr, w.cta_begin = w.run_panel = w.panel_runs = nullptr;
-    w.n_ctas = gx, w.n_runs = gx * st.n_panels;
-    st.pair_grid_x = gx;
-    // Balanced plan (cheb_pair.cu: pair_configure): one contiguous chunk of the (panel, patch, x) space per SM instead of
-    // whole patch columns -- C4 with 8 columns is 128 columns of 64 planes on 148 SMs.
+    // Balanced plan: one contiguous chunk of the (panel, patch, x) space per SM instead of whole patch columns -- C4 with 8
+    // columns is 128 columns of 64 planes on 148 SMs.
     constexpr int kPieceCost = 6;
-    const double classic_cost = (double)ceil_div((int64_t)gx * st.n_panels, (int64_t)sys->sm_count) * (double)ceil_div(w.n_items, gx) * (w.seg_len + kPieceCost);
-    const WorkPlan plan = best_balanced_plan(st.n_panels, w.n_patches, Lx, sys->sm_count, kPieceCost, 1.0);
-    const int force = env_int("BDG_CUBE_BALANCE", -1);
-    if (!(force >= 0 ? force != 0 : plan.longest < 0.93 * classic_cost)) return BDG_OK;
-    WorkLists lists;
-    BDG_TRY(upload_work_lists(sys, st.work_items, plan, st.n_panels, lists));
-    w.pieces = lists.pieces, w.cta_begin = lists.cta_begin, w.run_panel = lists.run_panel, w.panel_runs = lists.panel_runs;
-    w.n_ctas = lists.n_ctas, w.n_runs = lists.n_runs;
-    st.pair_grid_x = (int)ceil_div(lists.n_runs, st.n_panels);  // (sizes the partial-sum buffer)
+    BDG_TRY(choose_work_plan(sys, st.work_items, st.n_panels, w.n_patches, Lx, w.seg_len, w.n_items, sys->sm_count, kPieceCost, 1.0,
+                             sw.cube_balance, w.lists));
+    const CubeShape shape = cube_shape(chosen);
+    const bool listed = w.lists.pieces != nullptr;
+    const CubeKernel k = listed ? shape.listed : shape.kernel;
+    BDG_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)shape.smem));
+    st.cube_step = {k, dim3((unsigned)w.lists.n_ctas, listed ? 1u : (unsigned)st.n_panels), (unsigned)shape.warps * 32, shape.smem};
+    st.partial_runs = std::max(st.partial_runs, (int)ceil_div(w.lists.n_runs, st.n_panels));
     return BDG_OK;
 }
 
@@ -549,12 +538,9 @@ int cube_configure(bdg_system *sys) {
 int cube_launch(bdg_system *sys, bool first, const void *x_cur, void *x_io, double *dots_step) {
     ChebState &st = sys->cheb;
     const EllDev &e = sys->ell;
-    const CubeShape shape = cube_shape(st.cube_shape);
-    const bool listed = st.cube_walk.pieces != nullptr;
-    dim3 grid((unsigned)st.cube_walk.n_ctas, listed ? 1u : (unsigned)st.n_panels);
-    const CubeKernel k = listed ? shape.listed : shape.kernel;
-    note_launch(st, reinterpret_cast<const void *>(k));
-    k<<<grid, shape.warps * 32, shape.smem, sys->stream>>>(
+    const Launch<CubeKernel> &l = st.cube_step;
+    note_launch(st, reinterpret_cast<const void *>(l.fn));
+    l.fn<<<l.grid, l.threads, l.smem, sys->stream>>>(
         e.dcode3.as<int32_t>(), e.table.as<double>(), e.dtab.as<double>(), static_cast<const double2 *>(x_cur),
         static_cast<double2 *>(x_io), (int)e.n_sites, st.n_panels, 1.0 / st.scale, (first ? 2.0 : 4.0) / st.scale, first ? 1.0 : 2.0,
         first ? 1 : 0, st.partials.as<double>(), st.tickets.as<unsigned>(), dots_step, st.cube_walk);

@@ -521,9 +521,6 @@ patch_blocks(int64_t n, const int32_t *__restrict__ klist, const PatchArgs a) {
     }
 }
 
-using EllKernel = void (*)(const int32_t *, const int32_t *, const double *, const double *, const double2 *, double2 *,
-                           int, int, double, double, int, int, double *, unsigned *, double *, const RowWalk);
-
 template <int PW, int NP, bool DICT, bool DIAG, bool SD> EllKernel pick_ch(int width) {
     switch (width) {
         case 3: return cheb_step_ell<PW, 3, NP, DICT, DIAG, SD>;
@@ -562,14 +559,12 @@ EllKernel pick_ell(int fmt, int pw, int np, int width, bool self_diag) {
     return np == 2 ? pick_two_panels(width) : pick_shape<false, false>(pw, width);
 }
 
-bool ell_self_diag(const EllDev &e) { return e.self_diag_usable && env_int("BDG_ELL_SD", 1) != 0; }
-
 // Plan the row traversal for `slots` resident CTAs per panel group (RowWalk, bdg_internal.h).
-RowWalk plan_walk(const bdg_system *sys, int n_sites, int64_t slots) {
+RowWalk plan_walk(const bdg_system *sys, int n_sites, int64_t slots, const PlanSwitches &sw) {
     RowWalk w;
     const int Lx = sys->cubic[0], Ly = sys->cubic[1], Lz = sys->cubic[2];
     const bool cubic = (int64_t)Lx * Ly * Lz == n_sites && n_sites > 0;
-    if (!cubic || Ly * Lz < 2 * kWarps || Lx < 8 || env_int("BDG_ELL_WALK", 1) == 0) {
+    if (!cubic || Ly * Lz < 2 * kWarps || Lx < 8 || !sw.ell_walk) {
         // consecutive rows, one per warp: the wavefront sweep of cheb.cu
         w.Lz = std::max(n_sites, 1);
         w.Pz = kWarps;
@@ -578,8 +573,7 @@ RowWalk plan_walk(const bdg_system *sys, int n_sites, int64_t slots) {
         return w;
     }
     w.Lx = Lx, w.Ly = Ly, w.Lz = Lz;
-    w.Pz = Lz == 1 ? 1 : (Ly == 1 ? kWarps : 2);
-    w.Pz = std::max(1, std::min(env_int("BDG_ELL_PZ", w.Pz), kWarps));
+    w.Pz = sw.ell_pz > 0 ? std::min(sw.ell_pz, kWarps) : Lz == 1 ? 1 : (Ly == 1 ? kWarps : 2);
     while (kWarps % w.Pz) --w.Pz;
     w.Py = kWarps / w.Pz;
     w.nPz = (int)ceil_div(Lz, w.Pz);
@@ -587,7 +581,7 @@ RowWalk plan_walk(const bdg_system *sys, int n_sites, int64_t slots) {
     // Segment length: long segments amortise the two cold columns at the start of an item, many
     // items balance the CTAs.  Score = (share of CTA slots doing useful work) x (1 - cold share).
     double best = -1.0;
-    const int forced = env_int("BDG_ELL_SEG", 0);
+    const int forced = sw.ell_seg;
     for (int n_seg = 1; n_seg <= std::max(1, Lx / 8); ++n_seg) {
         const int len = forced > 0 ? forced : (int)ceil_div(Lx, n_seg);
         const int64_t items = (int64_t)w.n_patches * ceil_div(Lx, len);
@@ -600,7 +594,7 @@ RowWalk plan_walk(const bdg_system *sys, int n_sites, int64_t slots) {
         }
         if (forced > 0) break;
     }
-    w.prefetch = std::max(0, env_int("BDG_ELL_PREFETCH", 1)) * Ly * Lz;
+    w.prefetch = std::max(0, sw.ell_prefetch) * Ly * Lz;
     return w;
 }
 
@@ -802,8 +796,8 @@ int ell_patch(bdg_system *sys, int64_t n, const int32_t *klist, bool *ok) {
     return BDG_OK;
 }
 
-// Panels per group and grid size for the current recursion (ChebState::panel_width / n_panels).
-int ell_configure(bdg_system *sys) {
+// The single-step kernel of the current recursion, its panels per group, grid and row traversal.
+int ell_configure(bdg_system *sys, const PlanSwitches &sw) {
     ChebState &st = sys->cheb;
     const EllDev &e = sys->ell;
     // One panel per pass, each panel group marching the lattice on its own CTAs: with the marching
@@ -811,36 +805,36 @@ int ell_configure(bdg_system *sys) {
     // dictionary workload measured (profiles/r01/quickperf_np_v2.log).  The plain kernel on 3-D
     // lattices (long rows: more block bytes per record byte) still gains from two panels per pass.
     const bool dict = st.kernel != BDG_KERNEL_ELL;
-    const bool pair = !dict && st.panel_width == 8 && st.n_panels >= 2 && e.width >= 6;  // (pick_two_panels)
-    st.panels_per_group = pair ? 2 : 1;
-    st.n_groups = (int)ceil_div(st.n_panels, st.panels_per_group);
+    const int panels_per_group = !dict && st.panel_width == 8 && st.n_panels >= 2 && e.width >= 6 ? 2 : 1;  // (pick_two_panels)
+    const int n_groups = (int)ceil_div(st.n_panels, panels_per_group);
+    const EllKernel k = pick_ell(st.kernel, st.panel_width, panels_per_group, e.width, e.self_diag_usable && sw.ell_sd);
     int per_sm = 1;
-    BDG_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(
-        &per_sm, pick_ell(st.kernel, st.panel_width, st.panels_per_group, e.width, ell_self_diag(e)), kThreads, 0));
+    BDG_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k, kThreads, 0));
     per_sm = std::max(per_sm, 1);
-    const int64_t slots = std::max<int64_t>(1, (int64_t)sys->sm_count * per_sm / st.n_groups);
-    st.walk = plan_walk(sys, (int)e.n_sites, slots);
-    st.grid_x = (int)std::min<int64_t>(slots, st.walk.n_items);
+    const int64_t slots = std::max<int64_t>(1, (int64_t)sys->sm_count * per_sm / n_groups);
+    st.walk = plan_walk(sys, (int)e.n_sites, slots, sw);
+    const int gx = (int)std::min<int64_t>(slots, st.walk.n_items);
+    st.ell_step = {k, dim3((unsigned)gx, (unsigned)n_groups), kThreads, 0};
+    st.partial_runs = std::max(st.partial_runs, gx);
     return BDG_OK;
 }
 
 int ell_launch_step(bdg_system *sys, bool first, const void *x_cur, void *x_io, double *dots_step) {
     ChebState &st = sys->cheb;
     const EllDev &e = sys->ell;
-    const bool dict = st.kernel == BDG_KERNEL_DICT || st.kernel == BDG_KERNEL_DICT_DIAG;
-    EllKernel k = pick_ell(st.kernel, st.panel_width, st.panels_per_group, e.width, ell_self_diag(e));
-    note_launch(st, reinterpret_cast<const void *>(k));
+    const bool dict = st.kernel != BDG_KERNEL_ELL;
+    const Launch<EllKernel> &l = st.ell_step;
+    note_launch(st, reinterpret_cast<const void *>(l.fn));
     // Stream the matrix through L2 (evict-first) only when nothing will read it again soon: one
     // group per pass and a matrix that cannot stay resident in the 126 MB L2 anyway.
     const size_t matrix_bytes = (size_t)e.n_sites * e.width * 260;
-    const int stream_matrix = st.n_groups == 1 && matrix_bytes > (size_t)64 << 20;
-    dim3 grid((unsigned)st.grid_x, (unsigned)st.n_groups);
-    k<<<grid, kThreads, 0, sys->stream>>>(e.idx.as<int32_t>(), dict ? e.code.as<int32_t>() : nullptr,
-                                          dict ? e.table.as<double>() : e.data.as<double>(), e.dtab.as<double>(),
-                                          static_cast<const double2 *>(x_cur), static_cast<double2 *>(x_io),
-                                          (int)e.n_sites, st.n_panels, (first ? 1.0 : 2.0) / st.scale, first ? 0.0 : 1.0,
-                                          first ? 1 : 0, stream_matrix, st.partials.as<double>(),
-                                          st.tickets.as<unsigned>(), dots_step, st.walk);
+    const int stream_matrix = l.grid.y == 1 && matrix_bytes > (size_t)64 << 20;
+    l.fn<<<l.grid, l.threads, l.smem, sys->stream>>>(e.idx.as<int32_t>(), dict ? e.code.as<int32_t>() : nullptr,
+                                                     dict ? e.table.as<double>() : e.data.as<double>(), e.dtab.as<double>(),
+                                                     static_cast<const double2 *>(x_cur), static_cast<double2 *>(x_io),
+                                                     (int)e.n_sites, st.n_panels, (first ? 1.0 : 2.0) / st.scale, first ? 0.0 : 1.0,
+                                                     first ? 1 : 0, stream_matrix, st.partials.as<double>(),
+                                                     st.tickets.as<unsigned>(), dots_step, st.walk);
     BDG_CUDA(cudaGetLastError());
     return BDG_OK;
 }

@@ -231,19 +231,19 @@ cheb_pair_step(const int32_t *__restrict__ dcode, const double *__restrict__ tab
     const bool code_lane = lane < S * kDirs, self_lane = cdir == 0;
     const int plane_codes = wk.M * kDirs, all_codes = wk.Lx * plane_codes;
 
-    const int item0 = LISTED ? wk.cta_begin[blockIdx.x] : (int)blockIdx.x, item1 = LISTED ? wk.cta_begin[blockIdx.x + 1] : wk.n_items;
+    const int item0 = LISTED ? wk.lists.cta_begin[blockIdx.x] : (int)blockIdx.x, item1 = LISTED ? wk.lists.cta_begin[blockIdx.x + 1] : wk.n_items;
     for (int item = item0; item < item1; item += LISTED ? 1 : (int)gridDim.x) {
         int4 piece;  // panel, patch, x0, len
         if (LISTED) {
-            piece = wk.pieces[item];  // (run, patch, x0, len)
+            piece = wk.lists.pieces[item];  // (run, patch, x0, len)
             if (piece.x != run) {
                 if (run >= 0) {
-                    flush_dots<NW, 8>(d0, d1, d2, d3, pair_smem, run, wk.panel_runs[panel], wk.panel_runs[panel + 1], panel, n_panels, partials,
+                    flush_dots<NW, 8>(d0, d1, d2, d3, pair_smem, run, wk.lists.panel_runs[panel], wk.lists.panel_runs[panel + 1], panel, n_panels, partials,
                                       tickets, dots_step);
                     d0 = d1 = d2 = d3 = 0.0;
                 }
                 run = piece.x;
-                panel = wk.run_panel[run];
+                panel = wk.lists.run_panel[run];
             }
             piece.x = panel;
         } else {
@@ -470,7 +470,7 @@ cheb_pair_step(const int32_t *__restrict__ dcode, const double *__restrict__ tab
     }
     if (LISTED) {
         if (panel >= 0)
-            flush_dots<NW, 8>(d0, d1, d2, d3, pair_smem, run, wk.panel_runs[panel], wk.panel_runs[panel + 1], panel, n_panels, partials, tickets,
+            flush_dots<NW, 8>(d0, d1, d2, d3, pair_smem, run, wk.lists.panel_runs[panel], wk.lists.panel_runs[panel + 1], panel, n_panels, partials, tickets,
                               dots_step);
     } else {
         const int p = (int)blockIdx.y, r0 = p * (int)gridDim.x;
@@ -511,9 +511,6 @@ pair_codes(int n_sites, int width, int Lx, int M, const int32_t *__restrict__ ci
     if ((y == 0 && out[2] >= 0) || (y == M - 1 && out[3] >= 0)) *wraps = 1;
 }
 
-using PairKernel = void (*)(const int32_t *, const double *, const double *, const double2 *, const double2 *, double2 *,
-                            double2 *, int, int, double, double, double, int, double *, unsigned *, double *, const PairWalk);
-
 template <bool LISTED> PairKernel pick_pair(bool diag, bool self, bool t2, bool sd) {
     if (sd && !diag) {  // general hopping blocks, real-diagonal on-site blocks
         if (self) return t2 ? cheb_pair_step<false, true, 1, true, LISTED> : cheb_pair_step<false, true, 0, true, LISTED>;
@@ -532,26 +529,7 @@ constexpr int kPairThreads = kPairWarps * 32;
 constexpr size_t kPairSmem = ((size_t)kRingN * (kPairWarps * kPairSites + 2) + (size_t)kRing * kPairWarps * kPairSites + 2) * kRecBytes +
                              8 * (kRingN + 1);
 
-// On-site fragments per row straight from the table (SELF) when the dictionary is large: then the on-site blocks
-// differ from site to site (disorder, a self-consistent gap, a phase winding) and holding them in registers from
-// plane to plane would reload them on every row through the slow path.
-// Real-diagonal on-site blocks next to general hopping blocks: two multiplications instead of two MMAs (BDG_ELL_SD=0: off)
-bool pair_sd(const EllDev &e) { return e.self_diag_usable && !e.diag_usable && env_int("BDG_ELL_SD", 1) != 0; }
-
-bool pair_self(const EllDev &e) {
-    const int forced = env_int("BDG_PAIR_SELF", -1);
-    return forced >= 0 ? forced != 0 : e.n_unique > 64;
-}
-
-// The kernel for the matrix in hand; `listed`: the one that works through the lists of a balanced plan.
-PairKernel pair_kernel(const bdg_system *sys, bool t2, bool listed) {
-    const bool diag = sys->cheb.kernel == BDG_KERNEL_DICT_DIAG, self = pair_self(sys->ell), sd = pair_sd(sys->ell);
-    return listed ? pick_pair<true>(diag, self, t2, sd) : pick_pair<false>(diag, self, t2, sd);
-}
-
 }  // namespace
-
-bool pair_streams_onsite(const bdg_system *sys) { return pair_self(sys->ell); }
 
 // Does the current fixed-width copy qualify?  (dictionary built, one-dimensional x-planes of >= 3 sites, >= 3
 // planes, nearest-neighbour stencil -- open or periodic --, rows of <= 5 blocks)
@@ -589,31 +567,38 @@ int pair_probe(bdg_system *sys) {
     return BDG_OK;
 }
 
-// Patch size, segment length and grid for the current recursion.
-int pair_configure(bdg_system *sys) {
+// The two-step kernel of the current recursion (Pair or EvenPlane) with its patch size, segment length and grid.
+int pair_configure(bdg_system *sys, const PlanSwitches &sw) {
     ChebState &st = sys->cheb;
     const EllDev &e = sys->ell;
-    const PairKernel kernel = pair_kernel(sys, st.t2, false), listed = pair_kernel(sys, st.t2, true);
-    BDG_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPairSmem));
-    BDG_CUDA(cudaFuncSetAttribute(listed, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPairSmem));
+    const bool diag = st.kernel == BDG_KERNEL_DICT_DIAG, even = st.stepping == Stepping::EvenPlane;
+    // On-site fragments per row straight from the table (SELF) when the dictionary is large: then the on-site blocks
+    // differ from site to site (disorder, a self-consistent gap, a phase winding) and holding them in registers from
+    // plane to plane would reload them on every row through the slow path.
+    st.onsite_per_row = sw.pair_self >= 0 ? sw.pair_self != 0 : e.n_unique > 64;
+    // Real-diagonal on-site blocks next to general hopping blocks: two multiplications instead of two MMAs
+    st.onsite_diag = e.self_diag_usable && !e.diag_usable && sw.ell_sd;
+    const PairKernel classic = pick_pair<false>(diag, st.onsite_per_row, even, st.onsite_diag);
+    // (the occupancy query counts kPairSmem against the kernel's limit, so the limit is raised first)
+    BDG_CUDA(cudaFuncSetAttribute(classic, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPairSmem));
     int per_sm = 1;
-    BDG_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kPairThreads, kPairSmem));
+    BDG_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, classic, kPairThreads, kPairSmem));
     per_sm = std::max(per_sm, 1);
-    const int64_t slots = std::max<int64_t>(1, (int64_t)sys->sm_count * per_sm / st.n_panels);
+    const int64_t all_slots = (int64_t)sys->sm_count * per_sm;
+    const int64_t slots = std::max<int64_t>(1, all_slots / st.n_panels);
     PairWalk &w = st.pair_walk;
     w.Lx = sys->cubic[0];
     w.M = e.pair_M;
     const int p_max = kPairWarps * kPairSites - 2;
-    w.open = e.pair_open && env_int("BDG_PAIR_OPEN", 1) != 0 ? 1 : 0;
+    w.open = e.pair_open && sw.pair_open ? 1 : 0;
     const int to_cover = std::max(1, w.M - 2 * w.open);  // n patches own n P (+ 2: the rim sites of a plane with open ends) sites
     const int n_patches_min = (int)ceil_div(to_cover, p_max);
-    w.P = (int)ceil_div(to_cover, n_patches_min);  // balanced patches
-    w.P = std::max(1, std::min(env_int("BDG_PAIR_P", w.P), p_max));
+    w.P = sw.pair_p > 0 ? std::min(sw.pair_p, p_max) : (int)ceil_div(to_cover, n_patches_min);  // balanced patches
     w.n_patches = (int)ceil_div(to_cover, w.P);
     // Segment length: every item recomputes one plane of T_{n+1} on either side of its segment and
     // starts with a cold pipeline (about two more plane times); many items balance the CTAs.
     double best = -1.0;
-    const int forced = env_int("BDG_PAIR_SEG", 0);
+    const int forced = sw.pair_seg;
     for (int n_seg = 1; n_seg <= std::max(1, w.Lx / 4); ++n_seg) {
         const int len = forced > 0 ? std::min(forced, w.Lx) : (int)ceil_div(w.Lx, n_seg);
         const int64_t segs = ceil_div(w.Lx, len);
@@ -628,28 +613,14 @@ int pair_configure(bdg_system *sys) {
         }
         if (forced > 0) break;
     }
-    // ---- classic or balanced plan ------------------------------------------------------------------------------------
-    // Classic: every panel has its own `gx` CTAs (grid = (gx, panels)), CTA (bx, panel) takes the items bx, bx + gx, ...
-    // (segment-major: the grid sweeps the lattice as one wavefront, so the halo sites of a patch are in L2 when its neighbour
-    // reads them); the kernel computes its items from the item index.
-    // Balanced: the (panel, patch, x) space cut into one contiguous chunk per CTA slot, handed to the kernel as lists -- no
-    // wave quantisation, no per-panel slot quantisation, fewer segment halos.  Taken when its longest CTA is clearly shorter
-    // (small lattices with many panels: C2 / C3: +3 .. +17 %); on large lattices the classic plan is near-perfect already.
     constexpr int kPieceCost = 6;  // iterations a piece costs beyond its planes: two halo planes either side, cold pipeline
-    const int gx = (int)std::min<int64_t>(slots, w.n_items);
-    const int64_t all_slots = (int64_t)sys->sm_count * per_sm;
-    const double classic_cost = (double)ceil_div((int64_t)gx * st.n_panels, all_slots) * (double)ceil_div(w.n_items, gx) * (w.seg_len + kPieceCost);
-    w.pieces = nullptr, w.cta_begin = w.run_panel = w.panel_runs = nullptr;
-    w.n_ctas = gx, w.n_runs = gx * st.n_panels;
-    st.pair_grid_x = gx;
-    const WorkPlan plan = best_balanced_plan(st.n_panels, w.n_patches, w.Lx, all_slots, kPieceCost, 1.08);
-    const int force = env_int("BDG_PAIR_BALANCE", -1);
-    if (!(force >= 0 ? force != 0 : plan.longest < 0.93 * classic_cost)) return BDG_OK;
-    WorkLists lists;
-    BDG_TRY(upload_work_lists(sys, st.work_items, plan, st.n_panels, lists));
-    w.pieces = lists.pieces, w.cta_begin = lists.cta_begin, w.run_panel = lists.run_panel, w.panel_runs = lists.panel_runs;
-    w.n_ctas = lists.n_ctas, w.n_runs = lists.n_runs;
-    st.pair_grid_x = (int)ceil_div(lists.n_runs, st.n_panels);  // (sizes the partial-sum buffer: n_panels x pair_grid_x runs)
+    BDG_TRY(choose_work_plan(sys, st.work_items, st.n_panels, w.n_patches, w.Lx, w.seg_len, w.n_items, all_slots, kPieceCost, 1.08,
+                             sw.pair_balance, w.lists));
+    const bool listed = w.lists.pieces != nullptr;
+    const PairKernel k = listed ? pick_pair<true>(diag, st.onsite_per_row, even, st.onsite_diag) : classic;
+    if (listed) BDG_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPairSmem));
+    st.two_step = {k, dim3((unsigned)w.lists.n_ctas, listed ? 1u : (unsigned)st.n_panels), kPairThreads, kPairSmem};
+    st.partial_runs = std::max(st.partial_runs, (int)ceil_div(w.lists.n_runs, st.n_panels));
     return BDG_OK;
 }
 
@@ -657,11 +628,9 @@ int pair_configure(bdg_system *sys) {
 int pair_launch(bdg_system *sys, const void *x_prev, const void *x_cur, void *x_next1, void *x_next2, double *dots_step) {
     ChebState &st = sys->cheb;
     const EllDev &e = sys->ell;
-    const bool listed = st.pair_walk.pieces != nullptr;
-    dim3 grid((unsigned)st.pair_walk.n_ctas, listed ? 1u : (unsigned)st.n_panels);
-    const PairKernel k = pair_kernel(sys, false, listed);
-    note_launch(st, reinterpret_cast<const void *>(k));
-    k<<<grid, kPairThreads, kPairSmem, sys->stream>>>(
+    const Launch<PairKernel> &l = st.two_step;
+    note_launch(st, reinterpret_cast<const void *>(l.fn));
+    l.fn<<<l.grid, l.threads, l.smem, sys->stream>>>(
         e.dcode.as<int32_t>(), e.table.as<double>(), e.dtab.as<double>(), static_cast<const double2 *>(x_prev),
         static_cast<const double2 *>(x_cur), static_cast<double2 *>(x_next1), static_cast<double2 *>(x_next2),
         (int)e.n_sites, st.n_panels, 2.0 / st.scale, 0.0, 0.0, 0, st.partials.as<double>(), st.tickets.as<unsigned>(), dots_step,
@@ -673,13 +642,11 @@ int pair_launch(bdg_system *sys, const void *x_prev, const void *x_cur, void *x_
 // T2 mode: E_{j+1} = 2 T_2(H~) E_j - E_{j-1} written over E_{j-1} (x_io); first: E_1 = T_2(H~) E_0.
 int t2_launch(bdg_system *sys, bool first, const void *x_cur, void *x_io, double *dots_step) {
     ChebState &st = sys->cheb;
-    if (st.cube) return cube_launch(sys, first, x_cur, x_io, dots_step);
+    if (st.stepping == Stepping::EvenCube) return cube_launch(sys, first, x_cur, x_io, dots_step);
     const EllDev &e = sys->ell;
-    const bool listed = st.pair_walk.pieces != nullptr;
-    dim3 grid((unsigned)st.pair_walk.n_ctas, listed ? 1u : (unsigned)st.n_panels);
-    const PairKernel k = pair_kernel(sys, true, listed);
-    note_launch(st, reinterpret_cast<const void *>(k));
-    k<<<grid, kPairThreads, kPairSmem, sys->stream>>>(
+    const Launch<PairKernel> &l = st.two_step;
+    note_launch(st, reinterpret_cast<const void *>(l.fn));
+    l.fn<<<l.grid, l.threads, l.smem, sys->stream>>>(
         e.dcode.as<int32_t>(), e.table.as<double>(), e.dtab.as<double>(), static_cast<const double2 *>(x_io),
         static_cast<const double2 *>(x_cur), nullptr, static_cast<double2 *>(x_io), (int)e.n_sites, st.n_panels,
         1.0 / st.scale, (first ? 2.0 : 4.0) / st.scale, first ? 1.0 : 2.0, first ? 1 : 0, st.partials.as<double>(), st.tickets.as<unsigned>(),

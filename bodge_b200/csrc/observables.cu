@@ -173,7 +173,7 @@ extern "C" int bdg_cheb_local_begin(bdg_t *sys, int32_t n_coef, const double *co
     BDG_ENTER(sys);
     ChebState &st = sys->cheb;
     BDG_REQUIRE(st.active, "bdg_cheb_begin has not been called");
-    BDG_REQUIRE(!st.t2,
+    BDG_REQUIRE(!st.even(),
                 "the even-vector recursion (kernel T2) keeps only every second Chebyshev vector, so it cannot accumulate "
                 "local matrix elements of a series: begin the recursion with the pair or a single-step kernel");
     BDG_REQUIRE(st.steps_done == 0, "register the local accumulator right after bdg_cheb_begin (%d steps already taken)",

@@ -67,13 +67,7 @@ inline WorkPlan best_balanced_plan(int n_panels, int n_columns, int Lx, int64_t 
     return flat.longest < grouped.longest ? flat : grouped;
 }
 
-struct WorkLists {  // device pointers into one buffer
-    const int4 *pieces = nullptr;  // (run, patch column, x0, len)
-    const int *cta_begin = nullptr, *run_panel = nullptr, *panel_runs = nullptr;
-    int n_ctas = 0, n_runs = 0;
-};
-
-// Upload: pieces (16-byte aligned: first), cta_begin[n_ctas + 1], run_panel[n_runs], panel_runs[n_panels + 1].  A run = a
+// Upload (WorkLists, bdg_internal.h: device pointers into `buf`): pieces (16-byte aligned: first), cta_begin[n_ctas + 1], run_panel[n_runs], panel_runs[n_panels + 1].  A run = a
 // maximal sequence of pieces of one panel inside a CTA: its dot products go to partials[run].  Runs are numbered panel by
 // panel (and in CTA order inside a panel), so the runs of panel p are panel_runs[p] .. panel_runs[p + 1] and the last one to
 // arrive adds them up in that fixed order.
@@ -123,6 +117,25 @@ inline int upload_work_lists(bdg_system *sys, DevBuf &buf, const WorkPlan &plan,
     out.n_ctas = (int)plan.per_cta.size();
     out.n_runs = (int)runs.size();
     return BDG_OK;
+}
+
+// Classic or balanced plan for a launch of `n_items` items (patch, segment of `seg_len` planes) per panel on `slots` CTA slots.
+// Classic: every panel has its own gx CTAs (grid = (gx, panels)), CTA (bx, panel) takes the items bx, bx + gx, ... (segment-
+// major: the grid sweeps the lattice as one wavefront, so the halo sites of a patch are in L2 when its neighbour reads them);
+// the kernel computes its items from the item index.  Balanced (best_balanced_plan): the (panel, patch, x) space cut into one
+// contiguous chunk per CTA slot, handed to the kernel as lists -- no wave quantisation, no per-panel slot quantisation, fewer
+// segment halos.  Taken when its longest CTA is clearly shorter (small lattices with many panels: C2 / C3: +3 .. +17 %); on
+// large lattices the classic plan is near-perfect already.  `force`: 0 = classic, 1 = balanced, < 0 = decide.  `out`: the
+// uploaded lists, or the classic plan's n_ctas = gx, n_runs = gx x panels and no lists.
+inline int choose_work_plan(bdg_system *sys, DevBuf &buf, int n_panels, int n_patches, int Lx, int seg_len, int n_items,
+                            int64_t slots, int piece_cost, double flat_penalty, int force, WorkLists &out) {
+    const int gx = (int)std::min<int64_t>(std::max<int64_t>(1, slots / n_panels), n_items);
+    const double classic_cost = (double)ceil_div((int64_t)gx * n_panels, slots) * (double)ceil_div(n_items, gx) * (seg_len + piece_cost);
+    out = WorkLists();
+    out.n_ctas = gx, out.n_runs = gx * n_panels;
+    const WorkPlan plan = best_balanced_plan(n_panels, n_patches, Lx, slots, piece_cost, flat_penalty);
+    if (!(force >= 0 ? force != 0 : plan.longest < 0.93 * classic_cost)) return BDG_OK;
+    return upload_work_lists(sys, buf, plan, n_panels, out);
 }
 
 }  // namespace

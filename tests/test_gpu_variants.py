@@ -162,6 +162,24 @@ def test_cube_plans_agree_with_the_diagonal_kernel(systems, monkeypatch, case_id
     assert np.max(np.abs(base[2] - want[2])) <= 1e-13 * max(np.max(np.abs(want[2])), 1.0)
 
 
+def test_plan_switches_hold_for_the_recursion(systems, monkeypatch):
+    """cheb_begin reads the plan switches once: BDG_ELL_SD=0 set after it leaves the running recursion on the kernel
+    with the real-diagonal on-site product, and the vectors are those of an undisturbed run."""
+    case = vc.CASES["dict-square-gen-c13"]
+    system, _, _, scale = systems(case.geometry, case.model)
+    want = run(system, scale, monkeypatch, case)
+    set_env(monkeypatch, case.env)
+    sysn = system._sys
+    sysn.cheb_begin(n_random=case.n_cols, seed=SEED, scale=scale, kernel=case.kernel)
+    monkeypatch.setenv("BDG_ELL_SD", "0")
+    sysn.cheb_steps(case.steps)
+    launched = vc.short_names(sysn.cheb_launched())
+    cur, prev = sysn.cheb_vectors(case.n_cols, 0), sysn.cheb_vectors(case.n_cols, 1)
+    sysn.cheb_end()
+    assert launched == list(case.kernels) == want[0]
+    assert np.array_equal(cur, want[2]) and np.array_equal(prev, want[3])
+
+
 # ---- local accumulator ----------------------------------------------------------------------------------------------
 LOCAL_RUNS = [  # (kernel, columns, environment, kernel that must run)
     ("dict_diag", 1, (), "cheb_step_ell<1, 5, 1, true, true, false>"),

@@ -1,6 +1,7 @@
 """Host logic of the balanced plans (``bodge_b200/csrc/work_lists.h``): the planner that cuts the (panel, patch column, plane)
 space of a two-step launch into one chunk per CTA slot is plain C++ -- ``tests/cpp/work_lists_check.cpp`` compiles it with
-the host compiler and checks 13 k plans for exact cover, bounds, slot count and the cost it reports.  No GPU."""
+the host compiler and checks 13 k plans for exact cover, bounds, slot count and the cost it reports, and the choice between
+the classic and the balanced plan (``choose_work_plan``) with the lists it uploads.  No GPU."""
 
 import os
 import shutil
