@@ -16,7 +16,7 @@ ROOT = os.path.dirname(PKG)
 CSRC = os.path.join(PKG, "csrc")
 LIB = os.path.join(PKG, "libbdg.so")
 PACK = os.path.join(PKG, "_bdgpack.so")  # host-side dict packer (CPython API, no CUDA): csrc/pack_dict.c
-SOURCES = ["assemble.cu", "scan.cu", "cheb.cu", "cheb_ell.cu", "cheb_pair.cu", "cheb_cube.cu", "observables.cu", "multi.cu"]
+SOURCES = ["assemble.cu", "scan.cu", "cheb.cu", "cheb_ell.cu", "cheb_pair.cu", "cheb_cube.cu", "formats.cu", "observables.cu", "multi.cu"]
 
 
 def nvcc_path() -> str:

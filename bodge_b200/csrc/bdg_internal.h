@@ -203,9 +203,18 @@ static inline void note_launch(ChebState &st, const void *kernel) {
     st.launched.push_back(kernel);
 }
 
-// Kernel-native copy of the packed matrix for the ELL step kernel (cheb_ell.cu): every block row
-// padded to `width` slots, slot 0 = the diagonal block (zero block if absent), then the other
-// blocks in ascending column order; padding slots are zero blocks pointing at the row itself.
+// Direction codes (EllDev::dcode, dcode3): per site, the dictionary code of the row's block in each direction of a
+// nearest-neighbour stencil, so that a kernel finds a row's blocks without any index.
+constexpr int kPlaneCodes = 5;  // dcode (cheb_pair.cu): self, x-1, y-1, y+1, x+1 on the Lx x M torus
+constexpr int kCubeCodes = 8;   // dcode3 (cheb_cube.cu): self, x-1, y-1, z-1, z+1, y+1, x+1, padding on the open lattice
+constexpr int kNoBlock = -1;    // no block in that direction: the kernel multiplies by a zero fragment
+constexpr int kNoSite = -2;     // dcode3 only: no lattice site in that direction of y / z: the kernel keeps what it holds
+// The cube kernel holds its fragments in registers and takes a dictionary of at most this many distinct blocks.
+constexpr int64_t kCubeMaxUnique = 64;
+
+// Kernel-native copies of the packed matrix for the step kernels, built and patched by formats.cu.
+// Fixed-width rows (cheb_ell.cu): every block row padded to `width` slots, slot 0 = the diagonal block (zero block if
+// absent), then the other blocks in ascending column order; padding slots are zero blocks pointing at the row itself.
 //   idx  int32  [n_sites][width]
 //   data double [n_sites][width][4 (a)][2 (re, im)][4 (b)]   -- MMA B-fragment order, 256 B/block
 struct EllDev {
@@ -227,14 +236,14 @@ struct EllDev {
     bool pair_usable = false;
     bool pair_open = false;  // no block wraps around in-plane
     int pair_M = 0;
-    DevBuf dcode;  // int32 [n_sites][5]: dictionary code per stencil direction (self, x-1, y-1, y+1, x+1), -1 = none
-    // ... and its three-dimensional sibling (cheb_cube.cu): open nearest-neighbour stencil on a lattice with Ly, Lz >= 2.
+    DevBuf dcode;  // int32 [n_sites][kPlaneCodes]; kNoBlock = none
+    // ... and its three-dimensional sibling (cheb_cube.cu): open nearest-neighbour stencil on a lattice with Ly, Lz >= 2,
+    // real-diagonal hopping blocks, at most kCubeMaxUnique distinct blocks.
     bool cube_usable = false;
-    DevBuf dcode3;  // int32 [n_sites][8]: (self, x-1, y-1, z-1, z+1, y+1, x+1, pad); -1 = no block, -2 = no site in y / z
+    DevBuf dcode3;  // int32 [n_sites][kCubeCodes]; kNoBlock = no block, kNoSite = no site in y / z
     DevBuf tmp_keys, tmp_rep, tmp_where, tmp_dense;  // hash-table scratch of the dictionary build (kept for rebuilds)
     // ... and what stays alive for incremental updates (ell_patch): the hash table itself (tmp_keys, `hash_cap` slots),
-    // posid[hash position] = dictionary code (-1: unused), the table's capacity in entries, device counters
-    // {n_unique, pattern changed, table full, hash collision, off-site block not real-diagonal}.
+    // posid[hash position] = dictionary code (-1: unused), the table's capacity in entries, the device PatchStatus.
     DevBuf posid, counters;
     int64_t hash_cap = 0, table_cap = 0;
 };
@@ -287,24 +296,24 @@ int t2_finish_dots(bdg_system *sys);    // T2 mode: dot rows -> single-step form
 // Local accumulator: add the terms of T_n (vector x_a) and T_{n+1} (x_b, may be null) that fall inside the series.
 int local_accumulate(bdg_system *sys, int n, const void *x_a, const void *x_b);
 
-// cheb_ell.cu
+// formats.cu
 int ell_build(bdg_system *sys);                    // (re)build sys->ell from sys->packed when stale
-int ell_configure(bdg_system *sys, const PlanSwitches &sw);  // ChebState::ell_step and its row traversal
-int ell_launch_step(bdg_system *sys, bool first, const void *x_cur, void *x_io, double *dots_step);
 // After a scatter: bring `packed` and the kernel-native copies (fixed-width rows, dictionary, direction codes) up to date
 // for the `n` skeleton blocks listed in `klist` (device; < 0 = skip) instead of rebuilding them.  *ok = false: the zero
 // pattern changed, the table is full, ...: the caller invalidates the copies and the next recursion rebuilds them.
 int ell_patch(bdg_system *sys, int64_t n, const int32_t *klist, bool *ok);
 void ell_release(bdg_system *sys);
 
+// cheb_ell.cu
+int ell_configure(bdg_system *sys, const PlanSwitches &sw);  // ChebState::ell_step and its row traversal
+int ell_launch_step(bdg_system *sys, bool first, const void *x_cur, void *x_io, double *dots_step);
+
 // cheb_pair.cu
-int pair_probe(bdg_system *sys);      // sets sys->ell.pair_usable / pair_M (called by ell_build)
 int pair_configure(bdg_system *sys, const PlanSwitches &sw);  // ChebState::two_step and its patch / segment plan
 int pair_launch(bdg_system *sys, const void *x_prev, const void *x_cur, void *x_next1, void *x_next2, double *dots_step);
 int t2_launch(bdg_system *sys, bool first, const void *x_cur, void *x_io, double *dots_step);
 
 // cheb_cube.cu
-int cube_probe(bdg_system *sys);      // sets sys->ell.cube_usable / dcode3 (called by ell_build)
 int cube_configure(bdg_system *sys, const PlanSwitches &sw);  // ChebState::cube_step: patch shape, segment plan
 int cube_launch(bdg_system *sys, bool first, const void *x_cur, void *x_io, double *dots_step);
 

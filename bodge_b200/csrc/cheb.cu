@@ -522,8 +522,8 @@ extern "C" int bdg_cheb_begin(bdg_t *sys, int kind, int32_t n_cols, const int64_
         const bool small = sys->ell.n_sites <= (1 << 16);
         const bool pair_ok = sys->ell.pair_usable && (n_cols >= 5 || small);
         // Three-dimensional lattices: the even-vector recursion on 4-column panels (cheb_cube.cu): open stencil,
-        // real-diagonal hopping blocks, few distinct blocks (its fragments are held in registers).
-        const bool cube_ok = sys->ell.cube_usable && sys->ell.n_unique <= 64 && (n_cols >= 3 || small);
+        // real-diagonal hopping blocks, few distinct blocks (its fragments are held in registers): EllDev::cube_usable.
+        const bool cube_ok = sys->ell.cube_usable && (n_cols >= 3 || small);
         BDG_REQUIRE(kernel != BDG_KERNEL_PAIR || pair_ok,
                     "the two-steps-per-pass kernel needs >= 5 columns (any number on lattices of <= 65536 sites) and a block "
                     "dictionary on a lattice with one-dimensional x-planes and a nearest-neighbour stencil");
@@ -772,9 +772,9 @@ extern "C" int bdg_cheb_format(bdg_t *sys, int32_t *kernel, int64_t *matrix_byte
     if (n_distinct_blocks) *n_distinct_blocks = e.valid ? e.n_unique : 0;
     if (matrix_bytes_per_step) {
         if (st.stepping == Stepping::EvenCube)  // eight 4-byte codes per site, read once per panel and launch (= two steps)
-            *matrix_bytes_per_step = e.n_sites * 32 * st.n_panels / 2 + e.n_unique * 256;
+            *matrix_bytes_per_step = e.n_sites * kCubeCodes * 4 * st.n_panels / 2 + e.n_unique * 256;
         else if (st.stepping != Stepping::Single)  // one pass over the codes (and, site-dependent on-site blocks: over those) serves two steps
-            *matrix_bytes_per_step = e.n_sites * 5 * 4 / 2 + (st.onsite_per_row ? std::min(e.n_unique, e.n_sites) * (st.onsite_diag ? 32 : 256) / 2
+            *matrix_bytes_per_step = e.n_sites * kPlaneCodes * 4 / 2 + (st.onsite_per_row ? std::min(e.n_unique, e.n_sites) * (st.onsite_diag ? 32 : 256) / 2
                                                                                   : e.n_unique * 256);
         else if (st.kernel == BDG_KERNEL_DICT || st.kernel == BDG_KERNEL_DICT_DIAG)
             *matrix_bytes_per_step = e.n_sites * e.width * 8 + e.n_unique * 256;

@@ -18,12 +18,12 @@
 // bulk of any lattice model); when they differ each gets its own pair and every lane keeps its half.
 //
 // Matrix: block dictionary with real-diagonal hopping blocks (cheb_ell.cu: DICT + DIAG; the on-site block is any 4x4
-// block), open nearest-neighbour stencil, at most 64 distinct blocks (fragments are held in registers and reloaded when a
-// code changes).  dcode[site][8] holds the dictionary codes towards (self, x-1, y-1, z-1, z+1, y+1, x+1) = ascending
-// block column, so that the sums are those of the single-step kernel in the same order.  -1 = no block (zero
-// coefficient); -2 = "no lattice site there in y / z": the operand is a shared-memory record that is never written
-// (rings are cleared per item, copies and stores skip what is outside the lattice), so the held coefficient is kept
-// and a patch on the lattice boundary runs without reloading fragments.
+// block), open nearest-neighbour stencil, at most kCubeMaxUnique = 64 distinct blocks (fragments are held in registers and
+// reloaded when a code changes).  dcode[site][kCubeCodes] holds the dictionary codes towards (self, x-1, y-1, z-1, z+1,
+// y+1, x+1) = ascending block column, so that the sums are those of the single-step kernel in the same order.  kNoBlock =
+// no block (zero coefficient); kNoSite = "no lattice site there in y / z": the operand is a shared-memory record that
+// is never written (rings are cleared per item, copies and stores skip what is outside the lattice), so the held
+// coefficient is kept and a patch on the lattice boundary runs without reloading fragments.
 //
 // An item = (patch, segment [x0, x0 + len) of x).  Iteration i = 0 .. len + 1, planes t <-> x = x0 - 2 + t of E_j in a ring
 // of NE planes of (PY + 4) x (PZ + 4) records, staged by bulk async copies (one per y-row, issued by the lanes of warp 0,
@@ -49,7 +49,6 @@ namespace {
 
 constexpr int kRec4 = 256;     // one site record at PW = 4: 4 columns x 4 components x complex128
 constexpr int kRingU = 3;      // planes of the u ring
-constexpr int kCodeStride = 8; // int32 per site in dcode3 (seven directions + padding)
 
 __device__ __forceinline__ void mbar_arrive_plain(uint32_t bar) {
     asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];\n" ::"r"(bar) : "memory");
@@ -76,9 +75,9 @@ __device__ __forceinline__ double settle(double v, int n_panels /* > 0: the XOR 
 __device__ __forceinline__ void hold_cube(int jv, Held &H, const double *__restrict__ table, const double *__restrict__ dtab,
                                           int lane, int n_panels) {
     const bool code_lane = lane < 16 && (lane & 7) < 7;
-    const unsigned changed = __ballot_sync(kFull, code_lane && jv != H.jheld && jv != -2);
+    const unsigned changed = __ballot_sync(kFull, code_lane && jv != H.jheld && jv != kNoSite);
     if (changed) {
-        if (code_lane && jv != -2) H.jheld = jv;
+        if (code_lane && jv != kNoSite) H.jheld = jv;
         const bool upper = lane >= 16;
         if (changed & 0x0101u) {
             const int c0 = __shfl_sync(kFull, H.jheld, 0), c1 = __shfl_sync(kFull, H.jheld, 8);
@@ -265,7 +264,7 @@ cheb_cube_step(const int32_t *__restrict__ dcode, const double *__restrict__ tab
             existA[r] = row_ok && zf + half >= 0 && zf + half < wk.Lz;
             ownA[r] = existA[r] && aly[r] >= 1 && aly[r] <= PY && alz[r] + half >= 1 && alz[r] + half <= PZ;
             const int zs = zf + cs;
-            codeA[r] = code_lane && row_ok && zs >= 0 && zs < wk.Lz ? (y * wk.Lz + zs) * kCodeStride + cu : -1;
+            codeA[r] = code_lane && row_ok && zs >= 0 && zs < wk.Lz ? (y * wk.Lz + zs) * kCubeCodes + cu : -1;
         }
 #pragma unroll
         for (int r = 0; r < RB; ++r) {
@@ -273,21 +272,21 @@ cheb_cube_step(const int32_t *__restrict__ dcode, const double *__restrict__ tab
             const bool row_ok = warp + NW * r < NB && y < wk.Ly;
             existB[r] = row_ok && zf + half < wk.Lz;
             const int zs = zf + cs;
-            codeB[r] = code_lane && row_ok && zs < wk.Lz ? (y * wk.Lz + zs) * kCodeStride + cu : -1;
+            codeB[r] = code_lane && row_ok && zs < wk.Lz ? (y * wk.Lz + zs) * kCubeCodes + cu : -1;
             gB[r] = ((ptrdiff_t)y * wk.Lz + zf) * 16 + lane;
         }
         // codes of the plane of [A] in this / the next iteration, of the plane of [B] likewise (loaded one iteration ahead)
         int jA[RA], jAn[RA], jB[RB], jBn[RB];
         {
             const int xa = x0 - 1;
-            const size_t po = (size_t)max(xa, 0) * plane_sites * kCodeStride;
+            const size_t po = (size_t)max(xa, 0) * plane_sites * kCubeCodes;
 #pragma unroll
             for (int r = 0; r < RA; ++r) {
-                jA[r] = jAn[r] = -2;
+                jA[r] = jAn[r] = kNoSite;
                 if (xa >= 0 && codeA[r] >= 0) jA[r] = __ldg(dcode + po + codeA[r]);
             }
 #pragma unroll
-            for (int r = 0; r < RB; ++r) jB[r] = jBn[r] = -2;
+            for (int r = 0; r < RB; ++r) jB[r] = jBn[r] = kNoSite;
         }
         double2 pv[RB], pvn[RB];  // E_{j-1} of the plane of [B] in this / the next iteration
 #pragma unroll
@@ -303,16 +302,16 @@ cheb_cube_step(const int32_t *__restrict__ dcode, const double *__restrict__ tab
             {
                 const int xn = xa + 1;
                 const bool n_valid = i <= len && xn >= 0 && xn < wk.Lx;
-                const size_t pn = (size_t)(n_valid ? xn : 0) * plane_sites * kCodeStride;
-                const size_t pa = (size_t)(a_valid ? xa : 0) * plane_sites * kCodeStride;
+                const size_t pn = (size_t)(n_valid ? xn : 0) * plane_sites * kCubeCodes;
+                const size_t pa = (size_t)(a_valid ? xa : 0) * plane_sites * kCubeCodes;
 #pragma unroll
                 for (int r = 0; r < RA; ++r) {
-                    jAn[r] = -2;
+                    jAn[r] = kNoSite;
                     if (n_valid && codeA[r] >= 0) jAn[r] = __ldg(dcode + pn + codeA[r]);
                 }
 #pragma unroll
                 for (int r = 0; r < RB; ++r) {
-                    jBn[r] = -2;
+                    jBn[r] = kNoSite;
                     if (store && codeB[r] >= 0) jBn[r] = __ldg(dcode + pa + codeB[r]);
                     pv[r] = pvn[r];
                     if (store && existB[r] && !first) pvn[r] = ld_prev_rw(tio + (ptrdiff_t)xa * plane_sites * 16 + gB[r]);
@@ -402,39 +401,6 @@ cheb_cube_step(const int32_t *__restrict__ dcode, const double *__restrict__ tab
     }
 }
 
-// *bad = 1 unless every block column of the fixed-width copy is the row itself or one of its six nearest neighbours on
-// the open lattice (padding slots point at the row itself).
-__global__ void __launch_bounds__(256)
-cube_check(int64_t n_slots, int width, int Ly, int Lz, const int32_t *__restrict__ cidx, int *__restrict__ bad) {
-    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= n_slots) return;
-    const int row = (int)(t / width);
-    if (cube_direction(row, cidx[t], Ly, Lz) < 0) *bad = 1;
-}
-
-// dcode[row][dir]: dictionary code of the row's block towards dir (slot 0 of the fixed-width copy is the diagonal block);
-// -1 = no block, -2 = no lattice site in that in-plane direction.
-__global__ void __launch_bounds__(256)
-cube_codes(int n_sites, int width, int Ly, int Lz, const int32_t *__restrict__ cidx, const int32_t *__restrict__ ccode,
-           int32_t *__restrict__ dcode) {
-    const int row = blockIdx.x * blockDim.x + threadIdx.x;
-    if (row >= n_sites) return;
-    const int z = row % Lz, y = (row / Lz) % Ly;
-    int out[kCodeStride] = {-1, -1, -1, -1, -1, -1, -1, -1};
-    if (y == 0) out[2] = -2;
-    if (z == 0) out[3] = -2;
-    if (z == Lz - 1) out[4] = -2;
-    if (y == Ly - 1) out[5] = -2;
-    for (int u = 0; u < width; ++u) {
-        const int col = cidx[(size_t)row * width + u];
-        if (u > 0 && col == row) continue;  // padding
-        const int d = u == 0 ? 0 : cube_direction(row, col, Ly, Lz);
-        if (d >= 0) out[d] = ccode[(size_t)row * width + u];
-    }
-#pragma unroll
-    for (int k = 0; k < kCodeStride; ++k) dcode[(size_t)row * kCodeStride + k] = out[k];
-}
-
 struct CubeShape {
     int warps, py, pz, ne;
     int rounds;  // bodies per warp and iteration ([A] + [B])
@@ -463,33 +429,6 @@ CubeShape cube_shape(int which) {
 }
 
 }  // namespace
-
-// Does the current fixed-width copy qualify?  (dictionary with real-diagonal hopping blocks and few entries, cubic
-// lattice with Ly, Lz >= 2 and Lx >= 2, open nearest-neighbour stencil)
-int cube_probe(bdg_system *sys) {
-    EllDev &e = sys->ell;
-    e.cube_usable = false;
-    if (!e.usable || !e.dict_usable || !e.diag_usable || e.width > 7 || e.n_unique > 64) return BDG_OK;
-    const int Lx = sys->cubic[0], Ly = sys->cubic[1], Lz = sys->cubic[2];
-    if ((int64_t)Lx * Ly * Lz != e.n_sites || Lx < 2 || Ly < 2 || Lz < 2) return BDG_OK;
-    if (e.n_sites * kCodeStride > (int64_t)1 << 30) return BDG_OK;
-    BDG_TRY(ensure_scratch(sys, 2, 64));
-    int *bad = sys->scratch_i32[2].as<int>();
-    BDG_CUDA(cudaMemsetAsync(bad, 0, sizeof(int), sys->stream));
-    const int64_t n_slots = e.n_sites * e.width;
-    cube_check<<<(unsigned)ceil_div(n_slots, 256), 256, 0, sys->stream>>>(n_slots, e.width, Ly, Lz, e.idx.as<int32_t>(), bad);
-    BDG_CUDA(cudaGetLastError());
-    int host = 1;
-    BDG_CUDA(cudaMemcpyAsync(&host, bad, sizeof(int), cudaMemcpyDeviceToHost, sys->stream));
-    BDG_CUDA(cudaStreamSynchronize(sys->stream));
-    if (host != 0) return BDG_OK;
-    BDG_TRY(dev_alloc(sys, e.dcode3, (size_t)e.n_sites * kCodeStride * sizeof(int32_t)));
-    cube_codes<<<(unsigned)ceil_div(e.n_sites, 256), 256, 0, sys->stream>>>((int)e.n_sites, e.width, Ly, Lz, e.idx.as<int32_t>(),
-                                                                          e.code.as<int32_t>(), e.dcode3.as<int32_t>());
-    BDG_CUDA(cudaGetLastError());
-    e.cube_usable = true;
-    return BDG_OK;
-}
 
 // Patch shape, segment length and grid for the current recursion: the plan with the fewest body rounds on the
 // critical path (waves x planes per item x bodies per warp and plane).

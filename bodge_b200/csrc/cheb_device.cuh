@@ -42,30 +42,6 @@ __device__ __forceinline__ uint64_t mix64(uint64_t z) {
     return z ^ (z >> 31);
 }
 
-// Stencil direction of block column `col` seen from `row` on the Lx x M torus: 0 = the row itself, 1 = x-1,
-// 2 = y-1, 3 = y+1, 4 = x+1 (wrap-around included), -1 = none of these.  Lx, M >= 3 keep the five apart.
-__device__ __forceinline__ int torus_direction(int row, int col, int Lx, int M) {
-    const int xr = row / M, yr = row - xr * M, xc = col / M, yc = col - xc * M;
-    int dx = xc - xr, dy = yc - yr;
-    dx += dx < 0 ? Lx : 0;
-    dy += dy < 0 ? M : 0;
-    if (dx == 0) return dy == 0 ? 0 : (dy == M - 1 ? 2 : (dy == 1 ? 3 : -1));
-    if (dy != 0) return -1;
-    return dx == Lx - 1 ? 1 : (dx == 1 ? 4 : -1);
-}
-
-// Stencil direction of block column `col` seen from `row` on the OPEN Lx x Ly x Lz lattice (site = z + Lz (y + Ly x)):
-// 0 = the row itself, 1 = x-1, 2 = y-1, 3 = z-1, 4 = z+1, 5 = y+1, 6 = x+1, -1 = anything else (wrap-around included).
-__device__ __forceinline__ int cube_direction(int row, int col, int Ly, int Lz) {
-    const int zr = row % Lz, yr = (row / Lz) % Ly, xr = row / (Lz * Ly);
-    const int zc = col % Lz, yc = (col / Lz) % Ly, xc = col / (Lz * Ly);
-    const int dx = xc - xr, dy = yc - yr, dz = zc - zr;
-    if (dy == 0 && dz == 0) return dx == 0 ? 0 : (dx == -1 ? 1 : (dx == 1 ? 6 : -1));
-    if (dx == 0 && dz == 0) return dy == -1 ? 2 : (dy == 1 ? 5 : -1);
-    if (dx == 0 && dy == 0) return dz == -1 ? 3 : (dz == 1 ? 4 : -1);
-    return -1;
-}
-
 // ---- per-step reduction of the two dot products ---------------------------------------------
 // Every lane arrives with its partial sums for column `col` (valid iff col_ok and it is the
 // designated leader lane for that column inside the warp).  CTA partials go to global memory;

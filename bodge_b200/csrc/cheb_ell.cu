@@ -1,7 +1,8 @@
 // Chebyshev step on the kernel-native matrix format ("ELL"): fixed-width block rows, diagonal
 // block first, blocks stored in MMA B-fragment order.  This is the default step kernel for
 // lattice Hamiltonians (every row has <= 8 blocks and almost all rows have the same count);
-// ragged / long-row matrices use the generic BSR kernel in cheb.cu.
+// ragged / long-row matrices use the generic BSR kernel in cheb.cu.  formats.cu builds the format and
+// keeps it current after a scatter.
 //
 // Formulation.  For block B = Br + i Bi (4x4) and record X = Xr + i Xi (4 components x PW columns)
 //     Y^T = X^T B^T :   acc1 = Xr^T * Bop,  acc2 = Xi^T * Bop,   Bop[b][2a]   = Br[a][b]
@@ -249,278 +250,6 @@ cheb_step_ell(const int32_t *__restrict__ cidx, const int32_t *__restrict__ ccod
                             tickets, dots_step);
 }
 
-// ---- building the format ----------------------------------------------------------------------
-// need[row] = blocks of the row, +1 if the diagonal block is absent (slot 0 is reserved for it)
-__global__ void __launch_bounds__(256)
-ell_row_need(int n_sites, const int32_t *__restrict__ indptr, const int32_t *__restrict__ indices,
-             int *__restrict__ max_need) {
-    const int row = blockIdx.x * blockDim.x + threadIdx.x;
-    int need = 0;
-    if (row < n_sites) {
-        const int p0 = indptr[row], p1 = indptr[row + 1];
-        bool self = false;
-        for (int p = p0; p < p1; ++p) self |= indices[p] == row;
-        need = p1 - p0 + (self ? 0 : 1);
-    }
-#pragma unroll
-    for (int d = 16; d; d >>= 1) need = max(need, __shfl_xor_sync(0xffffffffu, need, d));
-    if ((threadIdx.x & 31) == 0 && need > 0) atomicMax(max_need, need);
-}
-
-// One warp per (row, slot); lane l writes double l of the slot in B-fragment order.
-__global__ void __launch_bounds__(256)
-ell_fill(int n_sites, int width, const int32_t *__restrict__ indptr, const int32_t *__restrict__ indices,
-         const double *__restrict__ data, int32_t *__restrict__ cidx, double *__restrict__ cdata) {
-    const int64_t w = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    const int lane = threadIdx.x & 31;
-    if (w >= (int64_t)n_sites * width) return;
-    const int row = (int)(w / width), slot = (int)(w % width);
-    const int p0 = indptr[row], cnt = indptr[row + 1] - p0;
-    int self = -1;  // position of the diagonal block inside the row
-    for (int t = 0; t < cnt; ++t)
-        if (indices[p0 + t] == row) self = t;
-    int src;  // position inside the row feeding this slot, or -1
-    if (slot == 0) {
-        src = self;
-    } else {
-        src = slot - 1;
-        if (self >= 0 && src >= self) src += 1;
-        if (src >= cnt) src = -1;
-    }
-    double v = 0.0;
-    if (src >= 0) {
-        const int a = lane >> 3, part = (lane >> 2) & 1, b = lane & 3;
-        v = data[((size_t)(p0 + src) * 16 + a * 4 + b) * 2 + part];
-    }
-    cdata[w * 32 + lane] = v;
-    if (lane == 0) cidx[w] = src >= 0 ? indices[p0 + src] : row;
-}
-
-// ---- block dictionary ---------------------------------------------------------------------------
-// Distinct blocks are found with an open-addressing hash table keyed by a 64-bit hash of the
-// block's 256 bytes; every slot is then compared bit for bit with its table entry, so a hash
-// collision can only disable the format, never change a result.
-constexpr unsigned long long kEmptyKey = ~0ull;
-
-// One warp per slot: hash, find-or-insert, remember the table position and the smallest slot id
-// holding that key (the representative whose bytes become the table entry).  The table is sized
-// for few distinct blocks; when more than `limit` keys have been inserted the pass is abandoned
-// (*overflow = 1) and the host retries with a larger table or gives the format up.
-__global__ void __launch_bounds__(256)
-dict_insert(int64_t n_slots, const double *__restrict__ cdata, unsigned long long *__restrict__ keys,
-            int *__restrict__ rep, unsigned cap_mask, int32_t *__restrict__ where, int *__restrict__ counter,
-            int limit, int *__restrict__ overflow) {
-    const int64_t w = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    const int lane = threadIdx.x & 31;
-    if (w >= n_slots) return;
-    const uint64_t bits = (uint64_t)__double_as_longlong(cdata[w * 32 + lane]);
-    uint64_t h = mix64(bits + 0x9E3779B97F4A7C15ull * (uint64_t)(lane + 1));
-#pragma unroll
-    for (int d = 16; d; d >>= 1) h += __shfl_xor_sync(0xffffffffu, h, d);
-    h = mix64(h);
-    if (h == kEmptyKey) h = 0x1234567ull;
-    if (lane != 0) return;
-    unsigned pos = (unsigned)h & cap_mask;
-    for (;;) {
-        unsigned long long seen = *((volatile unsigned long long *)(keys + pos));  // cheap hit for repeated blocks
-        if (seen == kEmptyKey) {
-            seen = atomicCAS(keys + pos, kEmptyKey, (unsigned long long)h);
-            if (seen == kEmptyKey && atomicAdd(counter, 1) >= limit) *overflow = 1;
-        }
-        if (seen == kEmptyKey || seen == h) break;
-        if (*((volatile int *)overflow)) {
-            where[w] = 0;
-            return;
-        }
-        pos = (pos + 1) & cap_mask;
-    }
-    if (*((volatile int *)(rep + pos)) > (int)w) atomicMin(rep + pos, (int)w);
-    where[w] = (int32_t)pos;
-}
-
-// flag[slot] = 1 iff the slot is the representative of its key (the smallest slot id holding that block).  The
-// exclusive scan of the flags numbers the distinct blocks in SLOT order, so the table follows the matrix: the
-// on-site blocks of consecutive sites sit next to each other (a kernel that fetches a site-dependent on-site
-// block per row then streams the table instead of gathering 256-byte pieces from all over it).
-__global__ void __launch_bounds__(256)
-dict_flag_reps(int64_t n_slots, const int *__restrict__ rep, const int32_t *__restrict__ where, int32_t *__restrict__ flag) {
-    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (t < n_slots) flag[t] = rep[where[t]] == (int)t;
-}
-
-// One warp per slot: code = rank of its representative among the representatives (dense[]: scanned flags); the
-// representative writes the table entry; everyone else is compared with the representative's bytes.
-__global__ void __launch_bounds__(256)
-dict_emit(int64_t n_slots, const double *__restrict__ cdata, const int *__restrict__ rep,
-          const int32_t *__restrict__ dense, const int32_t *__restrict__ where, int32_t *__restrict__ ccode,
-          double *__restrict__ table, int table_cap, int32_t *__restrict__ posid, int *__restrict__ mismatch) {
-    const int64_t w = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    const int lane = threadIdx.x & 31;
-    if (w >= n_slots) return;
-    const int r = rep[where[w]];
-    const int code = dense[r];
-    const long long mine = __double_as_longlong(cdata[w * 32 + lane]);
-    if (r == (int)w) {
-        if (code < table_cap) table[(size_t)code * 32 + lane] = __longlong_as_double(mine);
-        if (lane == 0) posid[where[w]] = code;  // hash position -> code: later updates look new blocks up here (ell_patch)
-    } else if (mine != __double_as_longlong(cdata[(int64_t)r * 32 + lane])) {
-        *mismatch = 1;
-    }
-    if (lane == 0) ccode[w] = code;
-}
-
-// dtab[code][a] = Re of diagonal entry (a, a) of table block `code`; isdiag[code] = the block has
-// nothing else (all other real and imaginary parts compare == 0).
-__global__ void __launch_bounds__(256)
-dict_diag_table(int n_unique, const double *__restrict__ table, double *__restrict__ dtab, int *__restrict__ isdiag) {
-    const int w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
-    if (w >= n_unique) return;
-    const double v = table[(size_t)w * 32 + lane];
-    const int a = lane >> 3, part = (lane >> 2) & 1, b = lane & 3;  // double `lane` = part (re/im) of entry (a, b)
-    const bool on_diag = part == 0 && a == b;
-    const unsigned other = __ballot_sync(0xffffffffu, !on_diag && v != 0.0);
-    if (on_diag) dtab[(size_t)w * 4 + a] = v;
-    if (lane == 0) isdiag[w] = other == 0u;
-}
-
-// bad[0] = 1 if any slot other than slot 0 holds a block that is not real-diagonal, bad[1] = 1 if any slot 0 does.
-__global__ void __launch_bounds__(256)
-dict_offsite_diag(int64_t n_slots, int width, const int32_t *__restrict__ ccode, const int *__restrict__ isdiag,
-                  int *__restrict__ bad) {
-    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= n_slots) return;
-    if (!isdiag[ccode[t]]) bad[t % width == 0 ? 1 : 0] = 1;
-}
-
-// ---- incremental update after a scatter (SURVEY 8f-3: re-enter `with`, change a few terms, ask again) -----------
-// One warp per touched skeleton block: copy it into its place in `packed`, into its fixed-width slot (fragment
-// order), look it up in -- or add it to -- the dictionary and rewrite the slot's code (and direction code).
-// status: [0] distinct blocks so far, [1] zero pattern changed, [2] table full, [3] hash collision, [4] an
-// off-site block that is not real-diagonal (the DIAG kernels no longer apply), [5] an on-site block that is not (SD).
-struct PatchArgs {
-    const int32_t *s_indices, *s_brow;
-    const double *s_data;
-    const int32_t *flags, *pos;
-    double *p_data;
-    int width;
-    const int32_t *cidx;
-    double *cdata;
-    int32_t *ccode;
-    int dict;
-    unsigned long long *keys;
-    int32_t *posid;
-    unsigned cap_mask;
-    double *table, *dtab;
-    int table_cap, diag_required, self_diag_required;
-    int32_t *dcode;
-    int Lx, M;
-    int32_t *dcode3;
-    int Ly, Lz;
-    int *status;
-};
-
-__global__ void __launch_bounds__(256)
-patch_blocks(int64_t n, const int32_t *__restrict__ klist, const PatchArgs a) {
-    const int64_t w = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    const int lane = threadIdx.x & 31;
-    if (w >= n) return;
-    const int k = klist[w];
-    if (k < 0) return;
-    const double vs = a.s_data[(size_t)k * 32 + lane];  // skeleton order: (row a, column b, re/im) = double (a*4+b)*2+part
-    const bool nz = __ballot_sync(kFull, vs != 0.0) != 0u;
-    if (nz != (a.flags[k] != 0)) {
-        if (lane == 0) a.status[1] = 1;
-        return;
-    }
-    if (!nz) return;
-    a.p_data[(size_t)a.pos[k] * 32 + lane] = vs;
-    if (a.width == 0) return;
-    const int row = a.s_brow[k], col = a.s_indices[k];
-    int u = 0;
-    if (col != row) {
-        const bool hit = lane >= 1 && lane < a.width && a.cidx[(size_t)row * a.width + lane] == col;
-        const unsigned m = __ballot_sync(kFull, hit);
-        if (m == 0u) {  // cannot happen for a block that was already stored
-            if (lane == 0) a.status[1] = 1;
-            return;
-        }
-        u = __ffs(m) - 1;
-    }
-    const int64_t slot = (int64_t)row * a.width + u;
-    const int fa = lane >> 3, part = (lane >> 2) & 1, fb = lane & 3;  // fragment order (ell_fill)
-    const double f = a.s_data[(size_t)k * 32 + (fa * 4 + fb) * 2 + part];
-    a.cdata[slot * 32 + lane] = f;
-    if (!a.dict) return;
-    uint64_t h = mix64((uint64_t)__double_as_longlong(f) + 0x9E3779B97F4A7C15ull * (uint64_t)(lane + 1));
-#pragma unroll
-    for (int d = 16; d; d >>= 1) h += __shfl_xor_sync(kFull, h, d);
-    h = mix64(h);
-    if (h == kEmptyKey) h = 0x1234567ull;
-    int id = -1, won = 0;
-    unsigned pos = 0;
-    if (lane == 0) {
-        pos = (unsigned)h & a.cap_mask;
-        for (;;) {
-            unsigned long long seen = *((volatile unsigned long long *)(a.keys + pos));
-            if (seen == kEmptyKey) {
-                seen = atomicCAS(a.keys + pos, kEmptyKey, (unsigned long long)h);
-                if (seen == kEmptyKey) {
-                    won = 1;
-                    id = atomicAdd(a.status, 1);
-                    if (id >= a.table_cap) {
-                        a.status[2] = 1;
-                        id = -2;
-                    }
-                    break;
-                }
-            }
-            if (seen == h) break;
-            pos = (pos + 1) & a.cap_mask;
-        }
-        if (!won) {  // someone holds the key: its code is published once the table entry is in place
-            while ((id = *((volatile int32_t *)(a.posid + pos))) == -1) {}
-        }
-    }
-    id = __shfl_sync(kFull, id, 0);
-    won = __shfl_sync(kFull, won, 0);
-    pos = __shfl_sync(kFull, pos, 0);
-    const bool on_diag = part == 0 && fa == fb;
-    const bool isdiag = __ballot_sync(kFull, !on_diag && f != 0.0) == 0u;
-    if (won) {
-        if (id >= 0) {
-            a.table[(size_t)id * 32 + lane] = f;
-            if (on_diag) a.dtab[(size_t)id * 4 + fa] = f;
-            __threadfence();
-        }
-        __syncwarp();
-        if (lane == 0) *((volatile int32_t *)(a.posid + pos)) = id;
-    }
-    if (id < 0) {
-        if (lane == 0) a.status[2] = 1;
-        return;
-    }
-    if (!won) {
-        const double have = *((volatile const double *)(a.table + (size_t)id * 32 + lane));
-        if (__ballot_sync(kFull, __double_as_longlong(have) != __double_as_longlong(f)) != 0u) {
-            if (lane == 0) a.status[3] = 1;
-            return;
-        }
-    }
-    if (lane == 0) {
-        if (u > 0 && a.diag_required && !isdiag) a.status[4] = 1;
-        if (u == 0 && a.self_diag_required && !isdiag) a.status[5] = 1;  // the SD variants no longer apply: the plain ones take over
-        a.ccode[slot] = id;
-        if (a.dcode) {
-            const int dir = u == 0 ? 0 : torus_direction(row, col, a.Lx, a.M);
-            if (dir >= 0) a.dcode[(size_t)row * 5 + dir] = id;
-        }
-        if (a.dcode3) {
-            const int dir = u == 0 ? 0 : cube_direction(row, col, a.Ly, a.Lz);
-            if (dir >= 0) a.dcode3[(size_t)row * 8 + dir] = id;
-        }
-    }
-}
-
 template <int PW, int NP, bool DICT, bool DIAG, bool SD> EllKernel pick_ch(int width) {
     switch (width) {
         case 3: return cheb_step_ell<PW, 3, NP, DICT, DIAG, SD>;
@@ -598,203 +327,7 @@ RowWalk plan_walk(const bdg_system *sys, int n_sites, int64_t slots, const PlanS
     return w;
 }
 
-// Build the block dictionary of the fixed-width matrix copy (e.idx / e.data must exist).
-int dict_build(bdg_system *sys) {
-    EllDev &e = sys->ell;
-    e.dict_usable = false;
-    e.n_unique = 0;
-    const int64_t n_slots = e.n_sites * e.width;
-    if (n_slots <= 0 || n_slots > (int64_t)1 << 30) return BDG_OK;
-    // Worth it when the table is a small fraction of the matrix (each distinct block is still
-    // read from HBM about once per step; the codes cost 4 bytes per slot).
-    const int64_t max_unique = std::max<int64_t>(1, n_slots * env_int("BDG_DICT_MAX_PERCENT", 35) / 100);
-    BDG_TRY(dev_alloc(sys, e.tmp_where, (size_t)n_slots * sizeof(int32_t)));
-    BDG_TRY(ensure_scratch(sys, 2, 64));
-    int *scal = sys->scratch_i32[2].as<int>();  // [0] keys inserted, [1] overflow, [2] distinct (scan), [3] mismatch
-    const unsigned warps_grid = (unsigned)ceil_div(n_slots * 32, 256);
-    // Lattice Hamiltonians have a handful of distinct blocks: start with a small table (cheap to
-    // clear and to scan) and grow it only when it fills up.
-    int64_t cap = 1 << 16;
-    int host[4] = {0, 0, 0, 0};
-    for (;;) {
-        const int limit = (int)std::min<int64_t>(cap / 2, max_unique);
-        BDG_TRY(dev_alloc(sys, e.tmp_keys, (size_t)cap * sizeof(unsigned long long)));
-        BDG_TRY(dev_alloc(sys, e.tmp_rep, (size_t)cap * sizeof(int)));
-        BDG_TRY(dev_alloc(sys, e.tmp_dense, (size_t)(n_slots + 1) * sizeof(int32_t)));
-        BDG_CUDA(cudaMemsetAsync(e.tmp_keys.ptr, 0xff, (size_t)cap * sizeof(unsigned long long), sys->stream));
-        BDG_CUDA(cudaMemsetAsync(e.tmp_rep.ptr, 0x7f, (size_t)cap * sizeof(int), sys->stream));
-        BDG_CUDA(cudaMemsetAsync(scal, 0, 4 * sizeof(int), sys->stream));
-        dict_insert<<<warps_grid, 256, 0, sys->stream>>>(n_slots, e.data.as<double>(), e.tmp_keys.as<unsigned long long>(),
-                                                         e.tmp_rep.as<int>(), (unsigned)(cap - 1), e.tmp_where.as<int32_t>(),
-                                                         scal, limit, scal + 1);
-        BDG_CUDA(cudaGetLastError());
-        BDG_CUDA(cudaMemcpyAsync(host, scal, 2 * sizeof(int), cudaMemcpyDeviceToHost, sys->stream));
-        BDG_CUDA(cudaStreamSynchronize(sys->stream));
-        e.n_unique = host[0];  // exact unless the pass was abandoned (then: at least this many)
-        if (!host[1]) break;
-        if (limit >= max_unique) return BDG_OK;  // too many distinct blocks: keep the plain format
-        cap <<= 4;
-    }
-    dict_flag_reps<<<(unsigned)ceil_div(n_slots, 256), 256, 0, sys->stream>>>(n_slots, e.tmp_rep.as<int>(), e.tmp_where.as<int32_t>(),
-                                                                              e.tmp_dense.as<int32_t>());
-    BDG_CUDA(cudaGetLastError());
-    BDG_TRY(exclusive_scan_i32(sys, e.tmp_dense.as<int32_t>(), e.tmp_dense.as<int32_t>(), n_slots, scal + 2));
-    const int n_unique = host[0];
-    // Head room for blocks that later scatters add (ell_patch): half as many again, at least 64 Ki, and never more than
-    // three quarters of the hash table.
-    e.hash_cap = cap;
-    e.table_cap = std::min<int64_t>(std::max<int64_t>(n_unique + n_unique / 2, n_unique + 65536), cap * 3 / 4);
-    e.table_cap = std::max<int64_t>(e.table_cap, n_unique);
-    BDG_TRY(dev_alloc(sys, e.code, (size_t)n_slots * sizeof(int32_t)));
-    BDG_TRY(dev_alloc(sys, e.table, (size_t)e.table_cap * 32 * sizeof(double)));
-    BDG_TRY(dev_alloc(sys, e.posid, (size_t)cap * sizeof(int32_t)));
-    BDG_TRY(dev_alloc(sys, e.counters, 8 * sizeof(int)));
-    BDG_CUDA(cudaMemsetAsync(e.posid.ptr, 0xff, (size_t)cap * sizeof(int32_t), sys->stream));
-    dict_emit<<<warps_grid, 256, 0, sys->stream>>>(n_slots, e.data.as<double>(), e.tmp_rep.as<int>(),
-                                                   e.tmp_dense.as<int32_t>(), e.tmp_where.as<int32_t>(),
-                                                   e.code.as<int32_t>(), e.table.as<double>(), n_unique, e.posid.as<int32_t>(),
-                                                   scal + 3);
-    BDG_CUDA(cudaGetLastError());
-    BDG_CUDA(cudaMemcpyAsync(host + 2, scal + 2, 2 * sizeof(int), cudaMemcpyDeviceToHost, sys->stream));
-    BDG_CUDA(cudaStreamSynchronize(sys->stream));
-    e.dict_usable = host[3] == 0 && host[2] == n_unique;  // no hash collision, table fully written
-    // Real-diagonal off-site blocks (DIAG kernels)?
-    e.diag_usable = false;
-    e.self_diag_usable = false;
-    if (e.dict_usable) {
-        BDG_TRY(dev_alloc(sys, e.dtab, (size_t)e.table_cap * 4 * sizeof(double)));
-        BDG_TRY(dev_alloc(sys, e.tmp_rep, (size_t)std::max<int64_t>(cap, n_unique) * sizeof(int)));  // reuse as isdiag[]
-        BDG_CUDA(cudaMemsetAsync(scal, 0, 2 * sizeof(int), sys->stream));
-        dict_diag_table<<<(unsigned)ceil_div((int64_t)n_unique * 32, 256), 256, 0, sys->stream>>>(
-            n_unique, e.table.as<double>(), e.dtab.as<double>(), e.tmp_rep.as<int>());
-        dict_offsite_diag<<<(unsigned)ceil_div(n_slots, 256), 256, 0, sys->stream>>>(
-            n_slots, e.width, e.code.as<int32_t>(), e.tmp_rep.as<int>(), scal);
-        BDG_CUDA(cudaGetLastError());
-        BDG_CUDA(cudaMemcpyAsync(host, scal, 2 * sizeof(int), cudaMemcpyDeviceToHost, sys->stream));
-        BDG_CUDA(cudaStreamSynchronize(sys->stream));
-        e.diag_usable = host[0] == 0;
-        e.self_diag_usable = host[1] == 0;
-    }
-    return BDG_OK;
-}
-
 }  // namespace
-
-void ell_release(bdg_system *sys) {
-    dev_free(sys, sys->ell.idx);
-    dev_free(sys, sys->ell.data);
-    dev_free(sys, sys->ell.code);
-    dev_free(sys, sys->ell.table);
-    dev_free(sys, sys->ell.dtab);
-    dev_free(sys, sys->ell.dcode);
-    dev_free(sys, sys->ell.dcode3);
-    dev_free(sys, sys->ell.tmp_keys);
-    dev_free(sys, sys->ell.tmp_rep);
-    dev_free(sys, sys->ell.tmp_where);
-    dev_free(sys, sys->ell.tmp_dense);
-    dev_free(sys, sys->ell.posid);
-    dev_free(sys, sys->ell.counters);
-    sys->ell = EllDev();
-}
-
-int ell_build(bdg_system *sys) {
-    EllDev &e = sys->ell;
-    if (e.valid) return BDG_OK;
-    BDG_TRY(build_packed(sys));
-    const BsrDev &m = sys->packed;
-    const int n = (int)m.n_sites;
-    e.usable = false;
-    e.dict_usable = false;
-    e.diag_usable = false;
-    e.self_diag_usable = false;
-    e.pair_usable = false;
-    e.cube_usable = false;
-    e.n_unique = 0;
-    e.n_sites = n;
-    if (n > 0) {
-        BDG_TRY(ensure_scratch(sys, 2, 64));
-        int *max_need = sys->scratch_i32[2].as<int>();
-        BDG_CUDA(cudaMemsetAsync(max_need, 0, sizeof(int), sys->stream));
-        ell_row_need<<<(unsigned)ceil_div(n, 256), 256, 0, sys->stream>>>(n, m.indptr.as<int32_t>(),
-                                                                         m.indices.as<int32_t>(), max_need);
-        BDG_CUDA(cudaGetLastError());
-        int need = 0;
-        BDG_CUDA(cudaMemcpyAsync(&need, max_need, sizeof(int), cudaMemcpyDeviceToHost, sys->stream));
-        BDG_CUDA(cudaStreamSynchronize(sys->stream));
-        const int width = std::max(need, 3);
-        // Padding costs matrix traffic: accept it when small, or when the matrix is too small to matter.
-        const bool cheap = (int64_t)n * width * 4 <= m.n_blocks * 5 || (int64_t)n * width <= (1 << 16);
-        if (width <= 8 && cheap) {
-            e.width = width;
-            BDG_TRY(dev_alloc(sys, e.idx, (size_t)n * width * sizeof(int32_t)));
-            BDG_TRY(dev_alloc(sys, e.data, (size_t)n * width * 32 * sizeof(double)));
-            const int64_t threads = (int64_t)n * width * 32;
-            ell_fill<<<(unsigned)ceil_div(threads, 256), 256, 0, sys->stream>>>(
-                n, width, m.indptr.as<int32_t>(), m.indices.as<int32_t>(), m.data.as<double>(), e.idx.as<int32_t>(),
-                e.data.as<double>());
-            BDG_CUDA(cudaGetLastError());
-            e.usable = true;
-            BDG_TRY(dict_build(sys));
-            BDG_TRY(pair_probe(sys));
-            BDG_TRY(cube_probe(sys));
-        }
-    }
-    e.valid = true;
-    sys->stats[1] += 1;
-    return BDG_OK;
-}
-
-int ell_patch(bdg_system *sys, int64_t n, const int32_t *klist, bool *ok) {
-    EllDev &e = sys->ell;
-    *ok = false;
-    if (!sys->packed_valid || !e.valid || !sys->pack_flags.ptr || !sys->pack_pos.ptr) return BDG_OK;
-    if (env_int("BDG_NO_PATCH", 0)) return BDG_OK;  // A/B: always rebuild
-    if (n == 0) {
-        *ok = true;
-        return BDG_OK;
-    }
-    const bool dict = e.usable && e.dict_usable;
-    if (e.usable && !dict && e.n_unique > 0) return BDG_OK;  // a dictionary was attempted and given up: rebuild decides again
-    BDG_TRY(dev_alloc(sys, e.counters, 8 * sizeof(int)));
-    int host[6] = {(int)e.n_unique, 0, 0, 0, 0, 0};
-    BDG_CUDA(cudaMemcpyAsync(e.counters.ptr, host, sizeof(host), cudaMemcpyHostToDevice, sys->stream));
-    PatchArgs a{};
-    a.s_indices = sys->skel.indices.as<int32_t>();
-    a.s_brow = sys->skel.brow.as<int32_t>();
-    a.s_data = sys->skel.data.as<double>();
-    a.flags = sys->pack_flags.as<int32_t>();
-    a.pos = sys->pack_pos.as<int32_t>();
-    a.p_data = sys->packed.data.as<double>();
-    a.width = e.usable ? e.width : 0;
-    a.cidx = e.idx.as<int32_t>();
-    a.cdata = e.data.as<double>();
-    a.ccode = e.code.as<int32_t>();
-    a.dict = dict ? 1 : 0;
-    a.keys = e.tmp_keys.as<unsigned long long>();
-    a.posid = e.posid.as<int32_t>();
-    a.cap_mask = (unsigned)(e.hash_cap - 1);
-    a.table = e.table.as<double>();
-    a.dtab = e.dtab.as<double>();
-    a.table_cap = (int)e.table_cap;
-    a.diag_required = e.diag_usable ? 1 : 0;
-    a.self_diag_required = e.self_diag_usable && !e.diag_usable ? 1 : 0;  // (only the SD kernel relies on it)
-    a.dcode = e.pair_usable ? e.dcode.as<int32_t>() : nullptr;
-    a.Lx = sys->cubic[0];
-    a.M = e.pair_M;
-    a.dcode3 = e.cube_usable ? e.dcode3.as<int32_t>() : nullptr;
-    a.Ly = sys->cubic[1];
-    a.Lz = sys->cubic[2];
-    a.status = e.counters.as<int>();
-    patch_blocks<<<(unsigned)ceil_div(n * 32, 256), 256, 0, sys->stream>>>(n, klist, a);
-    BDG_CUDA(cudaGetLastError());
-    BDG_CUDA(cudaMemcpyAsync(host, e.counters.ptr, sizeof(host), cudaMemcpyDeviceToHost, sys->stream));
-    BDG_CUDA(cudaStreamSynchronize(sys->stream));
-    if (host[1] || host[2] || host[3] || host[4]) return BDG_OK;  // pattern / capacity / collision / DIAG precondition: rebuild
-    e.n_unique = host[0];
-    if (host[5]) e.self_diag_usable = false;  // an on-site block with off-diagonal entries: same format, MMA on-site product
-    *ok = true;
-    return BDG_OK;
-}
 
 // The single-step kernel of the current recursion, its panels per group, grid and row traversal.
 int ell_configure(bdg_system *sys, const PlanSwitches &sw) {

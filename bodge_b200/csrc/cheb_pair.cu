@@ -60,14 +60,12 @@ constexpr int kRingN = 8;       // planes of the T_n ring: three in use, five in
 // ms/step, DESIGN 4.1-iv) left this one ahead.
 constexpr int kPairWarps = 8, kPairSites = 2, kPairMinBlocks = 2;
 
-constexpr int kDirs = 5;  // direction-ordered row: self, x-1, y-1, y+1, x+1 (= ascending block column)
-
 // B fragments of the S rows a warp handles (cheb_ell.cu: DICT / DIAG), held in registers from plane to
 // plane and reloaded only when a code differs from the held one.  Lane s * 5 + u carries the code of
 // row s, direction u; code < 0 = no block.  SELF: the on-site fragments (u = 0) are not held -- they are
 // fetched per row, one plane ahead (self_fragments) -- so their codes do not take part in the test.
 template <bool DIAG, bool SELF, int S, bool SD = false>
-__device__ __forceinline__ void hold_fragments(int jv, int &jheld, double (&keep)[S][kDirs], const double *__restrict__ table,
+__device__ __forceinline__ void hold_fragments(int jv, int &jheld, double (&keep)[S][kPlaneCodes], const double *__restrict__ table,
                                                const double *__restrict__ dtab, int lane, bool self_lane) {
     const unsigned changed = __ballot_sync(kFull, jv != jheld && !(SELF && self_lane));
     if (changed) {
@@ -75,9 +73,9 @@ __device__ __forceinline__ void hold_fragments(int jv, int &jheld, double (&keep
 #pragma unroll
         for (int s = 0; s < S; ++s) {
 #pragma unroll
-            for (int u = SELF ? 1 : 0; u < kDirs; ++u) {
-                const int code = __shfl_sync(kFull, jv, s * kDirs + u);
-                const unsigned take = changed >> (s * kDirs + u) & 1u;
+            for (int u = SELF ? 1 : 0; u < kPlaneCodes; ++u) {
+                const int code = __shfl_sync(kFull, jv, s * kPlaneCodes + u);
+                const unsigned take = changed >> (s * kPlaneCodes + u) & 1u;
                 const size_t c = (size_t)max(code, 0);
                 const double *entry = ((DIAG && u > 0) || (SD && u == 0)) ? dtab + c * 4 + (lane & 3) : table + c * 32 + lane;
                 ld_table_pred(keep[s][u], entry, take && code >= 0);
@@ -96,7 +94,7 @@ __device__ __forceinline__ void self_fragments(int jv, double (&f)[S], const dou
                                                int lane) {
 #pragma unroll
     for (int s = 0; s < S; ++s) {
-        const int code = __shfl_sync(kFull, jv, s * kDirs);
+        const int code = __shfl_sync(kFull, jv, s * kPlaneCodes);
         f[s] = 0.0;
         ld_table_pred(f[s], SD ? dtab + (size_t)max(code, 0) * 4 + (lane & 3) : table + (size_t)max(code, 0) * 32 + lane, code >= 0);
     }
@@ -134,7 +132,7 @@ template <bool DIAG, bool SD = false> struct RowSum {
 
 template <bool DIAG, bool SD = false>
 __device__ __forceinline__ void row_product(const double2 &x0, const double2 &x1, const double2 &x2, const double2 &x3,
-                                            const double2 &x4, double b0, const double (&bop)[kDirs], double &yr, double &yi) {
+                                            const double2 &x4, double b0, const double (&bop)[kPlaneCodes], double &yr, double &yi) {
     RowSum<DIAG, SD> r;
     r.begin(x0, b0);
     r.add(x1, bop[1]);
@@ -153,8 +151,8 @@ __device__ __forceinline__ void row_product(const double2 &x0, const double2 &x1
 //
 // Geometry is a TORUS: planes x and in-plane sites y are taken modulo Lx and M, so the halo of the first /
 // last patch and of the first / last segment is the opposite face of the lattice (staged by its own small bulk
-// copy).  What is connected is decided by the matrix alone: it arrives as `dcode[row][5]`, the dictionary code
-// of the row's block in each stencil direction (self, x-1, y-1, y+1, x+1; -1 = none), so the reference's
+// copy).  What is connected is decided by the matrix alone: it arrives as `dcode[row][kPlaneCodes]`, the dictionary
+// code of the row's block in each stencil direction (self, x-1, y-1, y+1, x+1; kNoBlock = none), so the reference's
 // periodic skeleton with the edges filled in (bodge/lattice.py:161-197) and the open lattice it leaves when they
 // are not run the same code: a direction without a block meets a zero fragment (whatever finite vector value
 // sits at the wrapped position is multiplied by zero; the rings are cleared once).  The records a row needs sit
@@ -220,16 +218,16 @@ cheb_pair_step(const int32_t *__restrict__ dcode, const double *__restrict__ tab
     uint32_t a1 = sT1 + (uint32_t)l0 * R + (uint32_t)lane * 16u;
     pin(aN), pin(a1);
 
-    double keep[S][kDirs];
+    double keep[S][kPlaneCodes];
     int jheld = -2;
 #pragma unroll
     for (int s = 0; s < S; ++s)
 #pragma unroll
-        for (int u = 0; u < kDirs; ++u) keep[s][u] = 0.0;
+        for (int u = 0; u < kPlaneCodes; ++u) keep[s][u] = 0.0;
     // lanes 0 .. 5 S - 1 carry the codes of the warp's rows: lane = s * 5 + direction
-    const int csite = lane / kDirs, cdir = lane - csite * kDirs;
-    const bool code_lane = lane < S * kDirs, self_lane = cdir == 0;
-    const int plane_codes = wk.M * kDirs, all_codes = wk.Lx * plane_codes;
+    const int csite = lane / kPlaneCodes, cdir = lane - csite * kPlaneCodes;
+    const bool code_lane = lane < S * kPlaneCodes, self_lane = cdir == 0;
+    const int plane_codes = wk.M * kPlaneCodes, all_codes = wk.Lx * plane_codes;
 
     const int item0 = LISTED ? wk.lists.cta_begin[blockIdx.x] : (int)blockIdx.x, item1 = LISTED ? wk.lists.cta_begin[blockIdx.x + 1] : wk.n_items;
     for (int item = item0; item < item1; item += LISTED ? 1 : (int)gridDim.x) {
@@ -303,7 +301,7 @@ cheb_pair_step(const int32_t *__restrict__ dcode, const double *__restrict__ tab
         // code index of this lane's (row, direction) in plane 0; rows past the halo (ragged patch) wrap anywhere valid
         int yl = (ya + csite) % wk.M;
         yl += yl < 0 ? wk.M : 0;
-        const int coff = yl * kDirs + cdir;
+        const int coff = yl * kPlaneCodes + cdir;
         int cplane = x0 - 1;  // plane of [A] in iteration 0
         cplane += cplane < 0 ? wk.Lx : 0;
         cplane *= plane_codes;
@@ -478,39 +476,6 @@ cheb_pair_step(const int32_t *__restrict__ dcode, const double *__restrict__ tab
     }
 }
 
-// *bad = 1 unless every block column of the fixed-width copy is the row itself or one of its four nearest
-// neighbours on the (x, in-plane) torus -- the open stencil and the reference's periodic one both qualify.
-__global__ void __launch_bounds__(256)
-pair_check(int64_t n_slots, int width, int Lx, int M, const int32_t *__restrict__ cidx, int *__restrict__ bad) {
-    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= n_slots) return;
-    const int row = (int)(t / width);
-    if (torus_direction(row, cidx[t], Lx, M) < 0) *bad = 1;
-}
-
-// dcode[row][dir] = dictionary code of the row's block towards (self, x-1, y-1, y+1, x+1), -1 = none.
-// Slot 0 of the fixed-width copy is the diagonal block; padding slots point at the row itself.
-__global__ void __launch_bounds__(256)
-pair_codes(int n_sites, int width, int Lx, int M, const int32_t *__restrict__ cidx, const int32_t *__restrict__ ccode,
-           int32_t *__restrict__ dcode, int *__restrict__ wraps /* set to 1 when a block wraps around in-plane */) {
-    const int row = blockIdx.x * blockDim.x + threadIdx.x;
-    if (row >= n_sites) return;
-    const int y = row % M;
-    int out[kDirs] = {-1, -1, -1, -1, -1};
-    for (int u = 0; u < width; ++u) {
-        const int c = ccode[(size_t)row * width + u];
-        const int d = u == 0 ? 0 : torus_direction(row, cidx[(size_t)row * width + u], Lx, M);
-        if (u == 0) out[0] = c;
-        else if (d == 1) out[1] = c;
-        else if (d == 2) out[2] = c;
-        else if (d == 3) out[3] = c;
-        else if (d == 4) out[4] = c;
-    }
-#pragma unroll
-    for (int k = 0; k < kDirs; ++k) dcode[(size_t)row * kDirs + k] = out[k];
-    if ((y == 0 && out[2] >= 0) || (y == M - 1 && out[3] >= 0)) *wraps = 1;
-}
-
 template <bool LISTED> PairKernel pick_pair(bool diag, bool self, bool t2, bool sd) {
     if (sd && !diag) {  // general hopping blocks, real-diagonal on-site blocks
         if (self) return t2 ? cheb_pair_step<false, true, 1, true, LISTED> : cheb_pair_step<false, true, 0, true, LISTED>;
@@ -530,42 +495,6 @@ constexpr size_t kPairSmem = ((size_t)kRingN * (kPairWarps * kPairSites + 2) + (
                              8 * (kRingN + 1);
 
 }  // namespace
-
-// Does the current fixed-width copy qualify?  (dictionary built, one-dimensional x-planes of >= 3 sites, >= 3
-// planes, nearest-neighbour stencil -- open or periodic --, rows of <= 5 blocks)
-int pair_probe(bdg_system *sys) {
-    EllDev &e = sys->ell;
-    e.pair_usable = false;
-    e.pair_M = 0;
-    if (!e.usable || !e.dict_usable || e.width > 5 || e.width < 3) return BDG_OK;
-    const int Lx = sys->cubic[0], Ly = sys->cubic[1], Lz = sys->cubic[2];
-    if ((int64_t)Lx * Ly * Lz != e.n_sites) return BDG_OK;
-    const int M = Lz == 1 ? Ly : (Ly == 1 ? Lz : 0);
-    if (M < 3 || Lx < 3) return BDG_OK;
-    BDG_TRY(ensure_scratch(sys, 2, 64));
-    int *bad = sys->scratch_i32[2].as<int>();
-    BDG_CUDA(cudaMemsetAsync(bad, 0, sizeof(int), sys->stream));
-    const int64_t n_slots = e.n_sites * e.width;
-    pair_check<<<(unsigned)ceil_div(n_slots, 256), 256, 0, sys->stream>>>(n_slots, e.width, Lx, M, e.idx.as<int32_t>(), bad);
-    BDG_CUDA(cudaGetLastError());
-    int host = 1;
-    BDG_CUDA(cudaMemcpyAsync(&host, bad, sizeof(int), cudaMemcpyDeviceToHost, sys->stream));
-    BDG_CUDA(cudaStreamSynchronize(sys->stream));
-    e.pair_usable = host == 0;
-    e.pair_M = M;
-    if (e.pair_usable) {
-        BDG_TRY(dev_alloc(sys, e.dcode, (size_t)e.n_sites * kDirs * sizeof(int32_t)));
-        pair_codes<<<(unsigned)ceil_div(e.n_sites, 256), 256, 0, sys->stream>>>((int)e.n_sites, e.width, Lx, M, e.idx.as<int32_t>(),
-                                                                              e.code.as<int32_t>(), e.dcode.as<int32_t>(), bad);
-        BDG_CUDA(cudaGetLastError());
-        // (`bad` is 0 here.)  Open plane ends let the rim patches own their rim site; the flag stays valid under incremental
-        // updates, which cannot add a block (a changed zero pattern rebuilds everything).
-        BDG_CUDA(cudaMemcpyAsync(&host, bad, sizeof(int), cudaMemcpyDeviceToHost, sys->stream));
-        BDG_CUDA(cudaStreamSynchronize(sys->stream));
-        e.pair_open = host == 0;
-    }
-    return BDG_OK;
-}
 
 // The two-step kernel of the current recursion (Pair or EvenPlane) with its patch size, segment length and grid.
 int pair_configure(bdg_system *sys, const PlanSwitches &sw) {

@@ -144,6 +144,34 @@ def test_patched_copies_equal_a_rebuild(gpu_api, tag):
     assert after["patched_scatters"] == before["patched_scatters"] and after["native_builds"] == before["native_builds"] + 1, after
 
 
+def test_patch_past_the_cube_kernels_dictionary_limit(gpu_api):
+    """The even-vector kernel for three-dimensional lattices holds at most 64 distinct blocks.  A patch that adds more
+    keeps the copies, takes that kernel out of the plan, and the other kernels carry on with the patched dictionary."""
+    import bodge_b200 as b
+    from bodge_b200 import workloads
+
+    shape = (6, 5, 4)
+    lattice = b.CubicLattice(shape)
+    blocks = [workloads.swave_3d(shape)]
+    system = _fresh(gpu_api, shape, blocks)
+    system.chebyshev_moments(16, vectors=2000, seed=1)
+    assert system._sys.cheb_format()["kernel"] == "t2"
+    base = system._sys.stats()
+
+    sites = list(lattice.sites())[:70]  # 70 new on-site blocks, less than a quarter of all blocks: the patch path
+    blocks.append(_onsite(sites, lattice, [(2.0 + 0.01 * k) * b.σ0 - 0.3 * b.σ3 for k in range(len(sites))]))
+    system.fill(*blocks[-1])
+    st = system._sys.stats()
+    assert st["patched_scatters"] == base["patched_scatters"] + 1, st
+    assert st["native_builds"] == base["native_builds"] and st["compactions"] == base["compactions"], st
+    with pytest.raises(ValueError):
+        system._sys.cheb_begin(n_random=8, seed=1, scale=10.0, kernel="t2")
+    system.chebyshev_moments(16, vectors=2000, seed=1)
+    assert system._sys.cheb_format()["kernel"] == "dict_diag" and system._sys.cheb_format()["distinct_blocks"] > 64
+    _check(system, blocks, shape, ("auto", "dict_diag", "dict", "ell"))
+    assert system._sys.stats()["native_builds"] == base["native_builds"]
+
+
 def test_dict_api_sweep_stays_incremental(gpu_api):
     """The reference's idiom verbatim: a loop that re-enters `with` for some on-site terms and asks for the free energy
     (tests/test_physics.py:175-228).  One build, then patches only; values equal those of freshly built systems."""
