@@ -619,7 +619,9 @@ int ell_patch(bdg_system *sys, int64_t n, const int32_t *klist, bool *ok) {
     a.dtab = e.dtab.as<double>();
     a.table_cap = (int)e.table_cap;
     a.diag_required = e.diag_usable ? 1 : 0;
-    a.self_diag_required = e.self_diag_usable && !e.diag_usable ? 1 : 0;  // (only the SD kernel relies on it)
+    // The single-step SD kernel (ell_configure) is picked whenever self_diag_usable holds, real-diagonal hopping or not: a
+    // forced "dict" runs it on a matrix that also qualifies for "dict_diag".
+    a.self_diag_required = e.self_diag_usable ? 1 : 0;
     a.dcode = e.pair_usable ? e.dcode.as<int32_t>() : nullptr;
     a.Lx = sys->cubic[0];
     a.M = e.pair_M;

@@ -23,9 +23,6 @@ from util import rel_err
 
 pytestmark = pytest.mark.gpu
 SEED = 11
-PLAN_VARS = ("BDG_ELL_WALK", "BDG_ELL_PZ", "BDG_ELL_SEG", "BDG_ELL_PREFETCH", "BDG_ELL_SD", "BDG_PAIR_SELF", "BDG_PAIR_BALANCE",
-             "BDG_PAIR_OPEN", "BDG_PAIR_P", "BDG_PAIR_SEG", "BDG_CUBE_SHAPE", "BDG_CUBE_BALANCE", "BDG_CUBE_SEG", "BDG_AUTO_PAIR",
-             "BDG_AUTO_CUBE")
 
 
 @pytest.fixture(scope="module")
@@ -43,16 +40,9 @@ def systems(gpu_api):
     return get
 
 
-def set_env(monkeypatch, env):
-    for name in PLAN_VARS:
-        monkeypatch.delenv(name, raising=False)
-    for name, value in env:
-        monkeypatch.setenv(name, str(value))
-
-
 def run(system, scale, monkeypatch, case, env=None, kernel=None, steps=None):
     """One forced recursion: (launched short names, T_n index n, T_n, T_{n-1} or None, moments, summed moments)."""
-    set_env(monkeypatch, case.env if env is None else env)
+    vc.set_env(monkeypatch, case.env if env is None else env)
     sysn = system._sys
     kernel = kernel or case.kernel
     sysn.cheb_begin(n_random=case.n_cols, seed=SEED, scale=scale, kernel=kernel)
@@ -168,7 +158,7 @@ def test_plan_switches_hold_for_the_recursion(systems, monkeypatch):
     case = vc.CASES["dict-square-gen-c13"]
     system, _, _, scale = systems(case.geometry, case.model)
     want = run(system, scale, monkeypatch, case)
-    set_env(monkeypatch, case.env)
+    vc.set_env(monkeypatch, case.env)
     sysn = system._sys
     sysn.cheb_begin(n_random=case.n_cols, seed=SEED, scale=scale, kernel=case.kernel)
     monkeypatch.setenv("BDG_ELL_SD", "0")
@@ -203,7 +193,7 @@ def test_local_accumulator_against_extended_precision(systems, monkeypatch, kern
     cols = np.concatenate([rng.integers(0, n_cols, 40), [n_cols - 1, n_cols - 1]])
     sites = np.concatenate([rng.integers(0, n_sites, 40), [n_sites - 1, n_sites - 1]])
     cols, sites = np.append(cols, cols[0]), np.append(sites, sites[0])
-    set_env(monkeypatch, env)
+    vc.set_env(monkeypatch, env)
     sysn = system._sys
     sysn.cheb_begin(n_random=n_cols, seed=SEED, scale=scale, kernel=kernel)
     sysn.cheb_local_begin(coef, cols, sites)
@@ -238,5 +228,5 @@ def test_order_parameter_on_a_balanced_plan(gpu_api, monkeypatch):
     lat = system.lattice
     sites = [(x, y, 0) for x in range(12) for y in range(20)]
     want = np.array([-1.5 * rho[4 * lat[s], 4 * lat[s] + 3] for s in sites])
-    set_env(monkeypatch, (("BDG_PAIR_BALANCE", 1),))
+    vc.set_env(monkeypatch, (("BDG_PAIR_BALANCE", 1),))
     assert np.max(np.abs(system.order_parameter(0.1, 1.5, sites) - want)) <= 1e-10

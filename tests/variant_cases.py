@@ -97,7 +97,8 @@ def _pool(api, rng, n=3):
 def fill(api, system, pairs, model, seed=7):
     """``model``: "diag" = README s-wave (on-site pairing, hopping -σ0: real-diagonal off-site blocks);
     "gen" = normal state with complex hopping from a pool of three 2x2 matrices and real-diagonal on-site blocks
-    (dictionary with general off-site blocks, SD-eligible); "pairgen" = "gen" plus on-site pairing (not SD-eligible)."""
+    (dictionary with general off-site blocks, SD-eligible); "pairgen" = "gen" plus on-site pairing (not SD-eligible);
+    "normal" = normal metal, hopping -σ0 and no pairing (real-diagonal off-site and on-site blocks: DIAG- and SD-eligible)."""
     rng = np.random.default_rng(seed)
     pool = _pool(api, rng)
     lattice = system.lattice
@@ -110,7 +111,7 @@ def fill(api, system, pairs, model, seed=7):
         for i, j in pairs:
             if (i, j) in done or i == j:
                 continue
-            h = -1.0 * api.σ0 if model == "diag" else pool[int(rng.integers(len(pool)))]
+            h = -1.0 * api.σ0 if model in ("diag", "normal") else pool[int(rng.integers(len(pool)))]
             H[i, j] = h
             H[j, i] = h.conj().T
             done.update(((i, j), (j, i)))
@@ -171,15 +172,33 @@ GEOMETRIES = {
 WIDTH = {"chain": 3, "ladder": 4, "square": 5, "slab": 6, "cube": 7, "hub8": 8}
 
 
-def build(api, geometry, model):
+def lattice_pairs(api, geometry):
+    """The geometry's lattice and the (i, j) coordinate pairs its hopping is set on."""
     kind, arg = GEOMETRIES[geometry]()
     if kind == "hub":
         lattice = hub_lattice(*arg)
-        pairs = list(lattice.bonds())
-    else:
-        lattice = api.CubicLattice(arg)
-        pairs = periodic_pairs(lattice) if kind == "torus" else list(lattice.bonds())
+        return lattice, list(lattice.bonds())
+    lattice = api.CubicLattice(arg)
+    return lattice, periodic_pairs(lattice) if kind == "torus" else list(lattice.bonds())
+
+
+def build(api, geometry, model):
+    lattice, pairs = lattice_pairs(api, geometry)
     return fill(api, api.Hamiltonian(lattice), pairs, model)
+
+
+# ---- planner switches ---------------------------------------------------------------------------------------------
+PLAN_VARS = ("BDG_ELL_WALK", "BDG_ELL_PZ", "BDG_ELL_SEG", "BDG_ELL_PREFETCH", "BDG_ELL_SD", "BDG_PAIR_SELF", "BDG_PAIR_BALANCE",
+             "BDG_PAIR_OPEN", "BDG_PAIR_P", "BDG_PAIR_SEG", "BDG_CUBE_SHAPE", "BDG_CUBE_BALANCE", "BDG_CUBE_SEG", "BDG_AUTO_PAIR",
+             "BDG_AUTO_CUBE")
+
+
+def set_env(monkeypatch, env):
+    """Clear every planner switch, then set ``env`` (``((name, value), ...)``)."""
+    for name in PLAN_VARS:
+        monkeypatch.delenv(name, raising=False)
+    for name, value in env:
+        monkeypatch.setenv(name, str(value))
 
 
 # ---- cases --------------------------------------------------------------------------------------------------------
