@@ -167,10 +167,6 @@ static int create_common(int device, bdg_system **out) {
     return BDG_OK;
 }
 
-#define BDG_ENTER(sys)                                                 \
-    BDG_REQUIRE((sys) != nullptr, "null handle");                      \
-    BDG_CUDA(cudaSetDevice((sys)->device))
-
 extern "C" int bdg_abi_version(void) { return BDG_ABI_VERSION; }
 extern "C" const char *bdg_last_error(void) { return g_error; }
 

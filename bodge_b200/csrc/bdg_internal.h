@@ -37,6 +37,11 @@ void bdg_set_error(const char *fmt, ...);
         }                                                                                   \
     } while (0)
 
+// First statement of every ABI function that takes a handle.
+#define BDG_ENTER(sys)                                                                      \
+    BDG_REQUIRE((sys) != nullptr, "null handle");                                           \
+    BDG_CUDA(cudaSetDevice((sys)->device))
+
 // ---- device buffers -----------------------------------------------------------------------
 // Thin owner of one cudaMalloc'd array; tracks bytes per handle.
 struct DevBuf {
@@ -107,19 +112,9 @@ struct CubeWalk {
 };
 
 // ---- Chebyshev state ----------------------------------------------------------------------
-// Plan switches (INTEGRATION.md): member x_y holds BDG_X_Y.  bdg_cheb_begin reads them once (read_plan_switches, which
-// holds the defaults) and the configure functions plan from this copy, so they hold for the whole recursion.  Extents and
-// segment lengths: <= 0 = the planner's; pair_self, cube_shape and the balances: < 0 = the planner's.
-struct PlanSwitches {
-    bool auto_pair, auto_cube;
-    bool ell_sd, ell_walk;
-    int ell_pz, ell_seg, ell_prefetch;
-    int pair_self, pair_p, pair_seg, pair_balance;
-    bool pair_open;
-    int cube_shape, cube_seg, cube_balance;
-};
+struct PlanSwitches;  // cheb_plan.h
 
-// How the recursion advances; ChebState::kernel keeps the matrix format of the single-step kernel.
+// How the recursion advances (plan_stepping, cheb_plan.h); ChebState::kernel keeps the matrix format of the single-step kernel.
 enum class Stepping {
     Single,     // one step per launch (cheb.cu, cheb_ell.cu)
     Pair,       // two steps per launch whenever two or more remain (cheb_pair.cu); T_1 and odd leftovers: single-step kernel

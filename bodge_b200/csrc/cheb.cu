@@ -22,20 +22,13 @@
 // because it removes the FP64 issue/broadcast overhead a scalar formulation has (SURVEY H3), not
 // to chase flops.  cheb_step_fma is the scalar-FMA formulation of the same step (A/B reference).
 #include <algorithm>
-#include <cstdlib>
 #include <cstring>
-#include <utility>
 
 #include "bdg_internal.h"
 #include "cheb_device.cuh"
+#include "cheb_plan.h"
 
 namespace {
-
-// AUTO runs two steps per pass wherever the DFMA variant of the pair kernel applies: 1.33x the single-step
-// dictionary kernel at C5 (profiles/r01/s4_pair_v2.log).  The DMMA variant (complex hopping / pairing on the
-// bonds, C3) is FP64-pipe-bound and slower than its single-step kernel, so it stays opt-in.
-constexpr bool kAutoPairDefault = true;
-
 
 // ---- the fused step: FP64 warp-MMA formulation --------------------------------------------------
 // CH = neighbour blocks handled per round; the host picks the smallest instantiated CH that
@@ -348,32 +341,6 @@ StepKernel pick_kernel(int kernel, int pw, bool first, int max_row) {
     }
 }
 
-// Every plan switch (PlanSwitches), read once per recursion.
-PlanSwitches read_plan_switches() {
-    // BDG_ELL_PZ, BDG_PAIR_P: a set value counts as at least 1; unset or empty: 0
-    const auto extent = [](const char *name) {
-        const char *v = getenv(name);
-        return v && *v ? std::max(1, atoi(v)) : 0;
-    };
-    PlanSwitches s;
-    s.auto_pair = env_int("BDG_AUTO_PAIR", kAutoPairDefault) != 0;
-    s.auto_cube = env_int("BDG_AUTO_CUBE", 1) != 0;
-    s.ell_sd = env_int("BDG_ELL_SD", 1) != 0;
-    s.ell_walk = env_int("BDG_ELL_WALK", 1) != 0;
-    s.ell_pz = extent("BDG_ELL_PZ");
-    s.ell_seg = env_int("BDG_ELL_SEG", 0);
-    s.ell_prefetch = env_int("BDG_ELL_PREFETCH", 1);
-    s.pair_self = env_int("BDG_PAIR_SELF", -1);
-    s.pair_open = env_int("BDG_PAIR_OPEN", 1) != 0;
-    s.pair_p = extent("BDG_PAIR_P");
-    s.pair_seg = env_int("BDG_PAIR_SEG", 0);
-    s.pair_balance = env_int("BDG_PAIR_BALANCE", -1);
-    s.cube_shape = env_int("BDG_CUBE_SHAPE", -1);
-    s.cube_seg = env_int("BDG_CUBE_SEG", 0);
-    s.cube_balance = env_int("BDG_CUBE_BALANCE", -1);
-    return s;
-}
-
 bool ell_format(int kernel) { return kernel == BDG_KERNEL_ELL || kernel == BDG_KERNEL_DICT || kernel == BDG_KERNEL_DICT_DIAG; }
 
 // DMMA / FMA: the FIRST and the next-step kernel on one grid -- enough CTAs to fill every SM at the kernel's occupancy, split
@@ -395,45 +362,17 @@ int bsr_configure(bdg_system *sys) {
     return BDG_OK;
 }
 
-int launch_step(bdg_system *sys, bool first) {
+int bsr_launch(bdg_system *sys, bool first, const void *x_cur, void *x_io, double *dots_step) {
     ChebState &st = sys->cheb;
     const BsrDev &m = sys->packed;
-    const int slot = first ? 0 : st.steps_done + 1;
-    const int stride = st.n_panels * st.panel_width;
-    double *dots_step = st.dots.as<double>() + (size_t)slot * 2 * stride;
-    const double2 *x_cur = st.vec[st.cur].as<double2>();
-    double2 *x_io = st.vec[st.prev].as<double2>();
-    if (ell_format(st.kernel)) {
-        BDG_TRY(ell_launch_step(sys, first, x_cur, x_io, dots_step));
-    } else {
-        const Launch<StepKernel> &l = first ? st.bsr_first : st.bsr_next;
-        note_launch(st, reinterpret_cast<const void *>(l.fn));
-        l.fn<<<l.grid, l.threads, l.smem, sys->stream>>>(m.indptr.as<int32_t>(), m.indices.as<int32_t>(), m.data.as<double2>(), x_cur,
-                                                         x_io, (int)m.n_sites, (first ? 1.0 : 2.0) / st.scale,
-                                                         first ? 0.0 : 1.0, st.partials.as<double>(), st.tickets.as<unsigned>(),
-                                                         dots_step, st.n_panels);
-        BDG_CUDA(cudaGetLastError());
-    }
-    std::swap(st.cur, st.prev);
-    st.launches += 1;
-    return local_accumulate(sys, slot + 1, x_io, nullptr);  // x_io now holds T_{slot+1}
-}
-
-// Two steps in one launch (cheb_pair.cu): T_{n+1}, T_{n+2} go to the two buffers holding neither
-// T_n nor T_{n-1}; dot products of steps n and n+1.
-int launch_pair(bdg_system *sys) {
-    ChebState &st = sys->cheb;
-    const int slot = st.steps_done + 1;
-    const int stride = st.n_panels * st.panel_width;
-    int out[2], n_out = 0;
-    for (int b = 0; b < 4; ++b)
-        if (b != st.cur && b != st.prev) out[n_out++] = b;
-    BDG_TRY(pair_launch(sys, st.vec[st.prev].ptr, st.vec[st.cur].ptr, st.vec[out[0]].ptr, st.vec[out[1]].ptr,
-                        st.dots.as<double>() + (size_t)slot * 2 * stride));
-    st.prev = out[0];
-    st.cur = out[1];
-    st.launches += 1;
-    return local_accumulate(sys, slot + 1, st.vec[out[0]].ptr, st.vec[out[1]].ptr);  // T_{slot+1}, T_{slot+2}
+    const Launch<StepKernel> &l = first ? st.bsr_first : st.bsr_next;
+    note_launch(st, reinterpret_cast<const void *>(l.fn));
+    l.fn<<<l.grid, l.threads, l.smem, sys->stream>>>(m.indptr.as<int32_t>(), m.indices.as<int32_t>(), m.data.as<double2>(),
+                                                     static_cast<const double2 *>(x_cur), static_cast<double2 *>(x_io),
+                                                     (int)m.n_sites, (first ? 1.0 : 2.0) / st.scale, first ? 0.0 : 1.0,
+                                                     st.partials.as<double>(), st.tickets.as<unsigned>(), dots_step, st.n_panels);
+    BDG_CUDA(cudaGetLastError());
+    return BDG_OK;
 }
 
 int ensure_dot_capacity(bdg_system *sys, int steps_total) {
@@ -451,6 +390,48 @@ int ensure_dot_capacity(bdg_system *sys, int steps_total) {
     dev_free(sys, st.dots);
     st.dots = grown;
     st.dot_capacity = cap;
+    return BDG_OK;
+}
+
+// One launch of the plan.  `first`: the launch of bdg_cheb_begin, T_1 = H~ T_0 (E_1 = T_2(H~) E_0 on the even-vector
+// steppings); `remaining`: the steps still asked for, of which Pair takes two per launch while two remain (T_1 and an odd
+// leftover run on its single-step kernel).  Even steppings always take two: an odd request is rounded up.
+int advance(bdg_system *sys, bool first, int remaining) {
+    ChebState &st = sys->cheb;
+    const bool pair = st.stepping == Stepping::Pair && !first && remaining >= 2;
+    if (st.even()) BDG_TRY(ensure_dot_capacity(sys, st.steps_done + 2));
+    // the dot rows of step `slot` (and slot + 1 on a two-step launch): step n = steps_done + 1 when T_n is current, 0 first
+    const int slot = first ? 0 : st.steps_done + 1;
+    double *dots_step = st.dots.as<double>() + (size_t)slot * 2 * st.n_panels * st.panel_width;
+    const void *x_cur = st.vec[st.cur].ptr;
+    void *x_io = st.vec[st.prev].ptr;
+    // (prev, cur) after the launch: T_{n+1} (E_{j+1}) is written over T_{n-1} (E_{j-1}); the pair kernel writes T_{n+1}, T_{n+2}
+    // into the two buffers holding neither T_n nor T_{n-1}.
+    int next[2] = {st.cur, st.prev};
+    if (pair)
+        for (int b = 0, k = 0; b < 4; ++b)
+            if (b != st.cur && b != st.prev) next[k++] = b;
+    switch (st.stepping) {
+        case Stepping::EvenPlane: BDG_TRY(t2_launch(sys, first, x_cur, x_io, dots_step)); break;
+        case Stepping::EvenCube: BDG_TRY(cube_launch(sys, first, x_cur, x_io, dots_step)); break;
+        case Stepping::Pair:
+            if (pair) {
+                BDG_TRY(pair_launch(sys, x_io, x_cur, st.vec[next[0]].ptr, st.vec[next[1]].ptr, dots_step));
+                break;
+            }
+            [[fallthrough]];
+        case Stepping::Single:
+            BDG_TRY(ell_format(st.kernel) ? ell_launch_step(sys, first, x_cur, x_io, dots_step)
+                                          : bsr_launch(sys, first, x_cur, x_io, dots_step));
+            break;
+    }
+    st.prev = next[0];
+    st.cur = next[1];
+    st.launches += 1;
+    // the new vectors, T_{slot+1} (and T_{slot+2}), into the local accumulator; the even-vector recursion keeps every second
+    // vector only and takes none (bdg_cheb_local_begin)
+    if (!st.even()) BDG_TRY(local_accumulate(sys, slot + 1, st.vec[next[pair ? 0 : 1]].ptr, pair ? st.vec[next[1]].ptr : nullptr));
+    st.steps_done += (pair || st.even() ? 2 : 1) - (first ? 1 : 0);
     return BDG_OK;
 }
 
@@ -494,10 +475,6 @@ void cheb_release(bdg_system *sys) {
     st.launches = launches;
 }
 
-#define BDG_ENTER(sys)                                                 \
-    BDG_REQUIRE((sys) != nullptr, "null handle");                      \
-    BDG_CUDA(cudaSetDevice((sys)->device))
-
 extern "C" int bdg_cheb_begin(bdg_t *sys, int kind, int32_t n_cols, const int64_t *probe_rows, uint64_t seed,
                               int64_t col_offset, double scale, int kernel) {
     BDG_ENTER(sys);
@@ -509,57 +486,15 @@ extern "C" int bdg_cheb_begin(bdg_t *sys, int kind, int32_t n_cols, const int64_
                 "unknown kernel %d", kernel);
     BDG_TRY(build_packed(sys));
     const PlanSwitches sw = read_plan_switches();
-    Stepping stepping = Stepping::Single;
-    if (kernel == BDG_KERNEL_AUTO || kernel == BDG_KERNEL_ELL || kernel == BDG_KERNEL_DICT || kernel == BDG_KERNEL_DICT_DIAG ||
-        kernel == BDG_KERNEL_PAIR || kernel == BDG_KERNEL_T2 || kernel == BDG_KERNEL_AUTO_MOMENTS) {
+    PlanFacts facts{};
+    if (kernel != BDG_KERNEL_DMMA && kernel != BDG_KERNEL_FMA) {  // every other kernel reads the copies of formats.cu
         BDG_TRY(ell_build(sys));
-        // The pair kernel works on 8-column panels of the dictionary format; single leftover steps
-        // (and T_1) run on the single-step dictionary kernel of the same format.
-        // The two-step kernels work on 8-column panels.  Fewer than 5 columns (ldos() of one site = 4) are padded to
-        // a panel when the vectors are small enough to live in L2 (<= 64 Ki sites: 32 MB per vector): such runs are
-        // launch-latency-bound, and two steps per launch halve the launches; at HBM-bound sizes the padding would
-        // cost more bytes than the fusion saves, so narrow panels stay on the single-step kernels there.
-        const bool small = sys->ell.n_sites <= (1 << 16);
-        const bool pair_ok = sys->ell.pair_usable && (n_cols >= 5 || small);
-        // Three-dimensional lattices: the even-vector recursion on 4-column panels (cheb_cube.cu): open stencil,
-        // real-diagonal hopping blocks, few distinct blocks (its fragments are held in registers): EllDev::cube_usable.
-        const bool cube_ok = sys->ell.cube_usable && (n_cols >= 3 || small);
-        BDG_REQUIRE(kernel != BDG_KERNEL_PAIR || pair_ok,
-                    "the two-steps-per-pass kernel needs >= 5 columns (any number on lattices of <= 65536 sites) and a block "
-                    "dictionary on a lattice with one-dimensional x-planes and a nearest-neighbour stencil");
-        BDG_REQUIRE(kernel != BDG_KERNEL_T2 || pair_ok || cube_ok,
-                    "the even-vector recursion needs a block dictionary on a lattice with a nearest-neighbour stencil: one-dimensional "
-                    "x-planes and >= 5 columns, or a three-dimensional open lattice with real-diagonal hopping blocks, <= 64 "
-                    "distinct blocks and >= 3 columns (any number of columns on lattices of <= 65536 sites)");
-        // The two-step kernels pay on every dictionary matrix they take (round 2, profiles/r02/41_* .. 43_*): rows of real-
-        // diagonal hopping blocks (DFMA), general hopping blocks next to real-diagonal on-site blocks (SD: d-wave / Rashba
-        // models, +12..44 % over the single-step kernel) and rows of ten MMAs (+22..42 % at 8 columns, +24..32 % at >= 64
-        // columns on 10^6 sites, level at C3 with 64..512 columns).
-        const bool prefer = pair_ok && sw.auto_pair;
-        // Callers that only read moments / observables get the even-vector recursion (three vector passes per
-        // two steps); callers that step and look at T_n, T_{n-1} the pair kernel (four).
-        // ... preferred where its items fill the machine without cutting x into segments (one CTA per SM marches an 8 x 8 patch:
-        // C4 = 64 patches x 2 panels); on smaller lattices the single-step kernel's finer grid wins.
-        const int64_t cube_items = ceil_div(sys->cubic[1], 8) * ceil_div(sys->cubic[2], 8) * ceil_div(n_cols, 4);
-        const bool prefer_cube = cube_ok && sw.auto_cube && 4 * cube_items >= 3 * (int64_t)sys->sm_count;
-        // (the even-vector recursion without pair_ok has cube_ok: the requirement above, or prefer_cube)
-        if (kernel == BDG_KERNEL_T2 || (kernel == BDG_KERNEL_AUTO_MOMENTS && (prefer || prefer_cube)))
-            stepping = pair_ok ? Stepping::EvenPlane : Stepping::EvenCube;
-        else if (kernel == BDG_KERNEL_PAIR || (kernel == BDG_KERNEL_AUTO && prefer))
-            stepping = Stepping::Pair;
-        if (kernel == BDG_KERNEL_PAIR || kernel == BDG_KERNEL_T2 || kernel == BDG_KERNEL_AUTO_MOMENTS) kernel = BDG_KERNEL_AUTO;
-        BDG_REQUIRE(kernel != BDG_KERNEL_ELL || sys->ell.usable,
-                    "the fixed-width (ELL) kernel needs block rows of <= 8 blocks with little padding");
-        BDG_REQUIRE(kernel != BDG_KERNEL_DICT || sys->ell.dict_usable,
-                    "the block-dictionary kernel needs a fixed-width matrix whose distinct blocks are few");
-        BDG_REQUIRE(kernel != BDG_KERNEL_DICT_DIAG || sys->ell.diag_usable,
-                    "the diagonal-hopping kernel needs a block dictionary whose off-site blocks are real and diagonal");
-        if (kernel == BDG_KERNEL_AUTO)
-            kernel = sys->ell.diag_usable   ? BDG_KERNEL_DICT_DIAG
-                     : sys->ell.dict_usable ? BDG_KERNEL_DICT
-                     : sys->ell.usable      ? BDG_KERNEL_ELL
-                                            : BDG_KERNEL_DMMA;
+        const EllDev &e = sys->ell;
+        facts = {e.usable, e.dict_usable, e.diag_usable, e.pair_usable, e.cube_usable, e.n_sites, sys->cubic[1], sys->cubic[2],
+                 sys->sm_count};
     }
+    const SteppingPlan plan = plan_stepping(kernel, n_cols, facts, sw);
+    BDG_REQUIRE(!plan.refusal, "%s", plan.refusal);
     const BsrDev &m = sys->packed;
     const int n = (int)m.n_sites;
     if (kind == BDG_X0_PROBE)
@@ -569,11 +504,11 @@ extern "C" int bdg_cheb_begin(bdg_t *sys, int kind, int32_t n_cols, const int64_
     // Buffers of a previous recursion are kept and reused when large enough (parameter sweeps).
     ChebState &st = sys->cheb;
     st.active = false;
-    st.kernel = kernel;
+    st.kernel = plan.format;
     st.n_cols = n_cols;
-    st.stepping = stepping;
-    st.panel_width = stepping == Stepping::EvenCube ? 4 : (n_cols >= 5 || stepping != Stepping::Single) ? 8 : (n_cols >= 3 ? 4 : n_cols);
-    st.n_panels = (int)ceil_div(n_cols, st.panel_width);
+    st.stepping = plan.stepping;
+    st.panel_width = plan.panel_width;
+    st.n_panels = plan.n_panels;
     st.scale = scale;
     st.steps_done = 0;
     st.cur = 0;
@@ -587,15 +522,15 @@ extern "C" int bdg_cheb_begin(bdg_t *sys, int kind, int32_t n_cols, const int64_
     // The kernels the recursion will launch: the single-step kernel (every step, or T_1 and odd leftovers of the pair
     // plan), the two-step kernel, or the even-vector one.
     st.partial_runs = 0;
-    if (stepping == Stepping::Single || stepping == Stepping::Pair)
+    if (st.stepping == Stepping::Single || st.stepping == Stepping::Pair)
         BDG_TRY(ell_format(st.kernel) ? ell_configure(sys, sw) : bsr_configure(sys));
-    if (stepping == Stepping::Pair || stepping == Stepping::EvenPlane) BDG_TRY(pair_configure(sys, sw));
-    if (stepping == Stepping::EvenCube) BDG_TRY(cube_configure(sys, sw));
+    if (st.stepping == Stepping::Pair || st.stepping == Stepping::EvenPlane) BDG_TRY(pair_configure(sys, sw));
+    if (st.stepping == Stepping::EvenCube) BDG_TRY(cube_configure(sys, sw));
 
     const size_t vec_elems = (size_t)st.n_panels * n * st.panel_width * 4;
-    for (int b = 0; b < (stepping == Stepping::Pair ? 4 : 2); ++b) BDG_TRY(dev_alloc(sys, st.vec[b], vec_elems * sizeof(double2)));
+    for (int b = 0; b < (st.stepping == Stepping::Pair ? 4 : 2); ++b) BDG_TRY(dev_alloc(sys, st.vec[b], vec_elems * sizeof(double2)));
     BDG_TRY(dev_alloc(sys, st.partials,
-                      (size_t)st.n_panels * st.partial_runs * (stepping == Stepping::Single ? 16 : 32) * sizeof(double)));
+                      (size_t)st.n_panels * st.partial_runs * (st.stepping == Stepping::Single ? 16 : 32) * sizeof(double)));
     BDG_TRY(dev_alloc(sys, st.tickets, (size_t)st.n_panels * sizeof(unsigned)));
     BDG_CUDA(cudaMemsetAsync(st.tickets.ptr, 0, (size_t)st.n_panels * sizeof(unsigned), sys->stream));
     BDG_TRY(ensure_dot_capacity(sys, 1024));
@@ -615,19 +550,9 @@ extern "C" int bdg_cheb_begin(bdg_t *sys, int kind, int32_t n_cols, const int64_
     }
     BDG_CUDA(cudaGetLastError());
     st.launches += 1;
-    if (st.even()) {
-        // E_1 = T_2(H~) E_0 into vec[1] and the dot products of steps 0 and 1 (moments 0..3): one step done.
-        BDG_TRY(ensure_dot_capacity(sys, 2));
-        BDG_TRY(t2_launch(sys, true, st.vec[0].ptr, st.vec[1].ptr, st.dots.as<double>()));
-        st.cur = 1;
-        st.prev = 0;
-        st.steps_done = 1;
-        st.launches += 1;
-        return BDG_OK;
-    }
-    // T_1 = H~ T_0 (written into vec[1]); afterwards cur = 1 holds T_1, vec[0] holds T_0.
-    BDG_TRY(launch_step(sys, true));
-    return BDG_OK;
+    // T_1 = H~ T_0 into vec[1] (cur = 1, vec[0] keeps T_0); the even-vector recursion: E_1 = T_2(H~) E_0 and the dot
+    // products of steps 0 and 1 (moments 0..3), one step done.
+    return advance(sys, true, 0);
 }
 
 extern "C" int bdg_cheb_steps(bdg_t *sys, int32_t n_steps, float *elapsed_ms) {
@@ -651,26 +576,7 @@ extern "C" int bdg_cheb_steps(bdg_t *sys, int32_t n_steps, float *elapsed_ms) {
         BDG_CUDA(cudaStreamSynchronize(sys->stream));
         BDG_CUDA(cudaEventRecord(e0, sys->stream));
     }
-    for (int s = 0; s < n_steps;) {
-        if (st.even()) {  // two steps per launch, always: an odd request is rounded up (moments-only mode)
-            const int stride = st.n_panels * st.panel_width;
-            BDG_TRY(ensure_dot_capacity(sys, st.steps_done + 2));
-            BDG_TRY(t2_launch(sys, false, st.vec[st.cur].ptr, st.vec[st.prev].ptr,
-                              st.dots.as<double>() + (size_t)(st.steps_done + 1) * 2 * stride));
-            std::swap(st.cur, st.prev);
-            st.launches += 1;
-            st.steps_done += 2;
-            s += 2;
-        } else if (st.stepping == Stepping::Pair && n_steps - s >= 2) {
-            BDG_TRY(launch_pair(sys));
-            st.steps_done += 2;
-            s += 2;
-        } else {
-            BDG_TRY(launch_step(sys, false));
-            st.steps_done += 1;
-            s += 1;
-        }
-    }
+    for (const int target = st.steps_done + n_steps; st.steps_done < target;) BDG_TRY(advance(sys, false, target - st.steps_done));
     if (elapsed_ms) {
         BDG_CUDA(cudaEventRecord(e1, sys->stream));
         BDG_CUDA(cudaEventSynchronize(e1));

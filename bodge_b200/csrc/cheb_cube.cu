@@ -42,6 +42,7 @@
 
 #include "bdg_internal.h"
 #include "cheb_device.cuh"
+#include "cheb_plan.h"
 #include "cheb_smem.cuh"
 #include "work_lists.h"
 

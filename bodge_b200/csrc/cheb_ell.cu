@@ -26,6 +26,7 @@
 
 #include "bdg_internal.h"
 #include "cheb_device.cuh"
+#include "cheb_plan.h"
 
 namespace {
 

@@ -46,6 +46,7 @@
 
 #include "bdg_internal.h"
 #include "cheb_device.cuh"
+#include "cheb_plan.h"
 #include "cheb_smem.cuh"
 #include "work_lists.h"
 
@@ -568,10 +569,9 @@ int pair_launch(bdg_system *sys, const void *x_prev, const void *x_cur, void *x_
     return BDG_OK;
 }
 
-// T2 mode: E_{j+1} = 2 T_2(H~) E_j - E_{j-1} written over E_{j-1} (x_io); first: E_1 = T_2(H~) E_0.
+// EvenPlane: E_{j+1} = 2 T_2(H~) E_j - E_{j-1} written over E_{j-1} (x_io); first: E_1 = T_2(H~) E_0.
 int t2_launch(bdg_system *sys, bool first, const void *x_cur, void *x_io, double *dots_step) {
     ChebState &st = sys->cheb;
-    if (st.stepping == Stepping::EvenCube) return cube_launch(sys, first, x_cur, x_io, dots_step);
     const EllDev &e = sys->ell;
     const Launch<PairKernel> &l = st.two_step;
     note_launch(st, reinterpret_cast<const void *>(l.fn));

@@ -86,10 +86,6 @@ __global__ void sum_columns(const double *__restrict__ in, int n, double *__rest
 
 }  // namespace
 
-#define BDG_ENTER(sys)                            \
-    BDG_REQUIRE((sys) != nullptr, "null handle"); \
-    BDG_CUDA(cudaSetDevice((sys)->device))
-
 static int check_active(bdg_system *sys, int32_t n_moments) {
     const ChebState &st = sys->cheb;
     BDG_REQUIRE(st.active, "bdg_cheb_begin has not been called");
