@@ -6,7 +6,11 @@ windows of >= 1 s); the time per ``order_parameter`` call at C1 (40 x 40, 1600 c
 alternative at C1, ``torch.linalg.eigh`` of the 6400 x 6400 matrix on the same GPU; and the largest difference
 between the KPM and the dense order parameter at C1.
 
-    python bench_density.py [--temperature 0.1] [--repeats 3] [--device 0]
+``--spacing S [S ...]`` measures instead ``order_parameter`` over every site of the README model on 1000 x 1000 sites
+from distance-classed columns (``spacing=S``, one column per class): seconds per call for each spacing, and the largest
+deviation from the one-column-per-site path at 50 sampled sites.
+
+    python bench_density.py [--temperature 0.1] [--repeats 3] [--device 0] [--spacing 8 16]
 
 It writes nothing into the tree.
 """
@@ -71,11 +75,39 @@ def timed_call(fn, repeats: int) -> list[float]:
     return out
 
 
+def spacing_case(dev: int, T: float, spacings, repeats: int) -> dict:
+    """``order_parameter`` over every site of the 1000 x 1000 README model with ``spacing=s``: seconds per call (every
+    call, the first included) and the largest deviation from the exact path at 50 sampled sites."""
+    from bodge_b200 import kpm
+
+    system = readme_system(1000, dev)
+    n = system.lattice.size
+    scale = system.spectral_bound()
+    sample = np.sort(np.random.default_rng(7).choice(n, 50, replace=False))
+    coords = [tuple(int(v) for v in c) for c in system.lattice.sites_array()[sample]]
+    t0 = time.perf_counter()
+    exact = system.order_parameter(T, 1.0, sites=coords)
+    out = {"sites": n, "n_coef": kpm.free_energy_moments(T, scale)[0], "scale": scale, "sampled_sites": len(sample),
+           "exact_sampled_s": time.perf_counter() - t0, "spacing": {}}
+    for s in spacings:
+        per_call = []
+        for _ in range(repeats):
+            t0 = time.perf_counter()
+            delta = system.order_parameter(T, 1.0, spacing=s)
+            per_call.append(time.perf_counter() - t0)
+        out["spacing"][str(s)] = {"classes": int(system._classes(s).max()) + 1, "per_call_s": per_call,
+                                  "max_abs_dev_sampled": float(np.max(np.abs(delta[sample] - exact))),
+                                  "delta_range": [float(np.min(np.abs(delta))), float(np.max(np.abs(delta)))]}
+    return out
+
+
 def main() -> None:
     ap = argparse.ArgumentParser(description=__doc__.splitlines()[0])
     ap.add_argument("--temperature", type=float, default=0.1)
     ap.add_argument("--repeats", type=int, default=3)
     ap.add_argument("--device", type=int, default=0)
+    ap.add_argument("--spacing", type=int, nargs="+", default=None,
+                    help="measure order_parameter(spacing=S) on 1000 x 1000 sites for each S instead")
     args = ap.parse_args()
 
     import torch
@@ -87,6 +119,10 @@ def main() -> None:
     dev, T, reps = args.device, args.temperature, args.repeats
     result = device_info(dev)
     result.update(model="readme_swave", temperature=T, potential=1.0)
+    if args.spacing:
+        result["order_parameter_spacing"] = spacing_case(dev, T, args.spacing, reps)
+        print(json.dumps(result))
+        return
 
     # --- C2: accumulator overhead on the recursion, then order_parameter end to end ---------------------------------
     c2 = readme_system(100, dev)

@@ -17,7 +17,7 @@ _PKG = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("BDG_LIB") or os.path.join(_PKG, "libbdg.so")  # BDG_LIB: a development build of kernel variants
 
 OK, E_INVALID, E_CUDA, E_NOT_NEIGHBOUR, E_NOT_HERMITIAN, E_OUT_OF_BOUNDS, E_NO_DEVICE = range(7)
-X0_PROBE, X0_RADEMACHER = 0, 1
+X0_PROBE, X0_RADEMACHER, X0_CLASS = 0, 1, 2
 MU_PER_COLUMN, MU_SUM = 0, 1
 KERNEL_AUTO, KERNEL_DMMA, KERNEL_FMA = 0, 1, 2
 KERNELS = {"auto": KERNEL_AUTO, "dmma": KERNEL_DMMA, "fma": KERNEL_FMA, "ell": 3, "dict": 6, "dict_diag": 7, "pair": 8, "t2": 9,
@@ -51,7 +51,9 @@ SIGNATURES = {
     "bdg_export_csr": [_vp, C.c_int, _i64p, _vp, _vp, _vp],
     "bdg_export_dense": [_vp, _vp],
     "bdg_import_data": [_vp, _vp],
+    "bdg_gather_blocks": [_vp, C.c_int64, _vp, _vp],
     "bdg_norm_inf": [_vp, _f64p],
+    "bdg_set_classes": [_vp, C.c_int64, _vp, C.c_int32],
     "bdg_cheb_begin": [_vp, C.c_int, C.c_int32, _vp, C.c_uint64, C.c_int64, C.c_double, C.c_int],
     "bdg_cheb_steps": [_vp, C.c_int32, C.POINTER(C.c_float)],
     "bdg_cheb_reserve": [_vp, C.c_int32],
@@ -328,15 +330,32 @@ class System:
             raise ValueError(f"expected data of shape {(self.n_blocks, 4, 4)}, got {data.shape}")
         check(load().bdg_import_data(self._h, _ptr(data)))
 
+    def gather_blocks(self, k) -> np.ndarray:
+        """The stored blocks at skeleton positions ``k`` (``lookup``) as ``[len(k), 4, 4]`` complex128."""
+        k = _as(k, np.int64)
+        out = np.empty((len(k), 4, 4), dtype=np.complex128)
+        check(load().bdg_gather_blocks(self._h, len(k), _ptr(k), _ptr(out)))
+        return out
+
     def norm_inf(self) -> float:
         v = C.c_double()
         check(load().bdg_norm_inf(self._h, C.byref(v)))
         return v.value
 
     # -- Chebyshev engine ---------------------------------------------------------------------
-    def cheb_begin(self, *, probe_rows=None, n_random=0, seed=0, col_offset=0, scale, kernel="auto"):
+    def set_classes(self, site_class, n_classes: int):
+        """Upload the distance class of every site (``bdg_set_classes``); the handle keeps it for ``class_rows``."""
+        site_class = _as_index(site_class, "site class")
+        check(load().bdg_set_classes(self._h, len(site_class), _ptr(site_class), int(n_classes)))
+
+    def cheb_begin(self, *, probe_rows=None, class_rows=None, n_random=0, seed=0, col_offset=0, scale, kernel="auto"):
+        """``probe_rows``: unit columns ``e_r``; ``class_rows``: class columns, ``4k + β`` = the indicator of class ``k``
+        (``set_classes``) in component ``β``; else ``n_random`` Rademacher columns."""
         lib = load()
-        if probe_rows is not None:
+        if class_rows is not None:
+            rows = _as(class_rows, np.int64)
+            check(lib.bdg_cheb_begin(self._h, X0_CLASS, len(rows), _ptr(rows), 0, 0, float(scale), KERNELS[kernel]))
+        elif probe_rows is not None:
             rows = _as(probe_rows, np.int64)
             check(lib.bdg_cheb_begin(self._h, X0_PROBE, len(rows), _ptr(rows), 0, 0, float(scale), KERNELS[kernel]))
         else:

@@ -196,6 +196,7 @@ extern "C" int bdg_destroy(bdg_t *sys) {
     dev_free(sys, sys->pack_pos);
     dev_free(sys, sys->multi_send);
     dev_free(sys, sys->multi_recv);
+    dev_free(sys, sys->site_class);
     dev_free(sys, sys->scalars);
     if (sys->host_scalars) {
         std::lock_guard<std::mutex> lock(g_cache_mutex);
@@ -1133,6 +1134,44 @@ extern "C" int bdg_export_dense(bdg_t *sys, double *out) {
     if (err == cudaSuccess) err = cudaMemcpyAsync(out, dense.ptr, bytes, cudaMemcpyDeviceToHost, sys->stream);
     if (err == cudaSuccess) err = cudaStreamSynchronize(sys->stream);
     dev_free(sys, dense);
+    BDG_CUDA(err);
+    return BDG_OK;
+}
+
+// One thread per complex element of the gathered blocks.
+__global__ void __launch_bounds__(kThreads)
+gather_blocks(int64_t n, const int64_t *__restrict__ k, const double2 *__restrict__ data, double2 *__restrict__ out) {
+    const int64_t t = (int64_t)blockIdx.x * kThreads + threadIdx.x;
+    if (t >= n * 16) return;
+    out[t] = data[k[t >> 4] * 16 + (t & 15)];
+}
+
+extern "C" int bdg_gather_blocks(bdg_t *sys, int64_t n, const int64_t *k, double *out) {
+    BDG_ENTER(sys);
+    BDG_REQUIRE(n >= 0 && (n == 0 || (k && out)), "bad arguments");
+    const BsrDev &m = sys->skel;
+    for (int64_t e = 0; e < n; ++e)
+        BDG_REQUIRE(k[e] >= 0 && k[e] < m.n_blocks, "entry %lld: block position %lld outside [0, %lld)", (long long)e,
+                    (long long)k[e], (long long)m.n_blocks);
+    if (n == 0) return BDG_OK;
+    DevBuf pos, val;
+    BDG_TRY(dev_alloc(sys, pos, (size_t)n * sizeof(int64_t)));
+    int rc = dev_alloc(sys, val, (size_t)n * 16 * sizeof(double2));
+    cudaError_t err = cudaSuccess;
+    if (rc == BDG_OK) {
+        err = cudaMemcpyAsync(pos.ptr, k, (size_t)n * sizeof(int64_t), cudaMemcpyHostToDevice, sys->stream);
+        if (err == cudaSuccess) {
+            gather_blocks<<<grid_for(n * 16), kThreads, 0, sys->stream>>>(n, pos.as<int64_t>(), m.data.as<double2>(),
+                                                                            val.as<double2>());
+            err = cudaGetLastError();
+        }
+        if (err == cudaSuccess)
+            err = cudaMemcpyAsync(out, val.ptr, (size_t)n * 16 * sizeof(double2), cudaMemcpyDeviceToHost, sys->stream);
+        if (err == cudaSuccess) err = cudaStreamSynchronize(sys->stream);
+    }
+    dev_free(sys, pos);
+    dev_free(sys, val);
+    BDG_TRY(rc);
     BDG_CUDA(err);
     return BDG_OK;
 }

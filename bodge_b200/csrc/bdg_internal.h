@@ -272,6 +272,9 @@ struct bdg_system {
     ChebState cheb;
     EllDev ell;
     DevBuf multi_send, multi_recv;  // moments of this GPU / of all GPUs around the NCCL collective (multi.cu)
+    // Distance classes of the sites for BDG_X0_CLASS start vectors (bdg_set_classes): int32 [n_sites], values < n_classes.
+    DevBuf site_class;
+    int32_t n_classes = 0;  // 0: none uploaded
 };
 
 // scan.cu

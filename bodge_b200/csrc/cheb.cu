@@ -240,6 +240,27 @@ init_rademacher(double2 *__restrict__ x, int64_t n_elems, int n_sites, int pw, i
     x[t] = make_double2(v, 0.0);
 }
 
+// Class columns: column c is the indicator of class class_rows[c] >> 2 in component class_rows[c] & 3.  One thread per
+// complex element of the padded vector set, like init_rademacher.
+__global__ void __launch_bounds__(kThreads)
+init_classes(double2 *__restrict__ x, int64_t n_elems, int n_sites, int pw, int n_cols, const int32_t *__restrict__ site_class,
+             const int64_t *__restrict__ class_rows) {
+    int64_t t = (int64_t)blockIdx.x * kThreads + threadIdx.x;
+    if (t >= n_elems) return;
+    const int alpha = (int)(t & 3);
+    const int c = (int)((t >> 2) % pw);
+    const int64_t rec = (t >> 2) / pw;
+    const int site = (int)(rec % n_sites);
+    const int panel = (int)(rec / n_sites);
+    const int colg = panel * pw + c;
+    double v = 0.0;
+    if (colg < n_cols) {
+        const int64_t q = class_rows[colg];
+        v = (alpha == (int)(q & 3) && (int64_t)site_class[site] == (q >> 2)) ? 1.0 : 0.0;
+    }
+    x[t] = make_double2(v, 0.0);
+}
+
 __global__ void init_probes(double2 *__restrict__ x, int n_sites, int pw, int n_cols,
                             const int64_t *__restrict__ probe_rows) {
     int c = blockIdx.x * blockDim.x + threadIdx.x;
@@ -477,13 +498,38 @@ void cheb_release(bdg_system *sys) {
     st.launches = launches;
 }
 
+extern "C" int bdg_set_classes(bdg_t *sys, int64_t n_sites, const int32_t *site_class, int32_t n_classes) {
+    BDG_ENTER(sys);
+    BDG_REQUIRE(n_sites == sys->skel.n_sites, "%lld site classes given for %lld sites", (long long)n_sites,
+                (long long)sys->skel.n_sites);
+    BDG_REQUIRE(n_classes >= 1, "need at least one class, %d given", n_classes);
+    BDG_REQUIRE(site_class != nullptr, "null argument");
+    for (int64_t i = 0; i < n_sites; ++i)
+        BDG_REQUIRE(site_class[i] >= 0 && site_class[i] < n_classes, "site %lld: class %d outside [0, %d)", (long long)i,
+                    site_class[i], n_classes);
+    sys->n_classes = 0;  // (no classes while the upload may fail half way)
+    BDG_TRY(dev_alloc(sys, sys->site_class, (size_t)n_sites * sizeof(int32_t)));
+    BDG_CUDA(cudaMemcpyAsync(sys->site_class.ptr, site_class, (size_t)n_sites * sizeof(int32_t), cudaMemcpyHostToDevice,
+                             sys->stream));
+    BDG_CUDA(cudaStreamSynchronize(sys->stream));  // site_class is borrowed only for this call
+    sys->n_classes = n_classes;
+    return BDG_OK;
+}
+
 extern "C" int bdg_cheb_begin(bdg_t *sys, int kind, int32_t n_cols, const int64_t *probe_rows, uint64_t seed,
                               int64_t col_offset, double scale, int kernel) {
     BDG_ENTER(sys);
-    BDG_REQUIRE(kind == BDG_X0_PROBE || kind == BDG_X0_RADEMACHER, "unknown start-vector kind %d", kind);
+    BDG_REQUIRE(kind == BDG_X0_PROBE || kind == BDG_X0_RADEMACHER || kind == BDG_X0_CLASS, "unknown start-vector kind %d", kind);
     BDG_REQUIRE(n_cols >= 1, "need at least one column");
     BDG_REQUIRE(scale > 0.0, "scale must be positive");
-    BDG_REQUIRE(kind != BDG_X0_PROBE || probe_rows != nullptr, "probe rows missing");
+    BDG_REQUIRE(kind == BDG_X0_RADEMACHER || probe_rows != nullptr, kind == BDG_X0_CLASS ? "class rows missing" : "probe rows missing");
+    if (kind == BDG_X0_CLASS) {
+        BDG_REQUIRE(sys->n_classes > 0, "no site classes uploaded (bdg_set_classes)");
+        for (int c = 0; c < n_cols; ++c)
+            BDG_REQUIRE(probe_rows[c] >= 0 && (probe_rows[c] >> 2) < sys->n_classes,
+                        "column %d: class row %lld names class %lld, beta %lld; classes are 0 .. %d", c, (long long)probe_rows[c],
+                        (long long)(probe_rows[c] >> 2), (long long)(probe_rows[c] & 3), sys->n_classes - 1);
+    }
     BDG_REQUIRE(kernel >= BDG_KERNEL_AUTO && kernel <= BDG_KERNEL_AUTO_MOMENTS && kernel != 4 && kernel != 5,  // 4, 5: unassigned (bdg.h)
                 "unknown kernel %d", kernel);
     BDG_TRY(build_packed(sys));
@@ -542,6 +588,12 @@ extern "C" int bdg_cheb_begin(bdg_t *sys, int kind, int32_t n_cols, const int64_
     if (kind == BDG_X0_RADEMACHER) {
         init_rademacher<<<(unsigned)ceil_div((int64_t)vec_elems, kThreads), kThreads, 0, sys->stream>>>(
             x0, (int64_t)vec_elems, n, st.panel_width, n_cols, seed, col_offset);
+    } else if (kind == BDG_X0_CLASS) {
+        BDG_TRY(dev_alloc(sys, st.mu_tmp, (size_t)n_cols * sizeof(int64_t)));
+        BDG_CUDA(cudaMemcpyAsync(st.mu_tmp.ptr, probe_rows, (size_t)n_cols * sizeof(int64_t), cudaMemcpyHostToDevice, sys->stream));
+        init_classes<<<(unsigned)ceil_div((int64_t)vec_elems, kThreads), kThreads, 0, sys->stream>>>(
+            x0, (int64_t)vec_elems, n, st.panel_width, n_cols, sys->site_class.as<int32_t>(), st.mu_tmp.as<int64_t>());
+        BDG_CUDA(cudaStreamSynchronize(sys->stream));  // probe_rows is borrowed only for this call
     } else {
         BDG_CUDA(cudaMemsetAsync(x0, 0, vec_elems * sizeof(double2), sys->stream));
         BDG_TRY(dev_alloc(sys, st.mu_tmp, (size_t)n_cols * sizeof(int64_t)));

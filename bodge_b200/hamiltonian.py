@@ -16,7 +16,7 @@ from __future__ import annotations
 import os
 import warnings
 
-from . import _native, distributed, kpm
+from . import _native, distributed, kpm, probing
 from .common import *
 from .helpers import dwave, pwave, ssd, swave  # the reference exports them from bodge.hamiltonian (hamiltonian.py:390-531)
 from .lattice import CubicLattice, Lattice
@@ -118,6 +118,7 @@ class Hamiltonian:
         # analytic periodic stencil; any other Lattice goes through its own iterator once.
         stock = isinstance(lattice, CubicLattice) and all(
             getattr(type(lattice), m) is getattr(CubicLattice, m) for m in ("index", "sites", "bonds", "edges"))
+        self._stock = stock
         if stock:
             self._sys = _native.System.cubic(lattice.shape, self.device)
         else:
@@ -127,6 +128,7 @@ class Hamiltonian:
             self._sys = _native.System.generic(lattice.size, pi, pj, self.device)
         self._structure = None  # host copy of (indptr, indices) of the skeleton, fetched lazily
         self._scale_cache = None
+        self._class_cache = None  # ((spacing, wrapping axes), class of every site) as last uploaded (bdg_set_classes)
 
     # ------------------------------------------------------------------------------------
     # context manager: collect dict entries, scatter them on exit
@@ -277,7 +279,7 @@ class Hamiltonian:
                              rows=rows, vectors=vectors, seed=seed, scale=scale, kernel=kernel, batch=batch, group=group)
 
     def _columns(self, moments, read, summed, *, rows=None, vectors=None, seed=1234, scale=None, kernel="auto",
-                 batch=None, group="auto", begin=None):
+                 batch=None, group="auto", begin=None, x0="probe", out=None):
         """Run the recursion for ``moments`` moments over all start columns -- sharded over the
         ranks of the process group, in batches on this GPU -- and reduce each batch ON THE DEVICE
         with ``read(system, n_columns)``, which returns ``[m, n_columns]`` (per column) or ``[m]``
@@ -285,7 +287,11 @@ class Hamiltonian:
 
         ``begin(system, c0, c1)`` is called after each batch's ``cheb_begin`` with the batch's columns ``[c0, c1)`` of
         the full list, to register a local accumulator.  ``moments`` is then the length of a series without moment
-        doubling (``moments - 1`` steps), and ``kernel="auto"`` stays on kernels that keep every vector."""
+        doubling (``moments - 1`` steps), and ``kernel="auto"`` stays on kernels that keep every vector.
+
+        ``x0="class"``: ``rows`` are class rows ``4k + β`` (``_classes``), each the indicator of class ``k`` in component
+        ``β``.  ``out`` (``summed`` only): ``read`` writes its batch's share into this array itself and returns nothing;
+        ``out`` is this rank's result, so the host holds one array whatever the number of batches."""
         if (rows is None) == (vectors is None):
             raise ValueError("give either rows= (probe columns) or vectors= (random columns)")
         scale = self.spectral_bound() if scale is None else float(scale)
@@ -302,7 +308,9 @@ class Hamiltonian:
         parts = []
         for b0 in range(0, n_local, batch):
             b1 = min(n_local, b0 + batch)
-            if rows is not None:
+            if rows is not None and x0 == "class":
+                self._sys.cheb_begin(class_rows=rows[lo + b0 : lo + b1], scale=scale, kernel=kernel)
+            elif rows is not None:
                 self._sys.cheb_begin(probe_rows=rows[lo + b0 : lo + b1], scale=scale, kernel=kernel)
             else:
                 self._sys.cheb_begin(n_random=b1 - b0, seed=seed, col_offset=lo + b0, scale=scale, kernel=kernel)
@@ -310,8 +318,12 @@ class Hamiltonian:
                 begin(self._sys, lo + b0, lo + b1)
             done = self._sys.cheb_available() // 2 - 1      # steps bdg_cheb_begin has already taken (1 with T2)
             self._sys.cheb_steps(max(0, steps - done))
-            parts.append(np.asarray(read(self._sys, b1 - b0), dtype=np.float64))
-        if summed:
+            part = read(self._sys, b1 - b0)
+            if out is None:
+                parts.append(np.asarray(part, dtype=np.float64))
+        if out is not None:
+            local = out
+        elif summed:
             local = np.sum(parts, axis=0) if parts else None
         else:
             local = np.concatenate(parts, axis=1) if parts else None
@@ -490,14 +502,49 @@ class Hamiltonian:
     # would need diagonalize(), a dense O((4N)^3) eigensolver)
     # ------------------------------------------------------------------------------------
     def _flat(self, coords) -> np.ndarray:
+        if self._stock:  # integer [n, 3] coordinates on a stock CubicLattice: one vectorised lookup, same errors
+            arr = np.asarray(coords)
+            if arr.ndim == 2 and arr.shape[1] == 3 and arr.dtype.kind in "iu":
+                return self.lattice.index_many(arr)
         return np.array([self.lattice[tuple(int(v) for v in c)] for c in coords], dtype=np.int64)
 
+    def _wrapping_axes(self) -> tuple[bool, bool, bool]:
+        """Per axis of the (cubic) lattice: does any non-zero stored block couple its two faces?  Read on the device from
+        the periodic-edge blocks of that axis only (``bdg_gather_blocks``).  Axes of length <= 2 count as open: their
+        edge pairs are the site itself or its bond, and the class rule gives the same classes either way."""
+        wraps = []
+        for axis, length in enumerate(self.lattice.shape):
+            if length <= 2:
+                wraps.append(False)
+                continue
+            lo, hi = self.lattice.edges_array(axis)
+            k = self._sys.lookup(np.concatenate([lo, hi]), np.concatenate([hi, lo]))
+            wraps.append(bool(self._sys.gather_blocks(k).any()))
+        return tuple(wraps)
+
+    def _classes(self, spacing) -> np.ndarray:
+        """Distance class of every site for ``spacing`` (``probing.site_classes``), uploaded to the device when it differs
+        from what the handle holds; the wrap of each axis is read from the matrix as it is now."""
+        if isinstance(spacing, bool) or not isinstance(spacing, (int, np.integer)) or spacing < 1:
+            raise ValueError(f"spacing must be a positive integer or None, got {spacing!r}")
+        if not self._stock:
+            raise ValueError(f"spacing= needs a CubicLattice (its distance classes are built per axis), not {self.lattice!r}")
+        key = (int(spacing), self._wrapping_axes())
+        if self._class_cache is None or self._class_cache[0] != key:
+            site_class, n_classes = probing.site_classes(self.lattice.shape, *key)
+            self._sys.set_classes(site_class, n_classes)
+            self._class_cache = (key, site_class)
+        return self._class_cache[1]
+
     def _fermi_local(self, temperature, rows, read_col, read_site, *, moments=None, scale=None, tol=1e-13,
-                     kernel="auto", batch=None, caller="density_matrix"):
+                     kernel="auto", batch=None, caller="density_matrix", site_class=None):
         """``acc[r, α] = f(H)[4 read_site[r] + α, rows[read_col[r]]]`` as complex ``[n_reads, 4]``: one probe column
         per entry of ``rows``, the Fermi series contracted on the device while the recursion runs (``bdg.h``:
         ``bdg_cheb_local_begin``).  Columns are batched and sharded like every other observable; the reads of a batch
-        land in their slots of one ``[n_reads, 4]`` array, so the ranks combine with a plain sum."""
+        land in their slots of one ``[n_reads, 4]`` array, so the ranks combine with a plain sum.
+
+        ``site_class`` given: ``rows`` are class rows ``4k + β`` and column ``c`` is the indicator of class ``k`` in
+        component ``β``, so the read is ``Σ_{j in class k} f(H)[4 read_site[r] + α, 4j + β]`` (``probing``)."""
         T = float(temperature)
         if not T > 0:
             raise ValueError(f"{caller} needs a temperature T > 0 (the Fermi function at T = 0 is a step function)")
@@ -507,6 +554,10 @@ class Hamiltonian:
         n_reads = len(read_col)
         scale = self.spectral_bound() if scale is None else float(scale)
         if scale == 0.0:  # H = 0: f(H) = f(0) 1 = 1/2
+            if site_class is not None:
+                q = rows[read_col]
+                hit = (np.arange(4) == (q & 3)[:, None]) & (site_class[read_site] == q >> 2)[:, None]
+                return np.where(hit, 0.5, 0.0).astype(np.complex128)
             alpha = 4 * read_site[:, None] + np.arange(4)
             return np.where(alpha == rows[read_col][:, None], 0.5, 0.0).astype(np.complex128)
         need, reached = kpm.free_energy_moments(T, scale, tol)
@@ -517,27 +568,32 @@ class Hamiltonian:
                           f"~{level:.1e} relative (tol = {tol:g} needs {int(np.ceil(-np.log(tol) * scale / (np.pi * T)))})",
                           AccuracyWarning, stacklevel=3)
         coef = kpm.fermi_coefficients(T, n_coef, scale)
-        batch_reads = []
+        # Every read belongs to one column, hence to one batch: the batches fill their slots of ONE array (host memory
+        # O(n_reads) whatever the batch count), and a batch finds its reads by bisection in the column order.
+        acc = np.zeros((n_reads, 4), dtype=np.complex128)
+        order = np.argsort(read_col, kind="stable")
+        sorted_col = read_col[order]
+        batch_reads = [None]
 
         def begin(sysn, c0, c1):
-            mine = np.flatnonzero((read_col >= c0) & (read_col < c1))
-            batch_reads.append(mine)
+            mine = order[np.searchsorted(sorted_col, c0):np.searchsorted(sorted_col, c1)]
+            batch_reads[0] = mine
             if len(mine):
                 sysn.cheb_local_begin(coef, read_col[mine] - c0, read_site[mine])
 
         def read(sysn, k):
-            full = np.zeros((n_reads, 4), dtype=np.complex128)
-            mine = batch_reads[-1]
+            mine = batch_reads[0]
             if len(mine):
-                full[mine] = sysn.cheb_local_read(len(mine))
-            return full.view(np.float64).ravel()
+                acc[mine] = sysn.cheb_local_read(len(mine))
 
         read.leading_dim = 8 * n_reads
-        total = self._columns(n_coef, read, True, rows=rows, scale=scale, kernel=kernel, batch=batch, begin=begin)
+        total = self._columns(n_coef, read, True, rows=rows, scale=scale, kernel=kernel, batch=batch, begin=begin,
+                              x0="probe" if site_class is None else "class", out=acc.view(np.float64).ravel())
         return np.ascontiguousarray(total, dtype=np.float64).view(np.complex128).reshape(n_reads, 4)
 
     def density_matrix(self, temperature: float, pairs, *, moments: int | None = None, scale: float | None = None,
-                       tol: float = 1e-13, kernel: str = "auto", batch: int | None = None) -> Matrix:
+                       tol: float = 1e-13, kernel: str = "auto", batch: int | None = None,
+                       spacing: int | None = None) -> Matrix:
         """Blocks of the one-body density matrix ``ρ = f(H)``, ``f(ε) = 1/(1 + e^{ε/T})``: complex
         ``[len(pairs), 4, 4]`` with ``result[p] = f(H)[4i:4i+4, 4j:4j+4]`` for ``pairs[p] = (i, j)`` (coordinates, like
         ``H[i, j]`` keys; basis e↑, e↓, h↑, h↓).  With the Nambu spinor ``Ψ = (c↑, c↓, c↑†, c↓†)``,
@@ -550,19 +606,28 @@ class Hamiltonian:
         truncation error ``tol``, the rule of ``free_energy`` (capped at 32768 terms); an explicit ``moments`` below
         that, or the cap, raise an ``AccuracyWarning``.  The series has no moment doubling: ``moments - 1`` steps.
         ``kernel="auto"`` runs the pair or a single-step kernel (the even-vector ``"t2"`` keeps every second vector
-        only and is refused).  T <= 0 raises ``ValueError``."""
+        only and is refused).  T <= 0 raises ``ValueError``.
+
+        ``spacing`` (``CubicLattice`` only): probe whole distance classes of sites instead of single sites
+        (``probing``): the four columns of class ``k`` are ``Σ_{j in class k} e_{4j+β}``, so the blocks of every site
+        take four columns per class -- about ``4 spacing²`` on a plane -- instead of four per site.  The block read for
+        ``(i, j)`` is then ``Σ_{j' in class(j)} f(H)[4i:4i+4, 4j':4j'+4]``: exactly today's block (up to rounding) when
+        ``spacing >= moments``, since the series has degree ``moments - 1``; with a smaller spacing it adds the elements
+        of ``f(H)`` between ``i`` and sites at least ``spacing`` hops away, which decay exponentially with the distance
+        at T > 0."""
         pairs = list(pairs)
+        site_class = None if spacing is None else self._classes(spacing)
         i = self._flat([p[0] for p in pairs])
         j = self._flat([p[1] for p in pairs])
         off = i != j
         if off.any():
             self._sys.lookup(i[off], j[off])  # IndexError for a pair that is no block of the skeleton
-        uj, pos = np.unique(j, return_inverse=True)
-        rows = (4 * uj[:, None] + np.arange(4)).ravel()
+        uj, pos = np.unique(j if site_class is None else site_class[j], return_inverse=True)
+        rows = (4 * uj[:, None] + np.arange(4)).ravel()  # probe rows of the sites j, or class rows of their classes
         read_col = (4 * pos[:, None] + np.arange(4)).ravel()  # read 4p + β: column (j_p, β) at site i_p
         read_site = np.repeat(i, 4)
         acc = self._fermi_local(temperature, rows, read_col, read_site, moments=moments, scale=scale, tol=tol,
-                                kernel=kernel, batch=batch, caller="density_matrix")
+                                kernel=kernel, batch=batch, caller="density_matrix", site_class=site_class)
         return acc.reshape(len(pairs), 4, 4).transpose(0, 2, 1).copy()  # acc[4p + β, α] -> [p, α, β]
 
     def _potential(self, potential, sites):
@@ -571,6 +636,14 @@ class Hamiltonian:
             table = {int(k): float(v) for k, v in zip(self._flat(list(potential)), potential.values())}
         else:
             table = None
+        if sites is None and self._stock:  # every site of a stock CubicLattice: vectorised, in index order
+            if table is not None:
+                V = np.zeros(self.lattice.size)
+                V[np.fromiter(table.keys(), np.int64, len(table))] = np.fromiter(table.values(), np.float64, len(table))
+            else:
+                V = np.full(self.lattice.size, float(potential))
+            flat = np.flatnonzero(V != 0.0)
+            return self.lattice.sites_array()[flat], flat, V[flat]
         if sites is None:
             sites = [s for s in self.lattice.sites()
                      if (table.get(self.lattice[s], 0.0) if table is not None else float(potential)) != 0.0]
@@ -586,12 +659,22 @@ class Hamiltonian:
 
         ``potential``: one ``V`` for every site, or a ``{site: V}`` dict; ``sites`` defaults to every site with
         ``V_i != 0``.  One probe column per site (row ``4i+3``) and one read, a quarter of ``density_matrix``'s work
-        for the same sites.  ``kpm_options``: ``moments``, ``scale``, ``tol``, ``kernel``, ``batch`` as there."""
+        for the same sites.  ``kpm_options``: ``moments``, ``scale``, ``tol``, ``kernel``, ``batch``, ``spacing`` as
+        there; with ``spacing`` one column per distance class (row ``3`` of the class) serves all its sites."""
         sites, flat, V = self._potential(potential, sites)
+        return self._order_parameter(temperature, flat, V, **kpm_options)
+
+    def _order_parameter(self, temperature, flat, V, *, spacing=None, **kpm_options):
+        site_class = None if spacing is None else self._classes(spacing)
         if len(flat) == 0:
             return np.zeros(0, dtype=np.complex128)
-        acc = self._fermi_local(temperature, 4 * flat + 3, np.arange(len(flat)), flat, caller="order_parameter",
-                                **kpm_options)
+        if site_class is None:
+            acc = self._fermi_local(temperature, 4 * flat + 3, np.arange(len(flat)), flat, caller="order_parameter",
+                                    **kpm_options)
+        else:
+            classes, pos = np.unique(site_class[flat], return_inverse=True)
+            acc = self._fermi_local(temperature, 4 * classes + 3, pos, flat, caller="order_parameter", site_class=site_class,
+                                    **kpm_options)
         return -V * acc[:, 0]
 
     def selfconsistent(self, temperature: float, potential, *, tol: float = 1e-8, max_iter: int = 500,
@@ -601,15 +684,17 @@ class Hamiltonian:
         ``max_i |Δ_i^new - Δ_i| <= tol``.  ``mixing`` < 1 moves only that fraction of the way per iteration.  Starts
         from the pairing the system holds (set a non-zero guess: ``Δ = 0`` is always a fixed point) and leaves the
         last state in it.  Each iteration rewrites N of the ~5N blocks of a square lattice, which the library patches
-        into its copies of the matrix in place.  Returns ``(Δ, iterations)``; warns if ``max_iter`` is reached."""
+        into its copies of the matrix in place.  Returns ``(Δ, iterations)``; warns if ``max_iter`` is reached.
+        ``kpm_options`` as for ``order_parameter``; with ``spacing`` the iteration converges to the fixed point of the
+        class-probed map (``density_matrix``), which is the exact one when ``spacing`` is at least the series length."""
         if not 0 < mixing <= 1:
             raise ValueError("mixing must be in (0, 1]")
-        sites, flat, V = self._potential(potential, None)
+        _, flat, V = self._potential(potential, None)
         if len(flat) == 0:
             return np.zeros(0, dtype=np.complex128), 0
-        delta = self._sys.export_bsr(False)[2][self._sys.lookup(flat, flat), 0, 3]
+        delta = self._sys.gather_blocks(self._sys.lookup(flat, flat))[:, 0, 3]  # the on-site blocks only, not the matrix
         for it in range(1, int(max_iter) + 1):
-            new = self.order_parameter(temperature, potential, sites, **kpm_options)
+            new = self._order_parameter(temperature, flat, V, **kpm_options)
             step = np.max(np.abs(new - delta))
             delta = delta + mixing * (new - delta)
             self.fill((), (), (), flat, flat, delta[:, None, None] * jσ2)

@@ -112,6 +112,10 @@ int bdg_export_bsr(bdg_t *sys, int eliminate_zeros, int64_t *n_blocks, int32_t *
  * bdg_export_dense: out[4N][4N] complex128, row-major. */
 int bdg_export_csr(bdg_t *sys, int transpose, int64_t *nnz, int32_t *indptr, int32_t *indices, double *data);
 int bdg_export_dense(bdg_t *sys, double *out);
+/* out[e] = the stored block at skeleton position k[e] (from bdg_lookup), [4][4] complex128 row-major: n * 32 doubles.
+ * A few chosen blocks without exporting the matrix, e.g. the periodic-edge blocks of one lattice axis, to learn whether
+ * any of them is non-zero (whether that axis wraps).  BDG_E_INVALID names the first position outside the skeleton. */
+int bdg_gather_blocks(bdg_t *sys, int64_t n, const int64_t *k, double *out);
 /* Overwrite all stored values from a host array laid out like the skeleton's data (inverse of
  * export with eliminate_zeros = 0; used for `system._data[...] = ...` style direct edits). */
 int bdg_import_data(bdg_t *sys, const double *data);
@@ -122,7 +126,7 @@ int bdg_norm_inf(bdg_t *sys, double *norm);
 
 /* ---- Chebyshev / KPM engine (no reference code; arithmetic = scipy bsr_matvecs on
  *      matrix("bsr"), consumers = free_energy / ldos, bodge/hamiltonian.py:253-387) --------- */
-enum { BDG_X0_PROBE = 0, BDG_X0_RADEMACHER = 1 };
+enum { BDG_X0_PROBE = 0, BDG_X0_RADEMACHER = 1, BDG_X0_CLASS = 2 };
 enum { BDG_MU_PER_COLUMN = 0, BDG_MU_SUM = 1 };
 /* AUTO = PAIR where it applies (DICT / DICT_DIAG matrix, nearest-neighbour stencil on a lattice with one-dimensional
  *        x-planes, >= 5 columns), else DICT_DIAG, else DICT, else ELL -- the first the matrix qualifies for -- else DMMA.
@@ -163,9 +167,20 @@ enum { BDG_KERNEL_AUTO = 0, BDG_KERNEL_DMMA = 1, BDG_KERNEL_FMA = 2, BDG_KERNEL_
        BDG_KERNEL_DICT = 6, BDG_KERNEL_DICT_DIAG = 7,
        BDG_KERNEL_PAIR = 8, BDG_KERNEL_T2 = 9, BDG_KERNEL_AUTO_MOMENTS = 10 };
 
+/* Distance classes of the sites for BDG_X0_CLASS start vectors: site_class[i] in [0, n_classes) for every site i < n_sites
+ * (n_sites must be the skeleton's).  Uploaded once and kept by the handle for every later recursion until the next call;
+ * BDG_E_INVALID names the first bad entry.  The caller chooses the classes so that two distinct sites of one class are
+ * far apart in the graph of the stored blocks: a polynomial p(H~) of degree m has no element between sites more than m
+ * hops apart, so a class column read at one of its sites gives p(H~)'s element there plus those to the class's other
+ * sites (Hamiltonian.density_matrix(spacing=...)). */
+int bdg_set_classes(bdg_t *sys, int64_t n_sites, const int32_t *site_class, int32_t n_classes);
+
 /* Start a recursion on n_cols start vectors resident on this GPU.
  *   kind = BDG_X0_PROBE:      column c = unit vector e_{probe_rows[c]}           (LDOS-type)
  *   kind = BDG_X0_RADEMACHER: column c = +-1 vector hashed from (seed, row, col_offset + c)
+ *   kind = BDG_X0_CLASS:      column c = sum of e_{4i+beta} over the sites i of class k (bdg_set_classes), given as the
+ *                             "class row" probe_rows[c] = 4k + beta, beta in 0..3 -- the probe row of a class instead
+ *                             of a site; k >= n_classes is refused with the column named
  * scale = a  (H~ = H / a must have its spectrum inside [-1, 1]).
  * Builds T_0 = X0 and T_1 = H~ T_0 and the first two dot products. */
 int bdg_cheb_begin(bdg_t *sys, int kind, int32_t n_cols, const int64_t *probe_rows, uint64_t seed,
